@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the cuberille hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--size S] [--period P]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--size S] [--period P] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path through the C-ABI (cub_count_async -> [count exchange] ->
 cub_emit_async: classify -> ownership sweep -> segment scan -> vertices -> faces) over a synthetic
@@ -15,6 +15,9 @@ separately (`gather`, `extras.weak`).  Rank 0 prints ONE JSON line.
 
 `--impl reference` times the CPU restatement of the reference filter (oracle/, single-threaded like
 GenerateData itself) on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes the mesh of the last timed step to DIR/*.npy (see dump_outputs); the
+volume is generated on the device from the arguments alone, so two builds can be compared file for file.
 """
 from __future__ import annotations
 
@@ -29,6 +32,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the tree this runs from may be read-only: nothing is written there
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
@@ -48,7 +52,15 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-gather", action="store_true", help="skip the all-gather of the meshes (N > 1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the mesh of the last timed step to DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs applies to --impl cuda (the reference's sample size depends on the host's speed)")
+    return args
 
 
 FIELD_KIND = {"gyroid": 0, "marschner_lobb": 1, "blobs": 2}
@@ -210,6 +222,43 @@ def workload_config(args, n, scaling=None):
             "timed regions only; every step still reads its slab from HBM after the previous step's 2+ GB of scratch and mesh traffic"}
 
 
+# rows of the points and of the cells that --dump-outputs writes, over all ranks: at most 12 + 4 * 8 bytes a row
+# (a float32 point, a quad's ids as float64), 46 MB in all
+DUMP_ROWS = 1 << 20
+
+
+def dump_outputs(out_dir, capi, h, dev, rank, n_ranks):
+    """Write the mesh the last step left in the handle, as a caller fetches it, to out_dir: `points` [n, 3] float32,
+    `cells` [m, k] vertex ids (float64, exact below 2**53) and `counts` (n, m).  A mesh of more than
+    DUMP_ROWS / n_ranks rows is sampled: the rows are seeded and sorted, so the same counts give the same rows.
+    With several ranks every rank writes its own part (ids global), with a `_rank<r>` suffix."""
+    import numpy as np
+    import torch
+    info = h.device_buffers()
+    n, m, k = info["n_points"], info["n_cells"], info["verts_per_cell"]
+    pts = torch.empty((max(n, 1), 3), dtype=torch.float32, device=dev)
+    cells = torch.empty((max(m, 1), k), dtype=torch.int32 if info["id_bytes"] == 4 else torch.int64, device=dev)
+    h.fetch_into(pts.data_ptr(), cells.data_ptr(), 0, capi.MEM_DEVICE)
+    rows = DUMP_ROWS // n_ranks
+
+    def sample(t, total, seed):
+        if total <= rows:
+            return t[:total].cpu().numpy()
+        idx = np.sort(np.random.default_rng(seed).choice(total, rows, replace=False))
+        return t.index_select(0, torch.from_numpy(idx).to(dev)).cpu().numpy()
+
+    suffix = f"_rank{rank}" if n_ranks > 1 else ""
+    cell_ids = sample(cells, m, 2)
+    if cell_ids.dtype == np.int32:
+        cell_ids = cell_ids.view(np.uint32)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"points{suffix}.npy"), sample(pts, n, 1))
+    np.save(os.path.join(out_dir, f"cells{suffix}.npy"), cell_ids.astype(np.float64))
+    np.save(os.path.join(out_dir, f"counts{suffix}.npy"), np.array([n, m], np.float64))
+    del pts, cells
+    torch.cuda.empty_cache()
+
+
 def bind_to_gpu_numa_node(local_rank):
     """Run this rank (and allocate its pinned buffers: first touch) on the NUMA node its GPU hangs off."""
     try:
@@ -351,6 +400,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     n_pts, n_quads, tot_p, tot_q = R.totals()
     tot = (tot_p, tot_q)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, capi, h, dev, rank, N)
 
     voxels_total = sum_ranks(S * S * (own1 - own0))
     gvox = voxels_total / (ms_step * 1e-3) / 1e9

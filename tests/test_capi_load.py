@@ -28,12 +28,19 @@ def test_default_params_are_the_reference_constructor_defaults():
 
 
 def test_no_cpu_fallback():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    P = pkg()
-    with pytest.raises(P.capi.CuberilleError):
-        P.capi.Handle(0)
+    # in a child process that sees no device (CUDA_VISIBLE_DEVICES hides one that is present)
+    import subprocess
+    import sys
+    code = ("import importlib, sys\n"
+            "P = importlib.import_module('midas-journal-740_b200')\n"
+            "try:\n"
+            "    P.capi.Handle(0)\n"
+            "except P.capi.CuberilleError:\n"
+            "    sys.exit(0)\n"
+            "sys.exit('a handle was created without a device')\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def test_product_does_not_import_the_oracle():
