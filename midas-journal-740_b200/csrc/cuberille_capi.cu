@@ -407,8 +407,7 @@ bool launch_fused(cub_handle h, const SweepArgs& ca, int cfg, unsigned* ctr, uns
   return false;
 }
 
-// K4 on `pts` (explicit count n), or - from_info - on the handle's point buffer with the range taken from the
-// device-side run info (n = the capacity of the buffer)
+// capacities of the result buffers, for k_check_caps (and the early record loads of k_vertices)
 Caps make_caps(cub_handle h, unsigned long long quads_cap) {
   Caps c;
   c.raster = h->raster ? 1 : 0;
@@ -418,8 +417,9 @@ Caps make_caps(cub_handle h, unsigned long long quads_cap) {
   return c;
 }
 
-int launch_project(cub_handle h, float* pts, size_t n, bool from_info, bool include_ghost, bool guard = false,
-                   unsigned long long quads_cap = ~0ull) {
+// K4 on `pts` (explicit count n), or - from_info - on the handle's point buffer with the range taken from the
+// device-side run info (n = the capacity of the buffer)
+int launch_project(cub_handle h, float* pts, size_t n, bool from_info, bool include_ghost) {
   if (n == 0) return CUB_OK;
   ProjArgs a;
   a.vol = h->d_vol;
@@ -435,8 +435,6 @@ int launch_project(cub_handle h, float* pts, size_t n, bool from_info, bool incl
   a.n_points = n;
   a.info = from_info ? h->d_info : nullptr;
   a.include_ghost = include_ghost ? 1 : 0;
-  a.guard = guard ? 1 : 0;
-  a.caps = make_caps(h, quads_cap);
   a.work = h->d_info + kInfoWords;
   a.refill = (unsigned)h->knobs.proj_refill;
   CU_TRY(h, cudaMemsetAsync(a.work, 0, sizeof(unsigned long long), h->stream));
@@ -901,8 +899,9 @@ int count_finish(cub_handle h) {
 
 // The vertex stage of cub_emit: K3a (reference order) or k_points_raster.  It needs the counts but not the id
 // base, so a multi-GPU caller can queue it before the ranks have exchanged their counts (cub_emit_vertices).
-// exact: the host knows the counts and sizes the buffers; otherwise the buffers keep their sizes (the kernels
-// guard their writes and flag an overflow).
+// exact: the host knows the counts, sizes the buffers and the grids from them; otherwise the buffers keep their
+// sizes and the grids cover their capacity (k_check_caps flags an emission that does not fit).  Either way the
+// kernels read the counts from the device-side run info.
 const int kNeedSizes = -1000;
 
 // quads, triangles with the fixed split, or quads into a scratch buffer that K5 splits by the diagonal test.
@@ -915,26 +914,31 @@ int emit_mode(cub_handle h) {
   return (P.project_vertices || h->geom.oriented) ? kEmitScratchQuads : kEmitTrisFixed;
 }
 
+int size_vertex_buffers(cub_handle h) {
+  const size_t n_pts_all = (size_t)(h->ghost_v + h->n_points);
+  CUB_TRY(ensure(h, h->points, 3 * (n_pts_all + n_pts_all / 16)));
+  if (!h->raster) {
+    CUB_TRY(ensure(h, h->perm, (size_t)h->n_active + (size_t)h->n_active / 16));
+    CUB_TRY(ensure(h, h->vtx, h->points.cap / 3));
+  }
+  return CUB_OK;
+}
+
 int emit_vertex_stage(cub_handle h, bool exact) {
   const Grid& g = h->g;
   const int mode = emit_mode(h);
   const int nz = h->zs1 - h->owner_z_min;
   if (exact) {
-    const size_t n_pts_all = (size_t)(h->ghost_v + h->n_points);
-    CUB_TRY(ensure(h, h->points, 3 * (n_pts_all + n_pts_all / 16)));
-    if (!h->raster) {
-      CUB_TRY(ensure(h, h->perm, (size_t)h->n_active + (size_t)h->n_active / 16));
-      CUB_TRY(ensure(h, h->vtx, h->points.cap / 3));
-    }
+    CUB_TRY(size_vertex_buffers(h));
     if (h->n_quads == 0) { h->vertices_done = true; return CUB_OK; }
   } else if (!h->points.p || (!h->raster && (!h->perm.p || !h->vtx.p))) {
     return kNeedSizes;
   }
   h->vertices_done = true;
   h->projected = false;
-  if (!exact && !h->caps_checked) {
-    // the one comparison of the device-side counts with the capacity of the buffers (the quads are checked again,
-    // with the cell buffers of the emission, in emit_launch)
+  if (!h->caps_checked) {
+    // the vertex stage queued ahead of the emission (cub_emit_vertices): the vertex buffers are checked now, the
+    // quads with the cell buffers of the emission, in emit_launch
     CU_TRY(h, launch_step(h, k_check_caps, dim3(1), dim3(32), true, h->d_info, make_caps(h, ~0ull)));
   }
   // the points of the vertices the slab underneath owns are only needed by the projected triangle split
@@ -951,11 +955,10 @@ int emit_vertex_stage(cub_handle h, bool exact) {
       a.cnt = h->cnt.p; a.own = h->own.p; a.seg = h->seg.p; a.cofs = h->cofs.p;
       a.Wx = g.Wx; a.EY = h->EY; a.EW = h->EW; a.NS = h->NS; a.z_begin = h->owner_z_min;
       a.ghost_row_end = (unsigned)((size_t)h->zs0 * h->EY);
-      a.vtx = h->vtx.p; a.info = h->d_info; a.caps = make_caps(h, ~0ull);
+      a.vtx = h->vtx.p; a.info = h->d_info;
       const int rows = kAssignThreads / 32;
       const dim3 grid((g.Wx + 31) / 32, (h->EY + rows - 1) / rows, nz + 1);
-      if (exact) CU_TRY(h, launch_step(h, k_assign<false>, grid, dim3(kAssignThreads), true, a));
-      else CU_TRY(h, launch_step(h, k_assign<true>, grid, dim3(kAssignThreads), true, a));
+      CU_TRY(h, launch_step(h, k_assign, grid, dim3(kAssignThreads), true, a));
     }
     if (n_blocks > 0) {
       // K3b: points + corner -> id map
@@ -967,17 +970,12 @@ int emit_vertex_stage(cub_handle h, bool exact) {
       VertexArgs a{};
       a.vtx = h->vtx.p; a.caps = make_caps(h, ~0ull); a.write_ghost_points = ghost_points ? 1 : 0;
       a.info = h->d_info;
-      a.n_host = (size_t)(h->ghost_v + h->n_points); a.first_point_host = (size_t)h->ghost_v;
       a.slice_first = si.slice_first; a.block_slice = si.block_slice; a.z_first = h->owner_z_min;
       a.act = h->act.p; a.cofs = h->cofs.p; a.EY = h->EY; a.EW = h->EW;
       a.plane_lo = h->zs0; a.plane_hi = h->zs1; a.geom = h->geom;
       a.coff[0] = (int)(h->i0[0] - h->pad); a.coff[1] = (int)(h->i0[1] - h->pad); a.coff[2] = (int)(h->i0[2] + g.zg0 - h->pad);
       a.points = h->points.p; a.perm = h->perm.p;
-      if (!exact) {
-        if (h->geom.oriented) CU_TRY(h, launch_step(h, k_vertices<true, true>, dim3(n_blocks), dim3(256), true, a));
-        else CU_TRY(h, launch_step(h, k_vertices<false, true>, dim3(n_blocks), dim3(256), true, a));
-      } else if (h->geom.oriented) CU_TRY(h, launch_step(h, k_vertices<true, false>, dim3(n_blocks), dim3(256), true, a));
-      else CU_TRY(h, launch_step(h, k_vertices<false, false>, dim3(n_blocks), dim3(256), true, a));
+      CU_TRY(h, launch_step(h, h->geom.oriented ? k_vertices<true> : k_vertices<false>, dim3(n_blocks), dim3(256), true, a));
     }
   } else {
     // raster order: vertex id = corner slot, points straight from the active masks
@@ -986,13 +984,10 @@ int emit_vertex_stage(cub_handle h, bool exact) {
     a.plane_lo = h->zs0; a.plane_hi = h->zs1;
     a.point_plane_lo = (ghost_points || h->own_z0 == 0) ? h->zs0 : h->zs0 + 1;
     a.coff[0] = (int)(h->i0[0] - h->pad); a.coff[1] = (int)(h->i0[1] - h->pad); a.coff[2] = (int)(h->i0[2] + g.zg0 - h->pad);
-    a.geom = h->geom; a.points = h->points.p; a.info = h->d_info; a.caps = make_caps(h, ~0ull);
+    a.geom = h->geom; a.points = h->points.p; a.info = h->d_info;
     const dim3 grid((unsigned)h->NS, (h->EY + 7) / 8, a.plane_hi - a.plane_lo + 1);
-    if (!exact) {
-      if (h->geom.oriented) k_points_raster<true, true><<<grid, 256, 0, h->stream>>>(a);
-      else k_points_raster<false, true><<<grid, 256, 0, h->stream>>>(a);
-    } else if (h->geom.oriented) k_points_raster<true, false><<<grid, 256, 0, h->stream>>>(a);
-    else k_points_raster<false, false><<<grid, 256, 0, h->stream>>>(a);
+    auto kern = h->geom.oriented ? k_points_raster<true> : k_points_raster<false>;
+    kern<<<grid, 256, 0, h->stream>>>(a);
     h->launches++;
     CU_TRY(h, cudaGetLastError());
   }
@@ -1023,16 +1018,17 @@ int emit_launch(cub_handle h, int id_bytes, bool exact) {
   size_t quads_cap = h->cells.cap / quad_bytes;
   if (mode == kEmitScratchQuads) quads_cap = std::min(quads_cap, h->quads.cap);
   if (cd) quads_cap = std::min(quads_cap, h->celldata.cap / cd_bytes);
-
-  if (h->timing) cudaEventRecord(h->ev[4], h->stream);
-  if (!exact) {
-    // one comparison of the device-side counts with the capacity of the buffers, for every kernel of the emission
-    CU_TRY(h, launch_step(h, k_check_caps, dim3(1), dim3(32), true, h->d_info, make_caps(h, quads_cap)));
-    h->caps_checked = true;
-  }
-  const bool ghost_points = (mode == kEmitScratchQuads) && h->owner_z_min < h->zs0;
   // a second emit of the same count (another id width, new id bases) starts from unprojected points again
   if (proj && h->projected) h->vertices_done = false;
+  // (the check below covers the vertex buffers of a vertex stage that runs with this emission)
+  if (exact && !h->vertices_done) CUB_TRY(size_vertex_buffers(h));
+
+  if (h->timing) cudaEventRecord(h->ev[4], h->stream);
+  // one comparison of the device-side counts with the capacity of the buffers, for every kernel of the emission
+  // (buffers sized from the counts always pass it)
+  CU_TRY(h, launch_step(h, k_check_caps, dim3(1), dim3(32), true, h->d_info, make_caps(h, quads_cap)));
+  h->caps_checked = true;
+  const bool ghost_points = (mode == kEmitScratchQuads) && h->owner_z_min < h->zs0;
   if (!exact || h->n_quads > 0) {
     Timer t(h, 2);
     if (!h->vertices_done) {
@@ -1048,7 +1044,6 @@ int emit_launch(cub_handle h, int id_bytes, bool exact) {
       a.act = h->act.p; a.cofs = h->cofs.p; a.seg = h->seg.p; a.perm = h->raster ? nullptr : h->perm.p;
       a.info = h->d_info;
       a.cells = (mode == kEmitScratchQuads) ? (void*)h->quads.p : (void*)h->cells.p;
-      a.caps = make_caps(h, quads_cap);
       a.mode = mode;
       a.vol = cd ? h->d_vol : nullptr;
       a.vX = h->gv.X; a.vY = h->gv.Y; a.vpad = h->pad; a.vzpad = h->zpad_lo;
@@ -1057,28 +1052,19 @@ int emit_launch(cub_handle h, int id_bytes, bool exact) {
       const dim3 blocks((g.Wx + 31) / 32, (g.Y + kFaceThreads / 32 - 1) / (kFaceThreads / 32), h->zs1 - h->zs0);
       // (behind an event of another stream the launch is an ordinary one: the id base comes from the count exchange)
       const bool pdl = h->wait_before_faces == nullptr;
-      cudaError_t fe = cudaSuccess;
-#define CUB_FACES(IdT, MODE)                                                                                  \
-      do {                                                                                                      \
-        if (!exact) {                                                                                           \
-          if (cd) fe = launch_step(h, k_faces<IdT, MODE, true, true>, blocks, dim3(kFaceThreads), pdl, a);      \
-          else fe = launch_step(h, k_faces<IdT, MODE, false, true>, blocks, dim3(kFaceThreads), pdl, a);        \
-        } else if (cd) fe = launch_step(h, k_faces<IdT, MODE, true, false>, blocks, dim3(kFaceThreads), pdl, a); \
-        else fe = launch_step(h, k_faces<IdT, MODE, false, false>, blocks, dim3(kFaceThreads), pdl, a);         \
-      } while (0)
-      if (mode == kEmitScratchQuads) CUB_FACES(uint32_t, kEmitScratchQuads);
-      else if (mode == kEmitQuads && id_bytes == 4) CUB_FACES(uint32_t, kEmitQuads);
-      else if (mode == kEmitQuads) CUB_FACES(unsigned long long, kEmitQuads);
-      else if (id_bytes == 4) CUB_FACES(uint32_t, kEmitTrisFixed);
-      else CUB_FACES(unsigned long long, kEmitTrisFixed);
-#undef CUB_FACES
-      CU_TRY(h, fe);
+      void (*kern)(FaceArgs);
+      if (mode == kEmitScratchQuads) kern = cd ? k_faces<uint32_t, kEmitScratchQuads, true> : k_faces<uint32_t, kEmitScratchQuads, false>;
+      else if (mode == kEmitQuads && id_bytes == 4) kern = cd ? k_faces<uint32_t, kEmitQuads, true> : k_faces<uint32_t, kEmitQuads, false>;
+      else if (mode == kEmitQuads) kern = cd ? k_faces<unsigned long long, kEmitQuads, true> : k_faces<unsigned long long, kEmitQuads, false>;
+      else if (id_bytes == 4) kern = cd ? k_faces<uint32_t, kEmitTrisFixed, true> : k_faces<uint32_t, kEmitTrisFixed, false>;
+      else kern = cd ? k_faces<unsigned long long, kEmitTrisFixed, true> : k_faces<unsigned long long, kEmitTrisFixed, false>;
+      CU_TRY(h, launch_step(h, kern, blocks, dim3(kFaceThreads), pdl, a));
     }
     t.stop();
   }
   if (proj && (!exact || h->n_points > 0)) {
     Timer t(h, 3);
-    CUB_TRY(launch_project(h, h->points.p, h->points.cap / 3, true, ghost_points, !exact, quads_cap));
+    CUB_TRY(launch_project(h, h->points.p, h->points.cap / 3, true, ghost_points));
     h->projected = true;
     t.stop();
   }
@@ -1087,9 +1073,9 @@ int emit_launch(cub_handle h, int id_bytes, bool exact) {
     const size_t want = exact ? (size_t)h->n_quads : quads_cap;
     const unsigned blocks = (unsigned)std::max<size_t>(1, std::min<size_t>((want + 255) / 256, (size_t)h->num_sms * 16));
     if (id_bytes == 4)
-      k_split_quads<uint32_t><<<blocks, 256, 0, h->stream>>>(h->quads.p, h->points.p, (uint32_t*)h->cells.p, h->d_info, make_caps(h, quads_cap), exact ? 0 : 1);
+      k_split_quads<uint32_t><<<blocks, 256, 0, h->stream>>>(h->quads.p, h->points.p, (uint32_t*)h->cells.p, h->d_info);
     else
-      k_split_quads<unsigned long long><<<blocks, 256, 0, h->stream>>>(h->quads.p, h->points.p, (unsigned long long*)h->cells.p, h->d_info, make_caps(h, quads_cap), exact ? 0 : 1);
+      k_split_quads<unsigned long long><<<blocks, 256, 0, h->stream>>>(h->quads.p, h->points.p, (unsigned long long*)h->cells.p, h->d_info);
     h->launches++;
     CU_TRY(h, cudaGetLastError());
     t.stop();

@@ -30,7 +30,6 @@ struct FaceArgs {
   const uint4* seg;            // [lattice rows][NS] segment bases {vertices, faces, active corners, -}
   const uint32_t* perm;        // slot -> scan-relative vertex id
   unsigned long long* info;    // kInfoMarkF: scan offset of the first own face; kInfoIdDelta: scan-relative vertex id -> final id
-  Caps caps;                   // (GUARD instantiation only)
   void* cells;                 // final cells (IdT) or scratch quads (uint32 scan-relative ids)
   int mode;                    // kEmit*
   const void* vol;             // for cell data (may be null)
@@ -116,15 +115,14 @@ struct FaceSmem {
 // One thread per 32-voxel word computes the face masks; the surface voxels of a warp's 32 words are then
 // compacted into a queue and handled one per lane, so a word with ten surface voxels does not stall the 31
 // lanes whose words have none.
-template <typename IdT, int MODE, bool CD, bool GUARD>
+template <typename IdT, int MODE, bool CD>
 __global__ void __launch_bounds__(kFaceThreads, 12) k_faces(const FaceArgs a) {
   pdl_enter();
   __shared__ FaceSmem sm;
-  // GUARD: the host queued the launch without knowing the counts (cub_emit_async): one check of the device-side
-  // counts against the capacity of the buffers, for the whole kernel.  The counts are requested here and looked at
-  // after the scan, when every other load of the thread has come back too (a branch on them up here would put one
-  // more L2 round trip in front of each of these short-lived blocks).
-  const bool fits = !GUARD || emission_fits(a.info);
+  // The verdict of k_check_caps (the device-side counts fit the buffers) is requested here and looked at after the
+  // scan, when every other load of the thread has come back too (a branch on it up here would put one more L2 round
+  // trip in front of each of these short-lived blocks).
+  const bool fits = emission_fits(a.info);
   const Grid& g = a.g;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   // grid: x = 32-word segments of a row, y = groups of 4 rows (one row per warp), z = own slices.  128-thread CTAs:
@@ -196,7 +194,7 @@ __global__ void __launch_bounds__(kFaceThreads, 12) k_faces(const FaceArgs a) {
     if (lane >= o) s0 += t0;
   }
   const uint32_t total = __shfl_sync(0xffffffffu, s0, 31) & 0xffffu;
-  if (GUARD && !fits) return;
+  if (!fits) return;
   if (total == 0) return;  // no surface voxel in the 1024 voxels of the segment
 
   if (U) {
@@ -268,10 +266,9 @@ __global__ void __launch_bounds__(kFaceThreads, 12) k_faces(const FaceArgs a) {
 // `>=` tie -> first split.
 template <typename IdT>
 __global__ void __launch_bounds__(256) k_split_quads(const uint4* __restrict__ quads, const float* __restrict__ points,
-                                                     IdT* __restrict__ tris, unsigned long long* __restrict__ info,
-                                                     Caps caps, int guard) {
+                                                     IdT* __restrict__ tris, unsigned long long* __restrict__ info) {
   // the number of quads and the id offset come from the device-side run info (no host round trip needed)
-  if (guard && !emission_fits(info)) return;
+  if (!emission_fits(info)) return;
   const size_t n_quads = (size_t)__ldg(info + kInfoQuads);
   const unsigned long long id_delta = __ldg(info + kInfoIdDelta);
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_quads; i += (size_t)gridDim.x * blockDim.x) {

@@ -32,10 +32,9 @@ struct ProjArgs {
   unsigned max_steps;
   float* points;
   size_t n_points;           // number of points (info == null)
-  unsigned long long* info;  // when set: the points are [ghost ? 0 : info[kInfoGhostV], info[kInfoGhostV] + info[kInfoPoints])
+  unsigned long long* info;  // when set: the points are [ghost ? 0 : info[kInfoGhostV], info[kInfoGhostV] + info[kInfoPoints]),
+                             // and nothing is projected unless k_check_caps found that the emission fits its buffers
   int include_ghost;
-  int guard;                 // queued before the host knew the counts: check them against caps first
-  Caps caps;
   long long i0[3];           // image index of buffer voxel (0, 0, 0) (cub_set_region_index): continuous indices are image indices
   unsigned long long* work;  // device counter (zeroed before the launch): next vertex to hand out
   unsigned refill;           // lanes of a warp that must still be iterating for the warp to skip the service phase (1..32)
@@ -119,7 +118,7 @@ __global__ void __launch_bounds__(128, ORIENTED ? 5 : 6) k_project(const ProjArg
   size_t n_points = a.n_points;
   float* const points = a.points + (a.info && !a.include_ghost ? 3 * (size_t)__ldg(a.info + kInfoGhostV) : 0);
   if (a.info) {
-    if (a.guard && !emission_fits(a.info)) return;
+    if (!emission_fits(a.info)) return;
     const size_t ghost = (size_t)__ldg(a.info + kInfoGhostV);
     const size_t all = ghost + (size_t)__ldg(a.info + kInfoPoints);
     n_points = a.include_ghost ? all : all - ghost;
@@ -452,7 +451,7 @@ __global__ void __launch_bounds__(128) k_project_alt(const ProjArgs a, int metho
   size_t n_points = a.n_points;
   float* const points = a.points + (a.info && !a.include_ghost ? 3 * (size_t)__ldg(a.info + kInfoGhostV) : 0);
   if (a.info) {
-    if (a.guard && !emission_fits(a.info)) return;
+    if (!emission_fits(a.info)) return;
     const size_t ghost = (size_t)__ldg(a.info + kInfoGhostV);
     const size_t all = ghost + (size_t)__ldg(a.info + kInfoPoints);
     n_points = a.include_ghost ? all : all - ghost;

@@ -50,19 +50,20 @@ enum {
   kInfoFlags = 12,                                  // bit 0: a result buffer was too small; bit 1: an interior slice of the range is empty
   kInfoWork = 13,                                   // work counter of the projection kernel
   kInfoSplitWork = 14,
-  kInfoFits = 15,                                   // written by k_check_caps: the queued emission fits its buffers
+  kInfoFits = 15,                                   // written by k_check_caps: the emission fits its buffers
   kInfoWords = 16
 };
 enum { kFlagBufferOverflow = 1, kFlagEmptyInteriorSlice = 2, kFlagIdOverflow = 4 };
 
-// Capacities of the result buffers, for launches queued before the host knows the counts (cub_emit_async): every
-// emission kernel compares them with the device-side counts ONCE, at its start, and the whole emission is skipped
-// (and flagged: cub_finish redoes it with larger buffers) if anything would not fit - no per-item checks.
+// Capacities of the result buffers.  k_check_caps compares them with the device-side counts ONCE per emission, and
+// every emission kernel reads its verdict: the whole emission is skipped (and flagged: cub_finish redoes it with
+// larger buffers) if anything would not fit - no per-item checks.  An emission queued before the host knows the
+// counts (cub_emit_async) can fail the check; one whose buffers were sized from the counts always passes it.
 struct Caps {
   unsigned long long points, perm, quads;
   int raster;
 };
-// one thread, queued in front of an emission whose host does not know the counts: the verdict every GUARD kernel reads
+// one thread, queued in front of every emission: the verdict every emission kernel reads
 __global__ void k_check_caps(unsigned long long* info, Caps c) {
   pdl_enter();
   if (threadIdx.x != 0 || blockIdx.x != 0) return;

@@ -25,6 +25,9 @@
 //
 // In raster vertex order (the opt-in canonical order) ids ARE slots and k_points_raster writes the points
 // straight from the active masks.
+//
+// k_assign, k_vertices and k_points_raster skip their work when k_check_caps found that the emission does not fit
+// its buffers (k_segscan.cuh).
 #pragma once
 #include "cbr_common.cuh"
 #include "k_segscan.cuh"
@@ -41,17 +44,15 @@ struct AssignArgs {
   unsigned ghost_row_end; // active corners of lattice rows below this one are not counted (the slab underneath owns them)
   uint32_t* vtx;          // [n vertices] cx | cy << 16 | oz << 31
   unsigned long long* info;
-  Caps caps;              // (GUARD instantiation only)
 };
 
 constexpr int kAssignThreads = 128;  // (one row segment per warp)
 
 // grid: x = 32-word segments of a voxel row, y = groups of kAssignThreads / 32 lattice rows (one row per warp),
 // z = planes of the scan range (one more than its voxel slices: the top corner plane)
-template <bool GUARD>
 __global__ void __launch_bounds__(kAssignThreads) k_assign(const AssignArgs a) {
   pdl_enter();
-  const bool fits = !GUARD || emission_fits(a.info);  // (looked at after the scan: see k_faces)
+  const bool fits = emission_fits(a.info);  // (looked at after the scan: see k_faces)
   const int lane = threadIdx.x & 31;
   const int w = blockIdx.x * 32 + lane, y = blockIdx.y * (kAssignThreads / 32) + (threadIdx.x >> 5), z = a.z_begin + blockIdx.z;
   if (y >= a.EY) return;  // (warp-uniform)
@@ -74,7 +75,7 @@ __global__ void __launch_bounds__(kAssignThreads) k_assign(const AssignArgs a) {
     if (lane >= o) incl += t;
   }
   const uint32_t excl = incl - (nv | (na << 16));
-  if (GUARD && !fits) return;
+  if (!fits) return;
   if (w < a.EW) a.cofs[e] = sb.z + (excl >> 16);
   // the corner column past the last voxel word of the row, when it starts a segment of its own (X a multiple of 1024):
   // it is the first word of that segment, its slot base is the segment base (the words after it are padding)
@@ -108,9 +109,8 @@ struct VertexArgs {
   const uint32_t* vtx;      // [n] packed corner of vertex id (scan-relative id): cx | cy << 16 | oz << 31
   const uint32_t* slice_first;  // [nz + 1] first id created by slice z_first + k; [nz] = UINT_MAX   (k_slice_index)
   const uint32_t* block_slice;  // [blocks of this launch] k of the block's first id                  (k_slice_index)
-  unsigned long long* info;  // GUARD: kInfoTotV = ghost vertices + own vertices, kInfoGhostV; else n_host / first_point_host hold them
-  size_t n_host, first_point_host;
-  Caps caps;                // (GUARD instantiation only)
+  unsigned long long* info;  // kInfoTotV = ghost vertices + own vertices, kInfoGhostV
+  Caps caps;                // caps.points bounds the record loads issued before the counts are known
   int z_first;              // first local slice of the scan range
   int write_ghost_points;   // also write the points of the vertices that belong to the slab underneath
   const uint32_t* act;      // entry lattice [Zl+1][EY][EW]
@@ -153,34 +153,24 @@ __global__ void __launch_bounds__(256) k_slice_index(const SliceIndexArgs a) {
 constexpr int kVertexPerThread = 4;                       // ids per thread: the loads of the 4 are in flight together
 constexpr int kVertexBlockIds = 256 * kVertexPerThread;   // (the kernel is a chain of 3 dependent loads otherwise)
 
-// GUARD: launched by cub_emit_async without the host knowing the counts (they are read from the device, every write
-// is checked against the capacity of its buffer)
-template <bool ORIENTED, bool GUARD>
+// The number of vertices comes from the device-side run info: the grid may be sized for the buffers' capacity
+// (cub_emit_async), and the blocks past the count return.
+template <bool ORIENTED>
 __global__ void __launch_bounds__(256, ORIENTED ? 4 : 8) k_vertices(const VertexArgs a) {
   pdl_enter();
-  // GUARD: the number of vertices comes from the device-side run info (the grid is sized for the buffers' capacity)
   const size_t id0 = (size_t)blockIdx.x * kVertexBlockIds + threadIdx.x;
   uint32_t v[kVertexPerThread];
-  if (GUARD) {
-    // the records are requested before the counts are looked at (any id below the capacity of the buffer is safe
-    // to read), so that the two round trips overlap
+  // the records are requested before the counts are looked at (any id below the capacity of the buffer is safe
+  // to read), so that the two round trips overlap
 #pragma unroll
-    for (int j = 0; j < kVertexPerThread; ++j) {
-      const size_t id = id0 + (size_t)j * 256;
-      v[j] = id < a.caps.points ? __ldcs(a.vtx + id) : 0u;
-    }
-    if (!emission_fits(a.info)) return;
+  for (int j = 0; j < kVertexPerThread; ++j) {
+    const size_t id = id0 + (size_t)j * 256;
+    v[j] = id < a.caps.points ? __ldcs(a.vtx + id) : 0u;
   }
-  const size_t n = GUARD ? (size_t)__ldg(a.info + kInfoTotV) : a.n_host;
+  if (!emission_fits(a.info)) return;
+  const size_t n = (size_t)__ldg(a.info + kInfoTotV);
   if ((size_t)blockIdx.x * kVertexBlockIds >= n) return;
-  const size_t first_point = a.write_ghost_points ? 0 : (GUARD ? (size_t)__ldg(a.info + kInfoGhostV) : a.first_point_host);
-  if (!GUARD) {
-#pragma unroll
-    for (int j = 0; j < kVertexPerThread; ++j) {
-      const size_t id = id0 + (size_t)j * 256;
-      v[j] = id < n ? __ldcs(a.vtx + id) : 0u;
-    }
-  }
+  const size_t first_point = a.write_ghost_points ? 0 : (size_t)__ldg(a.info + kInfoGhostV);
   int lo = (int)__ldg(a.block_slice + blockIdx.x);
   int cz[kVertexPerThread];
 #pragma unroll
@@ -235,12 +225,11 @@ struct RasterPointArgs {
   Geom geom;
   float* points;            // indexed by slot
   unsigned long long* info;
-  Caps caps;                // (GUARD instantiation only)
 };
 
-template <bool ORIENTED, bool GUARD>
+template <bool ORIENTED>
 __global__ void __launch_bounds__(256) k_points_raster(const RasterPointArgs a) {
-  if (GUARD && !emission_fits(a.info)) return;
+  if (!emission_fits(a.info)) return;
   // grid: x = 32-word segments of a corner row, y = groups of 8 rows (one per warp), z = planes
   const int lane = threadIdx.x & 31;
   const int w = blockIdx.x * 32 + lane, cy = blockIdx.y * 8 + (threadIdx.x >> 5), cz = a.plane_lo + blockIdx.z;

@@ -513,24 +513,68 @@ def test_emit_twice_gives_the_same_mesh():
     h.close()
 
 
+# the emit modes of the synchronous tests above, each with the volumes and the oracle comparison of its test
+ASYNC_MODES = {
+    "quads_u32": dict(volume="noise", tri=False, proj=False),
+    "quads_u64": dict(volume="noise", tri=False, proj=False, id_bytes=8),
+    "triangles_fixed_split": dict(volume="noise", tri=True, proj=False),
+    "triangles_projected": dict(volume="smooth", tri=True, proj=True),
+    "cell_data": dict(volume="smooth_i16", tri=True, proj=True, cell_data=True),
+    "raster_order": dict(volume="noise", tri=False, proj=False, cell_data=True, raster=True),
+    "oriented": dict(volume="smooth", tri=True, proj=True, direction="oblique"),
+}
+
+
 def test_async_pipeline_matches_and_survives_a_larger_second_run():
     """cub_count_async / cub_emit_async / cub_finish: buffers sized by a small first run, then a larger volume on the same
     handle overflows them on the device; cub_finish must redo the emission and return the complete mesh"""
+    check_async_pipeline("triangles_projected")
+
+
+@pytest.mark.parametrize("mode", sorted(set(ASYNC_MODES) - {"triangles_projected"}))
+def test_async_pipeline_in_the_other_emit_modes(mode):
+    """the same small / overflowing / smaller runs through cub_emit_async in every other emit mode"""
+    check_async_pipeline(mode)
+
+
+def check_async_pipeline(mode):
     O, P = oracle(), pkg()
-    h = P.capi.Handle(0)
+    m = ASYNC_MODES[mode]
+    tri, proj, cd, raster, id_bytes = m["tri"], m["proj"], m.get("cell_data", False), m.get("raster", False), m.get("id_bytes", 4)
+    kw = dict(triangles=tri, project=proj, cell_data=cd, thr=0.02)
     p = P.capi.default_params()
-    p.generate_triangles, p.project_vertices, p.surface_distance_threshold = 1, 1, 0.02
+    p.generate_triangles, p.project_vertices, p.save_pixel_as_cell_data = int(tri), int(proj), int(cd)
+    p.surface_distance_threshold = kw["thr"]
+    if raster:
+        p.vertex_order = P.capi.ORDER_RASTER
+    geo = {}
+    if "direction" in m:  # the image and projection arguments of test_direction_matrices
+        geo = dict(spacing=(0.5, 1.25, 2.0), origin=(3.0, -2.0, 7.0), direction=DIRECTIONS[m["direction"]])
+        kw.update(step=0.24, relax=0.95, max_steps=80)
+        p.step_length, p.step_relaxation, p.max_steps = kw["step"], kw["relax"], kw["max_steps"]
+    h = P.capi.Handle(0)
     for shape, seed in [((10, 12, 33), 1), ((30, 40, 70), 2), ((30, 40, 70), 3), ((12, 9, 20), 4)]:
-        vol, iso = smooth_volume(shape, np.float32, seed=seed)
+        if m["volume"] == "noise":
+            vol, iso = random_volume(shape, np.uint8, seed=seed)
+        else:
+            vol, iso = smooth_volume(shape, np.int16 if m["volume"] == "smooth_i16" else np.float32, seed=seed)
         p.iso_value = float(iso)
-        h.set_volume(vol)
+        h.set_volume(vol, **geo)
         h.count_async(p)
-        h.emit_async(4)
+        h.emit_async(id_bytes)
         n_pts, n_cells = h.finish()
-        ref = O.cuberille(vol, iso, triangles=True, project=True, thr=0.02)
+        mode_args = dict(mode=O.CLOSED_FORM) if m["volume"] == "noise" or geo else {}
+        ref = O.cuberille(vol, iso, **mode_args, **geo, **kw)
         assert (n_pts, n_cells) == (ref.points.shape[0], ref.cells.shape[0])
-        a, b, _ = h.fetch()
-        assert_mesh_equal(P.Mesh(a, b), ref, f"async {shape}")
+        a, b, c = h.fetch(want_cell_data=cd)
+        mesh = P.Mesh(a, b, c)
+        if raster:
+            assert_mesh_equal_up_to_vertex_order(mesh, ref, mesh, ref, f"async {mode} {shape}")
+        else:
+            assert_mesh_equal(mesh, ref, f"async {mode} {shape}")
+        assert b.dtype == (np.uint64 if id_bytes == 8 else np.uint32)
+        if cd:
+            assert c.dtype == vol.dtype
     h.close()
 
 
