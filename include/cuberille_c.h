@@ -112,7 +112,10 @@ const char *cub_last_error(cub_handle h);
  *   data      : x-fastest voxel buffer of dims[0]*dims[1]*dims[2] pixels
  *   mem_kind  : CUB_MEM_HOST -> copied to the device on the handle's stream;
  *               CUB_MEM_DEVICE -> borrowed (must stay valid until the next
- *               cub_set_volume / cub_destroy), no copy
+ *               cub_set_volume / cub_destroy), no copy; the pointer must be
+ *               aligned to the pixel size (else CUB_ERR_INVALID).  Any such
+ *               offset is accepted: the kernels that need a 4- or 16-byte
+ *               aligned buffer give way to others when it is not.
  *   direction : row-major 3x3 direction cosines (itk::ImageBase::GetDirection), or
  *               NULL = identity.  The identity is the non-oriented image every test
  *               of the reference has.  Any other (non-singular) matrix gives the

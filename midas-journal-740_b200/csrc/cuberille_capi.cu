@@ -14,8 +14,10 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/cuberille_c.h"
@@ -241,10 +243,19 @@ int pixel_bytes(int dtype) {
     default: break;                                          \
   }
 
-// (double)(T)iso : m_IsoSurfaceValue is an InputPixelType (h:326)
+// (double)(T)iso : m_IsoSurfaceValue is an InputPixelType (h:326).  An iso outside an integer T's range (or NaN) has
+// no such value, and converting it to T would be undefined behaviour: it comes back as NaN, which equals no iso.
+template <typename T>
+double iso_in_type(double iso) {
+  if (std::is_integral<T>::value &&
+      !(iso >= (double)std::numeric_limits<T>::min() && iso <= (double)std::numeric_limits<T>::max()))
+    return std::numeric_limits<double>::quiet_NaN();
+  return (double)(T)iso;
+}
+
 double iso_as_pixel(int dtype, double iso) {
   double r = iso;
-  DISPATCH_PIXEL(dtype, r = (double)(T)iso);
+  DISPATCH_PIXEL(dtype, r = iso_in_type<T>(iso));
   return r;
 }
 
@@ -631,6 +642,9 @@ int cub_set_volume(cub_handle h, const void* data, int dtype, const uint64_t dim
   CUB_TRY(set_geometry(h, dtype, dims, spacing, origin, direction));
   const size_t bytes = (size_t)dims[0] * dims[1] * dims[2] * h->pix_bytes;
   if (mem_kind == CUB_MEM_DEVICE) {
+    // every kernel loads whole pixels from the borrowed buffer
+    if (reinterpret_cast<uintptr_t>(data) % (uintptr_t)h->pix_bytes != 0)
+      return fail(h, CUB_ERR_INVALID, "device volume pointer %p is not aligned to the %d-byte pixel", data, h->pix_bytes);
     h->d_vol = data;
   } else if (mem_kind == CUB_MEM_HOST) {
     CUB_TRY(ensure(h, h->vol_owned, bytes));

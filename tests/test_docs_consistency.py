@@ -21,6 +21,27 @@ def test_every_tuning_knob_is_documented_and_read_once():
         assert name in create, f"{name} is not read in cub_create"
 
 
+def test_every_switch_the_tests_and_tools_set_is_read_by_the_library():
+    """a test that sets a variable the library no longer reads runs the same path twice and checks nothing"""
+    src = open(CAPI).read()
+    read = set(re.findall(r'env_int\("(CUB_[A-Z0-9_]+)"', src))
+    api = set(re.findall(r"\bCUB_[A-Z0-9_]+\b", open(os.path.join(ROOT, "include", "cuberille_c.h")).read()))
+    allowed = {"CUB_FORCE_BUILD"}  # read by __graft_entry__.build(), not by the library
+    named = {}
+    for top in ("tests", "tools"):
+        for d, _, files in os.walk(os.path.join(ROOT, top)):
+            for f in files:
+                path = os.path.join(d, f)
+                if path == os.path.abspath(__file__) or not f.endswith((".py", ".sh", ".md", ".cxx", ".txt")):
+                    continue  # (this file names switches that must not exist)
+                for name in re.findall(r"\bCUB_[A-Z0-9_]+\b", open(path, errors="replace").read()):
+                    named.setdefault(name, os.path.relpath(path, ROOT))
+    switches = {n: p for n, p in named.items() if n not in api}
+    assert "CUB_FUSE" in switches and "CUB_K1_PACKED" in switches
+    stale = {n: p for n, p in switches.items() if n not in read and n not in allowed}
+    assert not stale, f"variables named under tests/ or tools/ that cuberille_capi.cu does not read: {stale}"
+
+
 def test_fused_kernel_has_no_debug_switch_left():
     src = open(CAPI).read() + open(os.path.join(ROOT, "midas-journal-740_b200", "csrc", "k_fused.cuh")).read()
     assert "CUB_FUSE_DBG" not in src and "dbg" not in src

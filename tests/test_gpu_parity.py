@@ -144,18 +144,6 @@ def test_buffered_region_with_a_nonzero_index(tri, proj, border):
     assert not np.array_equal(ref0.points, ref.points)
 
 
-def test_assign_by_second_sweep_gives_the_same_mesh(monkeypatch):
-    """CUB_ASSIGN_SWEEP=1: K3a recomputes the ownership masks in a second sweep instead of reading the ones K2a
-    stored (32 B of scratch per lattice entry less)"""
-    O = oracle()
-    vol, iso = random_volume((17, 20, 97), np.uint8, seed=5, fill=0.4)
-    ref = O.cuberille(vol, iso, triangles=False, project=False, mode=O.CLOSED_FORM)
-    monkeypatch.setenv("CUB_ASSIGN_SWEEP", "1")
-    assert_mesh_equal(run_filter(vol, iso, triangles=False, project=False), ref, "second sweep")
-    monkeypatch.delenv("CUB_ASSIGN_SWEEP")
-    assert_mesh_equal(run_filter(vol, iso, triangles=False, project=False), ref, "stored masks")
-
-
 def test_sizes_beyond_the_corner_record_are_refused():
     P = pkg()
     h = P.capi.Handle(0)
