@@ -138,6 +138,21 @@ int cub_set_volume(cub_handle h, const void *data, int dtype, const uint64_t dim
  * WHOLE image's first voxel.                                                   */
 int cub_set_region_index(cub_handle h, const int64_t index[3]);
 
+/* Inside-range mode (no counterpart in the reference): with enable != 0 a
+ * voxel is inside when !(v < lower) && !(upper < v), compared in the pixel
+ * type, instead of !(v < iso_value).  A label k of a label map is the range
+ * [k, k]; a range of several labels meshes the surface of their union, and with
+ * save_pixel_as_cell_data every cell carries the value of the voxel that made
+ * it.  A NaN pixel is inside, as in iso mode.  [iso, type maximum] (or +inf)
+ * gives the mask of iso mode with that iso.  Both bounds must be pixel values
+ * of the current volume's type (the rule cub_count applies to iso_value), not
+ * NaN, and lower <= upper; else CUB_ERR_INVALID.  While the mode is on,
+ * cub_params.iso_value is ignored, and cub_count / cub_count_async with
+ * project_vertices != 0 and cub_debug_project_points return CUB_ERR_INVALID:
+ * the projection needs an iso-surface.  enable == 0 returns to iso mode.
+ * Call after cub_set_volume, which turns the mode off.                         */
+int cub_set_inside_range(cub_handle h, int enable, double lower, double upper);
+
 /* z-slab decomposition (no counterpart in the reference: GenerateData is a
  * single raster loop txx:136-206; concatenating z-slabs preserves its order).
  *   image_nz      : z size of the WHOLE image

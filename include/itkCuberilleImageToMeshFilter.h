@@ -181,6 +181,33 @@ public:
   itkSetMacro( ImageBorderFaces, bool );
   itkBooleanMacro( ImageBorderFaces );
 
+  /** Extension (off by default): mesh the voxels whose value lies in [lower, upper] instead of those >= the iso value
+   * (cub_set_inside_range).  A label k of a label map is SetLabelValue( k ) = the range [k, k]; a range of several labels
+   * gives the surface of their union.  The projection needs an iso-surface, so Update() throws while a range is set and
+   * ProjectVerticesToIsoSurface is on (the constructor default). */
+  void SetInsideRange( InputPixelType lower, InputPixelType upper )
+    {
+    if ( !m_InsideRangeOn || m_InsideRangeLower != lower || m_InsideRangeUpper != upper )
+      {
+      m_InsideRangeOn = true;
+      m_InsideRangeLower = lower;
+      m_InsideRangeUpper = upper;
+      this->Modified();
+      }
+    }
+  void SetLabelValue( InputPixelType label ) { this->SetInsideRange( label, label ); }
+  void InsideRangeOff()
+    {
+    if ( m_InsideRangeOn )
+      {
+      m_InsideRangeOn = false;
+      this->Modified();
+      }
+    }
+  itkGetMacro( InsideRangeOn, bool );
+  itkGetMacro( InsideRangeLower, InputPixelType );
+  itkGetMacro( InsideRangeUpper, InputPixelType );
+
   /** Projection knobs with the reference's clamp ranges (h:209-228). */
   itkGetMacro( ProjectVertexSurfaceDistanceThreshold, double );
   itkSetClampMacro( ProjectVertexSurfaceDistanceThreshold, double, 0.0, NumericTraits<InputPixelType>::max() );
@@ -222,6 +249,9 @@ protected:
     m_SavePixelAsCellData = false;
     m_RasterVertexOrder = false;
     m_ImageBorderFaces = false;
+    m_InsideRangeOn = false;
+    m_InsideRangeLower = NumericTraits< InputPixelType >::One;
+    m_InsideRangeUpper = NumericTraits< InputPixelType >::One;
     m_ProjectVertexSurfaceDistanceThreshold = 0.5;
     m_ProjectVertexStepLength = -1.0;
     m_ProjectVertexStepLengthRelaxationFactor = 0.95;
@@ -253,6 +283,9 @@ protected:
     os << indent << "GenerateTriangleFaces: " << m_GenerateTriangleFaces << std::endl;
     os << indent << "ProjectVerticesToIsoSurface: " << m_ProjectVerticesToIsoSurface << std::endl;
     os << indent << "SavePixelAsCellData: " << m_SavePixelAsCellData << std::endl;
+    os << indent << "InsideRange: " << m_InsideRangeOn << " ["
+       << static_cast< typename NumericTraits<InputPixelType>::PrintType >( m_InsideRangeLower ) << ", "
+       << static_cast< typename NumericTraits<InputPixelType>::PrintType >( m_InsideRangeUpper ) << "]" << std::endl;
     }
 
   virtual void GenerateOutputInformation() { } // do nothing (h:236)
@@ -307,6 +340,16 @@ protected:
                                  cuberille_detail::PixelCode<InputPixelType>::value,
                                  dims, spacing, origin, direction, CUB_MEM_HOST ) );
     this->Check( cub_set_region_index( m_Handle, regionIndex ) );
+    if ( m_InsideRangeOn )
+      {
+      if ( m_ProjectVerticesToIsoSurface )
+        {
+        itkExceptionMacro( << "an inside range has no iso-surface to project the vertices onto: call "
+                           "ProjectVerticesToIsoSurfaceOff() (projection is on by default)" );
+        }
+      this->Check( cub_set_inside_range( m_Handle, 1, static_cast<double>( m_InsideRangeLower ),
+                                         static_cast<double>( m_InsideRangeUpper ) ) );
+      }
     this->Check( cub_synchronize( m_Handle ) );
     const Clock::time_point t1 = Clock::now();
     cub_params params;
@@ -422,6 +465,9 @@ private:
   bool                m_SavePixelAsCellData;
   bool                m_RasterVertexOrder;
   bool                m_ImageBorderFaces;
+  bool                m_InsideRangeOn;
+  InputPixelType      m_InsideRangeLower;
+  InputPixelType      m_InsideRangeUpper;
   double              m_ProjectVertexSurfaceDistanceThreshold;
   double              m_ProjectVertexStepLength;
   double              m_ProjectVertexStepLengthRelaxationFactor;

@@ -27,7 +27,7 @@ CODE_DTYPES = {v: k for k, v in DTYPE_CODES.items()}
 # every symbol include/cuberille_c.h declares (tests check that the library exports all of them)
 SYMBOLS = [
     "cub_abi_version", "cub_default_params", "cub_create", "cub_destroy", "cub_last_error", "cub_set_volume",
-    "cub_set_region_index", "cub_set_slab", "cub_count", "cub_set_id_base", "cub_emit_vertices", "cub_emit", "cub_run", "cub_fetch", "cub_fetch_async",
+    "cub_set_region_index", "cub_set_inside_range", "cub_set_slab", "cub_count", "cub_set_id_base", "cub_emit_vertices", "cub_emit", "cub_run", "cub_fetch", "cub_fetch_async",
     "cub_synchronize", "cub_device_buffers",
     "cub_debug_bitmask", "cub_debug_project_points", "cub_generate_volume", "cub_download_volume",
     "cub_enable_timing", "cub_get_timings", "cub_launch_count", "cub_count_was_fused",
@@ -91,6 +91,8 @@ def load() -> C.CDLL:
     L.cub_set_volume.argtypes = [vp, vp, i, pu64, pd, pd, pd, i]
     L.cub_set_region_index.restype = i
     L.cub_set_region_index.argtypes = [vp, C.POINTER(C.c_int64)]
+    L.cub_set_inside_range.restype = i
+    L.cub_set_inside_range.argtypes = [vp, i, C.c_double, C.c_double]
     L.cub_set_slab.restype = i
     L.cub_set_slab.argtypes = [vp, u64, u64, u64, u64]
     L.cub_count.restype = i
@@ -236,6 +238,16 @@ class Handle:
     def set_region_index(self, index_xyz):
         """Image index of the buffer's first voxel (after set_volume, which resets it to 0)."""
         self._check(self._L.cub_set_region_index(self._h, (C.c_int64 * 3)(*[int(v) for v in index_xyz])))
+
+    def set_inside_range(self, lower, upper):
+        """Range mode: a voxel is inside when lower <= v <= upper in the pixel type (NaN pixels too), instead of
+        v >= iso.  Both bounds must be pixel values of the volume's type; a label k is (k, k).  Projection is refused
+        while the mode is on.  After set_volume, which turns the mode off."""
+        self._check(self._L.cub_set_inside_range(self._h, 1, float(lower), float(upper)))
+
+    def clear_inside_range(self):
+        """Back to iso mode."""
+        self._check(self._L.cub_set_inside_range(self._h, 0, 0.0, 0.0))
 
     def set_slab(self, image_nz: int, local_z0: int, own_z0: int, own_z1: int):
         self._check(self._L.cub_set_slab(self._h, image_nz, local_z0, own_z0, own_z1))

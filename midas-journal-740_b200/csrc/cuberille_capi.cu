@@ -117,6 +117,9 @@ struct cub_handle_s {
   uint64_t dims[3] = {0, 0, 0};
   Geom geom{};
   bool has_volume = false;
+  // inside-range mode (cub_set_inside_range): inside == !(v < range_lo) && !(range_hi < v) instead of !(v < iso)
+  bool range_on = false;
+  double range_lo = 0.0, range_hi = 0.0;
   // slab
   uint64_t image_nz = 0, local_z0 = 0, own_z0 = 0, own_z1 = 0;
   bool slab_set = false;
@@ -303,12 +306,14 @@ template <> struct is_packable<int16_t> { static constexpr bool value = true; };
 
 template <typename T, bool PACK = is_packable<T>::value>
 struct ClassifyPacked {
-  static bool launch(cub_handle, const T*, uint32_t*, const Grid&, unsigned long long, unsigned long long, cudaStream_t) { return false; }
+  template <typename In>
+  static bool launch(cub_handle, In, const T*, uint32_t*, const Grid&, unsigned long long, unsigned long long, cudaStream_t) { return false; }
 };
 template <typename T>
 struct ClassifyPacked<T, true> {
   // 4 bytes per lane per load (k_classify_packed): rows must be whole warp loads and the buffer 4-byte aligned
-  static bool launch(cub_handle h, const T* vol, uint32_t* bits, const Grid& g, unsigned long long rows,
+  template <typename In>
+  static bool launch(cub_handle h, In inside, const T* vol, uint32_t* bits, const Grid& g, unsigned long long rows,
                      unsigned long long max_blocks, cudaStream_t stream) {
     constexpr int vpl = 4 / (int)sizeof(T);
     if (g.X % (32 * vpl) != 0 || (reinterpret_cast<uintptr_t>(vol) & 3u) != 0 || h->knobs.k1_packed == 0) return false;
@@ -316,13 +321,20 @@ struct ClassifyPacked<T, true> {
     const unsigned long long tasks = rows * tasks_per_row;  // cub_count checks rows * groups < 2^32
     unsigned long long blocks = std::min<unsigned long long>((tasks + 7) / 8, max_blocks);
     if (blocks < 1) blocks = 1;
-    k_classify_packed<T><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, g, (T)h->params.iso_value, (unsigned)tasks, tasks_per_row);
+    k_classify_packed<T, In><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, g, inside.param(), (unsigned)tasks, tasks_per_row);
     return true;
   }
 };
 
-template <typename T>
-void launch_classify(cub_handle h, int z0, int z1, cudaStream_t stream, int ctas_per_sm) {
+// The inside predicate of the handle's mode, in the pixel type, handed to f: every classification route is instantiated
+// for both (k_classify.cuh), and iso mode keeps its own instantiations rather than running as a range.
+template <typename T, typename F>
+auto with_inside(cub_handle h, F&& f) {
+  return h->range_on ? f(Between<T>{(T)h->range_lo, (T)h->range_hi}) : f(AtLeast<T>{(T)h->params.iso_value});
+}
+
+template <typename T, typename In>
+void launch_classify(cub_handle h, In inside, int z0, int z1, cudaStream_t stream, int ctas_per_sm) {
   const unsigned long long max_blocks = (unsigned long long)h->num_sms * ctas_per_sm;
   h->launches++;
   if (h->pad) {
@@ -335,8 +347,8 @@ void launch_classify(cub_handle h, int z0, int z1, cudaStream_t stream, int ctas
     // slice z0 of the launch is lattice slice z0: the kernel's z origin moves with it
     const T* vol = static_cast<const T*>(h->d_vol);
     Grid sub = gb;
-    k_classify_padded<T><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, sub, gv.X, gv.Y, gv.Zl, h->zpad_lo - z0,
-                                                                (T)h->params.iso_value, (unsigned)words);
+    k_classify_padded<T, In><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, sub, gv.X, gv.Y, gv.Zl, h->zpad_lo - z0,
+                                                                    inside.param(), (unsigned)words);
     return;
   }
   Grid g = h->g;
@@ -349,19 +361,19 @@ void launch_classify(cub_handle h, int z0, int z1, cudaStream_t stream, int ctas
   const bool full = (g.X % 32 == 0) && (g.Wx % kWordsPerTask == 0);
   const T* vol = static_cast<const T*>(h->d_vol) + (size_t)z0 * g.Y * g.X;
   uint32_t* bits = h->bits.p + (size_t)z0 * g.Y * g.Wp;
-  if (ClassifyPacked<T>::launch(h, vol, bits, g, rows, max_blocks, stream)) return;
+  if (ClassifyPacked<T>::launch(h, inside, vol, bits, g, rows, max_blocks, stream)) return;
   if (full)
-    k_classify<T, true><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, g, (T)h->params.iso_value, tasks, groups);
+    k_classify<T, true, In><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, g, inside.param(), tasks, groups);
   else
-    k_classify<T, false><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, g, (T)h->params.iso_value, tasks, groups);
+    k_classify<T, false, In><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, g, inside.param(), tasks, groups);
 }
 
 // K1 + K2a as one kernel (k_fused.cuh).  Returns false (nothing launched) where the fused kernel does not apply: the
 // caller then runs the two kernels one after the other.
 constexpr int kFuseStages = 3;
 
-template <typename T, typename C>
-bool launch_fused_cfg(cub_handle h, const SweepArgs& ca, unsigned* ctr, unsigned* done) {
+template <typename T, typename C, typename In>
+bool launch_fused_cfg(cub_handle h, In inside, const SweepArgs& ca, unsigned* ctr, unsigned* done) {
   using Smem = FuseSmem<C, kFuseStages>;
   constexpr int WPT = kFuseStageBytes / (32 * (int)sizeof(T));
   const Grid& g = ca.g;
@@ -388,7 +400,7 @@ bool launch_fused_cfg(cub_handle h, const SweepArgs& ca, unsigned* ctr, unsigned
   if (tiles >= (1ull << 31)) return false;
   fa.n_tiles = (unsigned)tiles; fa.gx = (unsigned)gx; fa.gy = (unsigned)gy;
   fa.ctr = ctr; fa.done = done;
-  auto kern = k_classify_sweep<T, C, kFuseStages>;
+  auto kern = k_classify_sweep<T, C, kFuseStages, In>;
   // (set on every launch: the attribute belongs to the current device, and one process may drive several)
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)) != cudaSuccess) {
     cudaGetLastError();
@@ -397,13 +409,13 @@ bool launch_fused_cfg(cub_handle h, const SweepArgs& ca, unsigned* ctr, unsigned
   // persistent: every CTA resident (4 per SM: 64 registers x 256 threads, ~47 KB of shared memory)
   const unsigned long long want = std::max<unsigned long long>((fa.n_batches + 3) / 4, fa.n_tiles);
   const unsigned blocks = (unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>(want, (unsigned long long)h->num_sms * h->knobs.fuse_ctas));
-  kern<<<blocks, kFuseThreads, sizeof(Smem), h->stream>>>(fa, (T)h->params.iso_value);
+  kern<<<blocks, kFuseThreads, sizeof(Smem), h->stream>>>(fa, inside.param());
   h->launches++;
   return true;
 }
 
-template <typename T>
-bool launch_fused(cub_handle h, const SweepArgs& ca, int cfg, unsigned* ctr, unsigned* done) {
+template <typename T, typename In>
+bool launch_fused(cub_handle h, In inside, const SweepArgs& ca, int cfg, unsigned* ctr, unsigned* done) {
   if (!h->knobs.fuse || h->pad) return false;
   const Grid& g = ca.g;
   // 8- and 16-bit pixels keep their own classification kernel (4 pixels per lane per load) where it applies
@@ -413,8 +425,8 @@ bool launch_fused(cub_handle h, const SweepArgs& ca, int cfg, unsigned* ctr, uns
   // TMA bulk copies: 16-byte aligned rows
   if (((size_t)g.X * sizeof(T)) % 16 != 0 || (reinterpret_cast<uintptr_t>(h->d_vol) & 15u) != 0) return false;
   const int c = cfg >= 0 ? cfg : (g.Wx > 8 ? 2 : 10);
-  if (c == 2) return launch_fused_cfg<T, SweepCfg<17, 7, 2, MODE_COUNT>>(h, ca, ctr, done);
-  if (c == 10) return launch_fused_cfg<T, SweepCfg<9, 14, 2, MODE_COUNT>>(h, ca, ctr, done);
+  if (c == 2) return launch_fused_cfg<T, SweepCfg<17, 7, 2, MODE_COUNT>>(h, inside, ca, ctr, done);
+  if (c == 10) return launch_fused_cfg<T, SweepCfg<9, 14, 2, MODE_COUNT>>(h, inside, ca, ctr, done);
   return false;
 }
 
@@ -625,6 +637,7 @@ static int set_geometry(cub_handle h, int dtype, const uint64_t dims[3], const d
   h->dtype = dtype;
   h->pix_bytes = pb;
   h->i0[0] = h->i0[1] = h->i0[2] = 0;
+  h->range_on = false;
   h->image_nz = dims[2];
   h->local_z0 = 0;
   h->own_z0 = 0;
@@ -666,6 +679,25 @@ int cub_set_region_index(cub_handle h, const int64_t index[3]) {
     h->i0[k] = v;
   }
   h->counted = h->emitted = h->count_queued = false;
+  return CUB_OK;
+}
+
+int cub_set_inside_range(cub_handle h, int enable, double lower, double upper) {
+  if (!h) return CUB_ERR_INVALID;
+  if (!h->has_volume) return fail(h, CUB_ERR_INVALID, "cub_set_inside_range before cub_set_volume");
+  h->counted = h->emitted = h->count_queued = false;
+  if (!enable) {
+    h->range_on = false;
+    return CUB_OK;
+  }
+  // the bounds are pixel values, checked by the rule cub_count applies to the iso value
+  if (std::isnan(lower) || std::isnan(upper)) return fail(h, CUB_ERR_INVALID, "inside range bound is NaN");
+  if (iso_as_pixel(h->dtype, lower) != lower || iso_as_pixel(h->dtype, upper) != upper)
+    return fail(h, CUB_ERR_INVALID, "inside range [%.17g, %.17g] is not representable in the pixel type", lower, upper);
+  if (!(lower <= upper)) return fail(h, CUB_ERR_INVALID, "inside range [%.17g, %.17g]: lower exceeds upper", lower, upper);
+  h->range_on = true;
+  h->range_lo = lower;
+  h->range_hi = upper;
   return CUB_OK;
 }
 
@@ -717,8 +749,14 @@ int count_launch(cub_handle h, const cub_params* p) {
   h->wait_before_faces = nullptr;
   h->params = *p;
   CUB_TRY(setup_grid(h));
-  if (iso_as_pixel(h->dtype, p->iso_value) != p->iso_value)
+  if (h->range_on) {
+    // (the iso value plays no part in range mode)
+    if (p->project_vertices)
+      return fail(h, CUB_ERR_INVALID, "vertex projection needs an iso-surface and an inside range has none: turn "
+                                      "project_vertices off, or leave range mode (cub_set_inside_range with enable = 0)");
+  } else if (iso_as_pixel(h->dtype, p->iso_value) != p->iso_value) {
     return fail(h, CUB_ERR_INVALID, "iso value %.17g is not representable in the pixel type", p->iso_value);
+  }
   if (p->projection_method < CUB_PROJECT_DEFAULT || p->projection_method > CUB_PROJECT_LINESEARCH || p->reserved != 0)
     return fail(h, CUB_ERR_INVALID, "unknown projection_method %d", (int)p->projection_method);
   compute_step(h);
@@ -829,10 +867,12 @@ int count_launch(cub_handle h, const cub_params* p) {
     bool fused = false;
     {
       Timer t(h, 0);
-      DISPATCH_PIXEL(h->dtype, fused = launch_fused<T>(h, ca, h->knobs.count_cfg, h->d_fuse_ctr, h->d_fuse_done));
+      DISPATCH_PIXEL(h->dtype, (fused = with_inside<T>(h, [&](auto in) {
+                       return launch_fused<T>(h, in, ca, h->knobs.count_cfg, h->d_fuse_ctr, h->d_fuse_done);
+                     })));
       CU_TRY(h, cudaGetLastError());
       if (!fused) {
-        DISPATCH_PIXEL(h->dtype, launch_classify<T>(h, 0, g.Zl, h->stream, h->knobs.k1_ctas));
+        DISPATCH_PIXEL(h->dtype, (with_inside<T>(h, [&](auto in) { launch_classify<T>(h, in, 0, g.Zl, h->stream, h->knobs.k1_ctas); })));
         CU_TRY(h, cudaGetLastError());
       }
       t.stop();
@@ -1285,6 +1325,9 @@ int cub_debug_bitmask(cub_handle h, uint32_t* out, uint64_t* words_per_row) {
 int cub_debug_project_points(cub_handle h, const cub_params* p, float* points_xyz, uint64_t n_points) {
   if (!h) return CUB_ERR_INVALID;
   if (!p || !points_xyz) return fail(h, CUB_ERR_INVALID, "null argument");
+  if (h->range_on)
+    return fail(h, CUB_ERR_INVALID, "vertex projection needs an iso-surface and an inside range has none: leave range mode "
+                                    "(cub_set_inside_range with enable = 0)");
   CU_TRY(h, cudaSetDevice(h->device));
   h->params = *p;
   CUB_TRY(setup_grid(h));

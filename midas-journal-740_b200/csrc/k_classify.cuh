@@ -22,15 +22,41 @@ namespace cbr {
 
 constexpr int kWordsPerTask = 16;
 
+// The inside predicate, a template parameter of every classification kernel (K1 and the producers of k_fused.cuh).
+// AtLeast is the reference's rule !(v < iso) (txx:139-141, 167).  Between is the inside-range mode of
+// cub_set_inside_range, !(v < lo) && !(hi < v).  Both compare in the pixel type, so a NaN pixel is inside in either.
+// A kernel takes In::Param and builds the predicate from it.  For AtLeast that is the plain iso value: a struct
+// parameter would be loaded differently (as bytes for 8-bit pixels), and iso mode compiles to the same code as a
+// kernel that takes `T iso`.
+template <typename T>
+struct AtLeast {
+  static constexpr bool kRange = false;
+  using Param = T;
+  T iso;
+  __host__ __device__ __forceinline__ Param param() const { return iso; }
+  __device__ __forceinline__ bool operator()(const T v) const { return !(v < iso); }
+  __device__ __forceinline__ T lower() const { return iso; }
+};
+template <typename T>
+struct Between {
+  static constexpr bool kRange = true;
+  using Param = Between;
+  T lo, hi;
+  __host__ __device__ __forceinline__ Param param() const { return *this; }
+  __device__ __forceinline__ bool operator()(const T v) const { return !(v < lo) && !(hi < v); }
+  __device__ __forceinline__ T lower() const { return lo; }
+};
+
 template <typename T>
 __device__ __forceinline__ T load_stream(const T* p) {
   return __ldcs(p);  // read-once data: evict-first
 }
 
 // FULL: X % 32 == 0 and Wx % kWordsPerTask == 0 (no clamping, no partial tasks)
-template <typename T, bool FULL>
+template <typename T, bool FULL, typename In>
 __global__ void __launch_bounds__(256) k_classify(const T* __restrict__ vol, uint32_t* __restrict__ bits, Grid g,
-                                                  T iso, unsigned n_tasks, unsigned groups_per_row) {
+                                                  typename In::Param bounds, unsigned n_tasks, unsigned groups_per_row) {
+  const In inside{bounds};
   const int lane = threadIdx.x & 31;
   const unsigned warp0 = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const unsigned n_warps = (gridDim.x * blockDim.x) >> 5;
@@ -52,7 +78,7 @@ __global__ void __launch_bounds__(256) k_classify(const T* __restrict__ vol, uin
     }
     uint32_t word[kWordsPerTask];
 #pragma unroll
-    for (int k = 0; k < kWordsPerTask; ++k) word[k] = __ballot_sync(0xffffffffu, !(v[k] < iso));
+    for (int k = 0; k < kWordsPerTask; ++k) word[k] = __ballot_sync(0xffffffffu, inside(v[k]));
     if (lane == 0) {
       uint32_t* dst = bits + (size_t)row * g.Wp + w0;
       if (FULL) {
@@ -80,14 +106,20 @@ __global__ void __launch_bounds__(256) k_classify(const T* __restrict__ vol, uin
 // 128-byte store.  (A redux.sync per load over the G-lane groups was tried first: sub-warp masks serialise it.)
 // Requires X % (32 * VPL) == 0 and a 4-byte aligned buffer (else: k_classify above).
 template <typename T> struct PackedTraits;
+// a pixel value in every 1- or 2-byte field of a word
+template <typename T>
+__device__ __forceinline__ uint32_t replicate(const T v) {
+  return sizeof(T) == 1 ? 0x01010101u * (uint32_t)(uint8_t)v : 0x00010001u * (uint32_t)(uint16_t)v;
+}
 template <> struct PackedTraits<uint8_t>  { static constexpr bool is_signed = false; };
 template <> struct PackedTraits<int8_t>   { static constexpr bool is_signed = true; };
 template <> struct PackedTraits<uint16_t> { static constexpr bool is_signed = false; };
 template <> struct PackedTraits<int16_t>  { static constexpr bool is_signed = true; };
 
-template <typename T>
+template <typename T, typename In>
 __global__ void __launch_bounds__(256) k_classify_packed(const T* __restrict__ vol, uint32_t* __restrict__ bits, Grid g,
-                                                         T iso, unsigned n_tasks, unsigned tasks_per_row) {
+                                                         typename In::Param bounds, unsigned n_tasks, unsigned tasks_per_row) {
+  const In inside{bounds};
   constexpr int VPL = 4 / (int)sizeof(T);   // voxels per lane per load = words per warp load = bits per field
   constexpr int G = 32 / VPL;               // lanes per word = loads per task = fields per accumulator
   constexpr uint32_t H = sizeof(T) == 1 ? 0x80808080u : 0x80008000u;  // top bit of every pixel
@@ -96,9 +128,13 @@ __global__ void __launch_bounds__(256) k_classify_packed(const T* __restrict__ v
   const int grp = lane / G, m = lane % G;
   // iso in every pixel; signed compare == unsigned compare with the sign bits flipped (the lanes' sign flip is
   // folded into the final select below)
-  uint32_t iso_rep = sizeof(T) == 1 ? 0x01010101u * (uint32_t)(uint8_t)iso : 0x00010001u * (uint32_t)(uint16_t)iso;
+  uint32_t iso_rep = replicate<T>(inside.lower());
   if (SGN) iso_rep ^= H;
   const uint32_t iso_low = iso_rep & ~H;
+  // range mode: the upper bound in every pixel, sign bits flipped like iso_rep, and with every top bit set
+  uint32_t hi_rep = 0;
+  if constexpr (In::kRange) hi_rep = replicate<T>(inside.hi) ^ (SGN ? H : 0u);
+  const uint32_t hi_top = hi_rep | H;
   const unsigned warp0 = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const unsigned n_warps = (gridDim.x * blockDim.x) >> 5;
   for (unsigned task = warp0; task < n_tasks; task += n_warps) {
@@ -120,6 +156,14 @@ __global__ void __launch_bounds__(256) k_classify_packed(const T* __restrict__ v
       uint32_t ge;
       if (SGN) ge = (~a & ~iso_rep) | ((a ^ iso_rep) & t);   // a's sign bit flipped: a' = a ^ H
       else ge = (a & ~iso_rep) | (~(a ^ iso_rep) & t);
+      if constexpr (In::kRange) {
+        // per pixel hi >= a, the same compare with the operands swapped: u = (hi | H) - (a & ~H).  Every field of the
+        // minuend is at least H and every field of the subtrahend below H, so no field borrows from the one above it;
+        // u's top bit per pixel is (low bits of hi) >= (low bits of a), and the top bits decide unless they are equal
+        const uint32_t u = hi_top - (a & ~H);
+        if (SGN) ge &= (hi_rep & a) | ((hi_rep ^ a) & u);       // hi_rep is hi' = hi ^ H, a' = a ^ H
+        else ge &= (hi_rep & ~a) | (~(hi_rep ^ a) & u);
+      }
       // top bits of the VPL pixels -> the VPL top bits of the word -> field k
       uint32_t f;
       if (VPL == 4) f = ((ge & H) * 0x00204081u) >> 28;
@@ -148,9 +192,11 @@ __global__ void __launch_bounds__(256) k_classify_packed(const T* __restrict__ v
 // Every later kernel runs unchanged on the padded grid: its clamped neighbours at the padded border are outside
 // on both sides, so no face is lost and none is invented.  One warp per 32-voxel word; the loads are one
 // element off the 128-byte alignment, which costs this opt-in mode a few percent of bandwidth.
-template <typename T>
+template <typename T, typename In>
 __global__ void __launch_bounds__(256) k_classify_padded(const T* __restrict__ vol, uint32_t* __restrict__ bits, Grid gb,
-                                                         int vX, int vY, int vZl, int zpad, T iso, unsigned n_words_total) {
+                                                         int vX, int vY, int vZl, int zpad, typename In::Param bounds,
+                                                         unsigned n_words_total) {
+  const In inside{bounds};
   const int lane = threadIdx.x & 31;
   const unsigned warp0 = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const unsigned n_warps = (gridDim.x * blockDim.x) >> 5;
@@ -161,7 +207,7 @@ __global__ void __launch_bounds__(256) k_classify_padded(const T* __restrict__ v
     const int x = 32 * w + lane - 1, y = yb - 1, z = zb - zpad;
     bool in = false;
     if (x >= 0 && x < vX && y >= 0 && y < vY && z >= 0 && z < vZl)
-      in = !(__ldcs(vol + ((size_t)z * vY + y) * vX + x) < iso);
+      in = inside(__ldcs(vol + ((size_t)z * vY + y) * vX + x));
     const uint32_t word = __ballot_sync(0xffffffffu, in);
     if (lane == 0) bits[(size_t)row * gb.Wp + w] = word;
   }

@@ -11,7 +11,7 @@
 //   * warpgroup 0 = four PRODUCER warps.  Each owns a private ring of kFuseStages 4 KB shared-memory stages that one
 //     elected lane fills with TMA bulk copies (cp.async.bulk global -> shared, completion on an mbarrier), so the
 //     bytes in flight per SM are set by shared memory, not by registers or by the number of resident warps; the warp
-//     reads a landed stage one voxel per lane, the ballot of `!(v < iso)` is the output word (as in k_classify), and
+//     reads a landed stage one voxel per lane, the ballot of the inside predicate is the output word (as in k_classify), and
 //     lane 0 stores the words with an L2 evict-last hint (the consumers read them a few slices later).
 //     Tasks (<= 4 KB of one row) are handed out in raster order, `batch` at a time through one atomic ticket (the next
 //     ticket is requested while the current batch is issued); a finished batch is published with one release-add per
@@ -106,9 +106,10 @@ __device__ __forceinline__ unsigned ld_acquire(const unsigned* p) {
 }
 
 // ---- producer warp: classification tasks through the warp's private TMA ring ---------------------------------------
-template <typename T, int S>
-__device__ __forceinline__ void fused_producer(const FuseArgs& a, const T iso, FuseProducerSmem<S>& sm, const int warp,
-                                               const int lane) {
+template <typename T, int S, typename In>
+__device__ __forceinline__ void fused_producer(const FuseArgs& a, const typename In::Param bounds, FuseProducerSmem<S>& sm,
+                                               const int warp, const int lane) {
+  const In inside{bounds};
   constexpr int WPT = kFuseStageBytes / (32 * (int)sizeof(T));  // words per task
   static_assert(WPT >= 4 && WPT % 4 == 0, "16-byte stores of the words of a task");
   const T* __restrict__ vol = static_cast<const T*>(a.vol);
@@ -197,14 +198,14 @@ __device__ __forceinline__ void fused_producer(const FuseArgs& a, const T iso, F
       for (int k4 = 0; k4 < WPT; k4 += 4) {
         uint32_t w[4];
 #pragma unroll
-        for (int k = 0; k < 4; ++k) w[k] = __ballot_sync(0xffffffffu, !(sp[(k4 + k) * 32] < iso));
+        for (int k = 0; k < 4; ++k) w[k] = __ballot_sync(0xffffffffu, inside(sp[(k4 + k) * 32]));
         if (lane == 0) st_keep(dst + k4, make_uint4(w[0], w[1], w[2], w[3]), keep);
       }
     } else {
       // ragged end of a row: lanes past it re-read the row's last voxel ("replicate bit X-1", k_classify.cuh)
       const int nw = (nvox + 31) >> 5, last = nvox - 1 - lane;
       for (int k = 0; k < nw; ++k) {
-        const uint32_t w = __ballot_sync(0xffffffffu, !(sp[min(k * 32, last)] < iso));
+        const uint32_t w = __ballot_sync(0xffffffffu, inside(sp[min(k * 32, last)]));
         if (lane == 0) dst[k] = w;
       }
     }
@@ -251,15 +252,15 @@ __device__ __forceinline__ void fused_consumer(const FuseArgs& a, SweepSmem<C>& 
   }
 }
 
-template <typename T, typename C, int S>
-__global__ void __launch_bounds__(kFuseThreads, 4) k_classify_sweep(const FuseArgs a, const T iso) {
+template <typename T, typename C, int S, typename In>
+__global__ void __launch_bounds__(kFuseThreads, 4) k_classify_sweep(const FuseArgs a, const typename In::Param bounds) {
   pdl_enter();
   static_assert(C::NTP == 128, "the consumer role is one warpgroup");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   FuseSmem<C, S>& sm = *reinterpret_cast<FuseSmem<C, S>*>(smem_raw);
   if (threadIdx.x < 32 * kFuseProducerWarps) {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kFuseProducerRegs));
-    fused_producer<T, S>(a, iso, sm.p, (int)(threadIdx.x >> 5), (int)(threadIdx.x & 31));
+    fused_producer<T, S, In>(a, bounds, sm.p, (int)(threadIdx.x >> 5), (int)(threadIdx.x & 31));
   } else {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kFuseConsumerRegs));
     fused_consumer<C>(a, sm.sw, &sm.tile, (int)threadIdx.x - 32 * kFuseProducerWarps);

@@ -53,6 +53,7 @@ class CuberilleImageToMeshFilter:
         self._raster_order = False
         self._border_faces = False
         self._projection_method = capi.PROJECT_DEFAULT
+        self._inside_range = None   # (lower, upper): range mode instead of the iso value
         self._thr = 0.5
         self._step = -1.0
         self._relax = 0.95
@@ -107,6 +108,15 @@ class CuberilleImageToMeshFilter:
     def SetRasterVertexOrder(self, b): self._set("_raster_order", bool(b))
     def GetRasterVertexOrder(self): return self._raster_order
 
+    # extension: inside range instead of the iso value (cub_set_inside_range); a label k is the range [k, k].  The
+    # projection needs an iso-surface: Update() raises while a range is set and ProjectVerticesToIsoSurface is on.
+    def SetInsideRange(self, lower, upper): self._set("_inside_range", (lower, upper))
+    def SetLabelValue(self, k): self.SetInsideRange(k, k)
+    def InsideRangeOff(self): self._set("_inside_range", None)
+    def GetInsideRange(self): return self._inside_range
+    def GetInsideRangeLower(self): return None if self._inside_range is None else self._inside_range[0]
+    def GetInsideRangeUpper(self): return None if self._inside_range is None else self._inside_range[1]
+
     def SetProjectVertexSurfaceDistanceThreshold(self, v):
         # itkSetClampMacro(.., 0.0, NumericTraits<InputPixelType>::max())  h:210
         hi = float("inf")
@@ -149,6 +159,8 @@ class CuberilleImageToMeshFilter:
             self._step = max(img.spacing) * 0.25  # sticky, txx:82-85
         self._handle.set_volume(img.data, img.spacing, img.origin, img.direction)
         self._handle.set_region_index(getattr(img, "region_index", (0, 0, 0)))
+        if self._inside_range is not None:
+            self._handle.set_inside_range(*self._inside_range)
         self._handle.run(self.params(), self._id_bytes)
         pts, cells, cd = self._handle.fetch(self._cell_data)
         self._output = Mesh(pts, cells, cd)
@@ -159,4 +171,5 @@ class CuberilleImageToMeshFilter:
 
     def __str__(self):  # PrintSelf, txx:501-520
         return (f"IsoSurfaceValue: {self._iso}\nGenerateTriangleFaces: {int(self._triangles)}\n"
-                f"ProjectVerticesToIsoSurface: {int(self._project)}\n")
+                f"ProjectVerticesToIsoSurface: {int(self._project)}\n"
+                + (f"InsideRange: [{self._inside_range[0]}, {self._inside_range[1]}]\n" if self._inside_range is not None else ""))

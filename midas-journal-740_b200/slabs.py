@@ -124,7 +124,7 @@ def gather_mesh(handle, comm, want_cell_data: bool = False):
 
 def run_streamed_rank(handles, streams, vol_ptr: int, dtype, dims_xyz, image_nz: int, local_z0: int, own: tuple[int, int],
                       params, out_points_ptr: int, out_cells_ptr: int, device_volume, exchange, id_bytes: int = 4,
-                      halo: int = 2, spacing=(1.0, 1.0, 1.0), origin=(0.0, 0.0, 0.0)):
+                      halo: int = 2, spacing=(1.0, 1.0, 1.0), origin=(0.0, 0.0, 0.0), inside_range=None):
     """One rank of a multi-GPU run, host volume in, host mesh out.  The rank's buffer (pinned, slices
     [local_z0, local_z0 + nz) of the image, its own range `own` plus halo) is copied once, in len(handles)
     consecutive pieces on a copy stream, into `device_volume`; sub-slab c is counted on handles[c] as soon as its
@@ -132,6 +132,7 @@ def run_streamed_rank(handles, streams, vol_ptr: int, dtype, dims_xyz, image_nz:
     counted, so the run has two phases: (1) upload + count all sub-slabs, exchange(points, quads) -> this rank's
     (point base, quad base) [an all-gather of two integers], (2) emit + copy out sub-slab by sub-slab.
     Outputs: this rank's part of the mesh at the start of its (pinned) output buffers.
+    `inside_range`: (lower, upper) meshes that range instead of the iso value (Handle.set_inside_range).
     Returns (n_points, n_cells, point_base, cell_base) of the rank."""
     import ctypes
     import numpy as np
@@ -166,6 +167,8 @@ def run_streamed_rank(handles, streams, vol_ptr: int, dtype, dims_xyz, image_nz:
         streams[c].wait_event(events[c])
         h.set_volume_ptr(device_volume.data_ptr() + (lo - local_z0) * slice_bytes, dtype, (nx, ny, hi - lo), capi.MEM_DEVICE,
                          spacing, origin)
+        if inside_range is not None:
+            h.set_inside_range(*inside_range)
         h.set_slab(image_nz, lo, s.own_z0, s.own_z1)
         h.count_async(params)
     counts = []
@@ -190,7 +193,7 @@ def run_streamed_rank(handles, streams, vol_ptr: int, dtype, dims_xyz, image_nz:
 
 def run_streamed(handles, vol_ptr: int, dtype, dims_xyz, params, n_slabs: int, out_points_ptr: int, out_cells_ptr: int,
                  id_bytes: int = 4, halo: int = 2, spacing=(1.0, 1.0, 1.0), origin=(0.0, 0.0, 0.0),
-                 device_volume=None, streams=None):
+                 device_volume=None, streams=None, inside_range=None):
     """One GPU, host volume in, host mesh out, streamed: the image is cut into `n_slabs` z-slabs that travel
     through `handles` (>= 2 capi.Handle objects, each on its own stream) round-robin, so the host->device copy
     of slab c+1, the kernels of slab c and the device->host copy of slab c-1 overlap.  Ids are global: the id
@@ -203,7 +206,9 @@ def run_streamed(handles, vol_ptr: int, dtype, dims_xyz, params, n_slabs: int, o
       CUB_MEM_HOST); works for volumes larger than the device memory, re-sends 2 * halo slices per cut;
     * `device_volume` (a torch uint8 CUDA tensor of the volume's size) + `streams` (the torch streams the
       handles were created on): the volume is copied once, in n_slabs consecutive pieces on a copy stream, into
-      that buffer and the handles borrow windows of it (CUB_MEM_DEVICE); nothing is sent twice."""
+      that buffer and the handles borrow windows of it (CUB_MEM_DEVICE); nothing is sent twice.
+
+    `inside_range`: (lower, upper) meshes that range instead of the iso value (Handle.set_inside_range)."""
     import numpy as np
     from . import capi
     nx, ny, nz = dims_xyz
@@ -245,6 +250,8 @@ def run_streamed(handles, vol_ptr: int, dtype, dims_xyz, params, n_slabs: int, o
         else:
             h.set_volume_ptr(vol_ptr + s.local_z0 * slice_bytes, dtype, (nx, ny, s.local_z1 - s.local_z0), capi.MEM_HOST,
                              spacing, origin)
+        if inside_range is not None:
+            h.set_inside_range(*inside_range)
         h.set_slab(nz, s.local_z0, s.own_z0, s.own_z1)
 
     upload(0)
