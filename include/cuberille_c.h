@@ -169,6 +169,55 @@ int cub_set_inside_range(cub_handle h, int enable, double lower, double upper);
 int cub_set_slab(cub_handle h, uint64_t image_nz, uint64_t local_z0,
                  uint64_t own_z0, uint64_t own_z1);
 
+/* Label maps (no counterpart in the reference).
+ *
+ * cub_label_bounds: one pass over the current volume on the device that finds,
+ * for every label k of the window [first_label, first_label + n_labels), its
+ * voxel count and bounding box.  out is a host buffer of n_labels x 8 values:
+ * {count, xmin, ymin, zmin, xmax, ymax, zmax, 0} of label first_label + i at
+ * out[8 * i], in buffer indices, maxima inclusive; a label with count 0 has all
+ * six bounds 0.  Pixels outside the window are ignored.  Integer pixel types
+ * only (CUB_ERR_UNSUPPORTED for float32 / float64); 1 <= n_labels <= 65536 and
+ * the window must lie inside the pixel type's range, else CUB_ERR_INVALID, as
+ * while a region of interest or a z-slab is set.  Synchronises.                */
+int cub_label_bounds(cub_handle h, int64_t first_label, uint32_t n_labels, uint64_t *out);
+
+/* Region of interest: from now on cub_count / cub_count_async (and
+ * cub_debug_bitmask, cub_download_volume, cub_debug_project_points) work on the
+ * box [lo, lo + size) of the current volume.  The result is exactly that of
+ * cub_set_volume on a copy of the box followed by cub_set_region_index(region
+ * index + lo), in every mode: interpolation and gradients of the projection
+ * clamp at the box, as for an image cut out with ITK's ExtractImageFilter.  A
+ * box of whole rows and slices (full x and y extent) is used in place; any
+ * other box is copied, on the handle's stream, into a buffer the handle owns.
+ * lo == NULL returns to the whole volume.  An empty box, one that leaves the
+ * volume, or a call before cub_set_volume returns CUB_ERR_INVALID; combining
+ * the box with cub_set_slab, in either order, CUB_ERR_UNSUPPORTED.
+ * cub_set_volume and cub_generate_volume clear the box; cub_set_region_index
+ * stays the index of the whole buffer, and the box's lo adds to it.             */
+int cub_set_region_of_interest(cub_handle h, const uint64_t lo[3], const uint64_t size[3]);
+
+/* Every label of a label map in one call: labels[i] is meshed as the inside
+ * range [k, k] and the meshes are concatenated in the given order, point ids of
+ * label i offset by the points of labels 0..i-1.  point_offsets and
+ * cell_offsets (n_labels + 1 entries each) receive the start of every label's
+ * part and, last, the totals.  The result is read with cub_fetch /
+ * cub_device_buffers like any other run; its cell data, when asked for, is the
+ * label.  Each part is bit-identical to cub_set_inside_range(k, k) + cub_count
+ * + cub_set_id_base(point_offsets[i], cell_offsets[i]) + cub_emit on the whole
+ * volume, in every emit mode, because each label is meshed in its bounding box
+ * grown by one voxel and clipped to the image (DESIGN.md §2): one
+ * cub_label_bounds pass finds the boxes, and a label without voxels gives an
+ * empty part and launches nothing.  The labels must be pixel values of the
+ * volume's integer type (the rule of cub_set_inside_range), each given once,
+ * else CUB_ERR_INVALID; so do project_vertices != 0 (a label has no
+ * iso-surface), a set region of interest and a z-slab.  A float volume returns
+ * CUB_ERR_UNSUPPORTED.  The handle's own inside-range setting is left as it
+ * was.  cub_last_warning names the labels whose mesh has an empty interior
+ * slice.  Synchronises once per label.                                         */
+int cub_run_labels(cub_handle h, const cub_params *p, const double *labels, uint64_t n_labels,
+                   int id_bytes, uint64_t *point_offsets, uint64_t *cell_offsets);
+
 /* Phase 1 of GenerateData (txx:136-173 without the emission): classify every
  * voxel against iso, find faces and first-touch corner owners, scan.
  * Returns the number of points / quads this handle's own z-range produces.

@@ -36,6 +36,7 @@
 
 #include <chrono>
 #include <cstdint>
+#include <limits>
 #include <type_traits>
 #include <vector>
 
@@ -208,6 +209,24 @@ public:
   itkGetMacro( InsideRangeLower, InputPixelType );
   itkGetMacro( InsideRangeUpper, InputPixelType );
 
+  /** Extension (off by default): mesh every label of a label map in one Update() (cub_run_labels).  Each label k is
+   * meshed as the range [k, k]; the meshes are concatenated in the given order into the one output mesh, point ids of
+   * a label offset by the points of the labels before it.  GetLabelPointOffsets() / GetLabelCellOffsets() (one entry
+   * per label plus the totals) give where each label's part starts.  Integer pixel types only; the projection and an
+   * inside range must be off.  An empty vector turns it off, as ClearLabelValues() does. */
+  void SetLabelValues( const std::vector<InputPixelType> & labels )
+    {
+    if ( m_LabelValues != labels )
+      {
+      m_LabelValues = labels;
+      this->Modified();
+      }
+    }
+  void ClearLabelValues() { this->SetLabelValues( std::vector<InputPixelType>() ); }
+  const std::vector<InputPixelType> & GetLabelValues() const { return m_LabelValues; }
+  const std::vector<uint64_t> & GetLabelPointOffsets() const { return m_LabelPointOffsets; }
+  const std::vector<uint64_t> & GetLabelCellOffsets() const { return m_LabelCellOffsets; }
+
   /** Projection knobs with the reference's clamp ranges (h:209-228). */
   itkGetMacro( ProjectVertexSurfaceDistanceThreshold, double );
   itkSetClampMacro( ProjectVertexSurfaceDistanceThreshold, double, 0.0, NumericTraits<InputPixelType>::max() );
@@ -286,6 +305,12 @@ protected:
     os << indent << "InsideRange: " << m_InsideRangeOn << " ["
        << static_cast< typename NumericTraits<InputPixelType>::PrintType >( m_InsideRangeLower ) << ", "
        << static_cast< typename NumericTraits<InputPixelType>::PrintType >( m_InsideRangeUpper ) << "]" << std::endl;
+    os << indent << "LabelValues:";
+    for ( size_t i = 0; i < m_LabelValues.size(); i++ )
+      {
+      os << " " << static_cast< typename NumericTraits<InputPixelType>::PrintType >( m_LabelValues[i] );
+      }
+    os << std::endl;
     }
 
   virtual void GenerateOutputInformation() { } // do nothing (h:236)
@@ -340,6 +365,23 @@ protected:
                                  cuberille_detail::PixelCode<InputPixelType>::value,
                                  dims, spacing, origin, direction, CUB_MEM_HOST ) );
     this->Check( cub_set_region_index( m_Handle, regionIndex ) );
+    const bool labels = !m_LabelValues.empty();
+    if ( labels )
+      {
+      if ( m_ProjectVerticesToIsoSurface )
+        {
+        itkExceptionMacro( << "a label has no iso-surface to project the vertices onto: call "
+                           "ProjectVerticesToIsoSurfaceOff() (projection is on by default)" );
+        }
+      if ( m_InsideRangeOn )
+        {
+        itkExceptionMacro( << "SetLabelValues meshes each label on its own: call InsideRangeOff() first" );
+        }
+      if ( !std::numeric_limits<InputPixelType>::is_integer )
+        {
+        itkExceptionMacro( << "SetLabelValues needs an integer pixel type" );
+        }
+      }
     if ( m_InsideRangeOn )
       {
       if ( m_ProjectVerticesToIsoSurface )
@@ -370,7 +412,22 @@ protected:
     // refuses more): the ids travel as 32-bit values - half the bytes over PCIe - and are widened when the cells
     // are created below.
     uint64_t numberOfPoints = 0, numberOfCells = 0;
-    this->Check( cub_run( m_Handle, &params, 4, &numberOfPoints, &numberOfCells ) );
+    if ( labels )
+      {
+      std::vector<double> values( m_LabelValues.begin(), m_LabelValues.end() );
+      m_LabelPointOffsets.assign( values.size() + 1, 0 );
+      m_LabelCellOffsets.assign( values.size() + 1, 0 );
+      this->Check( cub_run_labels( m_Handle, &params, values.data(), values.size(), 4, m_LabelPointOffsets.data(),
+                                   m_LabelCellOffsets.data() ) );
+      numberOfPoints = m_LabelPointOffsets.back();
+      numberOfCells = m_LabelCellOffsets.back();
+      }
+    else
+      {
+      m_LabelPointOffsets.clear();
+      m_LabelCellOffsets.clear();
+      this->Check( cub_run( m_Handle, &params, 4, &numberOfPoints, &numberOfCells ) );
+      }
     this->Check( cub_synchronize( m_Handle ) );
     const Clock::time_point t2 = Clock::now();
     const char * warning = cub_last_warning( m_Handle );
@@ -468,6 +525,9 @@ private:
   bool                m_InsideRangeOn;
   InputPixelType      m_InsideRangeLower;
   InputPixelType      m_InsideRangeUpper;
+  std::vector<InputPixelType> m_LabelValues;
+  std::vector<uint64_t> m_LabelPointOffsets;
+  std::vector<uint64_t> m_LabelCellOffsets;
   double              m_ProjectVertexSurfaceDistanceThreshold;
   double              m_ProjectVertexStepLength;
   double              m_ProjectVertexStepLengthRelaxationFactor;

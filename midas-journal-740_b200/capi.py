@@ -27,7 +27,8 @@ CODE_DTYPES = {v: k for k, v in DTYPE_CODES.items()}
 # every symbol include/cuberille_c.h declares (tests check that the library exports all of them)
 SYMBOLS = [
     "cub_abi_version", "cub_default_params", "cub_create", "cub_destroy", "cub_last_error", "cub_set_volume",
-    "cub_set_region_index", "cub_set_inside_range", "cub_set_slab", "cub_count", "cub_set_id_base", "cub_emit_vertices", "cub_emit", "cub_run", "cub_fetch", "cub_fetch_async",
+    "cub_set_region_index", "cub_set_inside_range", "cub_set_slab", "cub_label_bounds", "cub_set_region_of_interest",
+    "cub_run_labels", "cub_count", "cub_set_id_base", "cub_emit_vertices", "cub_emit", "cub_run", "cub_fetch", "cub_fetch_async",
     "cub_synchronize", "cub_device_buffers",
     "cub_debug_bitmask", "cub_debug_project_points", "cub_generate_volume", "cub_download_volume",
     "cub_enable_timing", "cub_get_timings", "cub_launch_count", "cub_count_was_fused",
@@ -95,6 +96,12 @@ def load() -> C.CDLL:
     L.cub_set_inside_range.argtypes = [vp, i, C.c_double, C.c_double]
     L.cub_set_slab.restype = i
     L.cub_set_slab.argtypes = [vp, u64, u64, u64, u64]
+    L.cub_label_bounds.restype = i
+    L.cub_label_bounds.argtypes = [vp, C.c_int64, C.c_uint32, pu64]
+    L.cub_set_region_of_interest.restype = i
+    L.cub_set_region_of_interest.argtypes = [vp, pu64, pu64]
+    L.cub_run_labels.restype = i
+    L.cub_run_labels.argtypes = [vp, C.POINTER(Params), pd, u64, i, pu64, pu64]
     L.cub_count.restype = i
     L.cub_count.argtypes = [vp, C.POINTER(Params), pu64, pu64]
     L.cub_set_id_base.restype = i
@@ -198,6 +205,7 @@ class Handle:
         self._keep = None
         self.dtype = None
         self.dims = None
+        self._whole_dims = None   # the volume's dims while a region of interest is set (self.dims: the box)
 
     def close(self):
         if self._h:
@@ -225,7 +233,7 @@ class Handle:
         og = (C.c_double * 3)(*origin)
         dr = (C.c_double * 9)(*direction) if direction is not None else None
         self._check(self._L.cub_set_volume(self._h, vol.ctypes.data, DTYPE_CODES[vol.dtype], dims, sp, og, dr, MEM_HOST))
-        self.dtype, self.dims = vol.dtype, (vol.shape[2], vol.shape[1], vol.shape[0])
+        self.dtype, self.dims, self._whole_dims = vol.dtype, (vol.shape[2], vol.shape[1], vol.shape[0]), None
 
     def set_volume_ptr(self, ptr: int, dtype, dims_xyz, mem_kind, spacing=(1.0, 1.0, 1.0), origin=(0.0, 0.0, 0.0)):
         """Raw pointer (host pinned or device) with dims (x, y, z)."""
@@ -233,7 +241,7 @@ class Handle:
         sp = (C.c_double * 3)(*spacing)
         og = (C.c_double * 3)(*origin)
         self._check(self._L.cub_set_volume(self._h, C.c_void_p(ptr), DTYPE_CODES[np.dtype(dtype)], dims, sp, og, None, mem_kind))
-        self.dtype, self.dims = np.dtype(dtype), tuple(dims_xyz)
+        self.dtype, self.dims, self._whole_dims = np.dtype(dtype), tuple(dims_xyz), None
 
     def set_region_index(self, index_xyz):
         """Image index of the buffer's first voxel (after set_volume, which resets it to 0)."""
@@ -249,6 +257,35 @@ class Handle:
         """Back to iso mode."""
         self._check(self._L.cub_set_inside_range(self._h, 0, 0.0, 0.0))
 
+    def label_bounds(self, first: int, n: int) -> np.ndarray:
+        """(n, 8) uint64: {count, xmin, ymin, zmin, xmax, ymax, zmax, 0} of the labels first .. first + n - 1 of the
+        current integer volume (buffer indices, inclusive maxima; all zero for an absent label)."""
+        out = np.zeros((int(n), 8), np.uint64)
+        self._check(self._L.cub_label_bounds(self._h, int(first), int(n), out.ctypes.data_as(C.POINTER(C.c_uint64))))
+        return out
+
+    def set_region_of_interest(self, lo_xyz, size_xyz):
+        """Count on the box [lo, lo + size) of the current volume, as on a copy of it with the region index moved by lo."""
+        self._check(self._L.cub_set_region_of_interest(self._h, (C.c_uint64 * 3)(*[int(v) for v in lo_xyz]),
+                                                       (C.c_uint64 * 3)(*[int(v) for v in size_xyz])))
+        self._whole_dims = self._whole_dims or self.dims
+        self.dims = tuple(int(v) for v in size_xyz)
+
+    def clear_region_of_interest(self):
+        self._check(self._L.cub_set_region_of_interest(self._h, None, None))
+        self.dims, self._whole_dims = self._whole_dims or self.dims, None
+
+    def run_labels(self, params: Params, labels, id_bytes: int = 4):
+        """Mesh every label as the range [k, k], concatenated in the given order; returns (point_offsets, cell_offsets),
+        n_labels + 1 entries each.  Read the mesh with fetch() / device_buffers()."""
+        lab = np.ascontiguousarray(labels, np.float64).reshape(-1)
+        po = np.zeros(lab.size + 1, np.uint64)
+        co = np.zeros(lab.size + 1, np.uint64)
+        self._check(self._L.cub_run_labels(self._h, C.byref(params), lab.ctypes.data_as(C.POINTER(C.c_double)), lab.size,
+                                           id_bytes, po.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                           co.ctypes.data_as(C.POINTER(C.c_uint64))))
+        return po, co
+
     def set_slab(self, image_nz: int, local_z0: int, own_z0: int, own_z1: int):
         self._check(self._L.cub_set_slab(self._h, image_nz, local_z0, own_z0, own_z1))
 
@@ -258,7 +295,7 @@ class Handle:
         d = (C.c_uint64 * 3)(*dims_xyz)
         im = (C.c_uint64 * 3)(*image_dims_xyz)
         self._check(self._L.cub_generate_volume(self._h, kind, d, im, z_offset, p0, p1, seed))
-        self.dtype, self.dims = np.dtype(np.float32), tuple(dims_xyz)
+        self.dtype, self.dims, self._whole_dims = np.dtype(np.float32), tuple(dims_xyz), None
 
     def download_volume(self) -> np.ndarray:
         x, y, z = self.dims

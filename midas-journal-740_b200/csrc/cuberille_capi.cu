@@ -30,6 +30,7 @@
 #include "k_sweep.cuh"
 #include "k_fused.cuh"
 #include "k_vertices.cuh"
+#include "k_labels.cuh"
 
 using namespace cbr;
 
@@ -123,6 +124,17 @@ struct cub_handle_s {
   // slab
   uint64_t image_nz = 0, local_z0 = 0, own_z0 = 0, own_z1 = 0;
   bool slab_set = false;
+  // region of interest (cub_set_region_of_interest): while it is set, d_vol / dims / i0 describe the box and these
+  // the whole volume; a box that is not whole rows and slices is a copy in roi_buf
+  bool roi_on = false;
+  const void* full_vol = nullptr;
+  uint64_t full_dims[3] = {0, 0, 0};
+  uint64_t roi_lo[3] = {0, 0, 0};
+  DevBuf<unsigned char> roi_buf;
+  // cub_label_bounds: the device table; cub_run_labels: the concatenation of the parts
+  DevBuf<unsigned long long> label_table;
+  DevBuf<float> cat_points;
+  DevBuf<unsigned char> cat_cells, cat_celldata;
 
   // scratch
   DevBuf<uint32_t> bits, cnt, act, cofs, perm;
@@ -587,6 +599,8 @@ int cub_destroy(cub_handle h) {
   cudaFree(h->ctrl.p); cudaFree(h->cofs.p); cudaFree(h->vtx.p); cudaFree(h->vsl.p);
   if (h->h_info) cudaFreeHost(h->h_info);
   cudaFree(h->points.p); cudaFree(h->cells.p); cudaFree(h->celldata.p); cudaFree(h->quads.p);
+  cudaFree(h->roi_buf.p); cudaFree(h->label_table.p);
+  cudaFree(h->cat_points.p); cudaFree(h->cat_cells.p); cudaFree(h->cat_celldata.p);
   for (int i = 0; i < 10; ++i) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
   if (h->own_stream) cudaStreamDestroy(h->stream);
   delete h;
@@ -638,6 +652,8 @@ static int set_geometry(cub_handle h, int dtype, const uint64_t dims[3], const d
   h->pix_bytes = pb;
   h->i0[0] = h->i0[1] = h->i0[2] = 0;
   h->range_on = false;
+  h->roi_on = false;
+  h->slab_set = false;
   h->image_nz = dims[2];
   h->local_z0 = 0;
   h->own_z0 = 0;
@@ -676,7 +692,7 @@ int cub_set_region_index(cub_handle h, const int64_t index[3]) {
   for (int k = 0; k < 3; ++k) {
     const long long v = index ? (long long)index[k] : 0;
     if (v < -(1ll << 30) || v > (1ll << 30)) return fail(h, CUB_ERR_INVALID, "region index beyond +-2^30 is not supported");
-    h->i0[k] = v;
+    h->i0[k] = v + (h->roi_on ? (long long)h->roi_lo[k] : 0);
   }
   h->counted = h->emitted = h->count_queued = false;
   return CUB_OK;
@@ -704,6 +720,7 @@ int cub_set_inside_range(cub_handle h, int enable, double lower, double upper) {
 int cub_set_slab(cub_handle h, uint64_t image_nz, uint64_t local_z0, uint64_t own_z0, uint64_t own_z1) {
   if (!h) return CUB_ERR_INVALID;
   if (!h->has_volume) return fail(h, CUB_ERR_INVALID, "cub_set_slab before cub_set_volume");
+  if (h->roi_on) return fail(h, CUB_ERR_UNSUPPORTED, "a z-slab cannot be combined with a region of interest");
   const uint64_t zl = h->dims[2];
   if (image_nz == 0 || image_nz >= (1ull << 31) || local_z0 + zl > image_nz)
     return fail(h, CUB_ERR_INVALID, "local buffer [%llu,%llu) exceeds image_nz %llu", (unsigned long long)local_z0,
@@ -918,6 +935,11 @@ int count_launch(cub_handle h, const cub_params* p) {
 }
 
 // ---- the host learns the counts: one device -> host copy and one synchronisation -----------------------------------
+const char* const kEmptySliceRemark =
+    "an empty voxel slice lies between occupied slices: the reference filter merges vertices of different corner "
+    "planes there (its lookup-plane rotation only advances on inside voxels, txx:155-161); this mesh follows the "
+    "intended rule and may differ from the reference's";
+
 int count_finish(cub_handle h) {
   CU_TRY(h, cudaSetDevice(h->device));
   if (h->wait_before_faces) CU_TRY(h, cudaStreamWaitEvent(h->stream, h->wait_before_faces, 0));
@@ -943,10 +965,7 @@ int count_finish(cub_handle h) {
   h->cell_base = h->h_info[kInfoCellBase];
   h->flags = h->h_info[kInfoFlags];
   h->warning.clear();
-  if (h->flags & kFlagEmptyInteriorSlice)
-    h->warning = "an empty voxel slice lies between occupied slices: the reference filter merges vertices of different corner "
-                 "planes there (its lookup-plane rotation only advances on inside voxels, txx:155-161); this mesh follows the "
-                 "intended rule and may differ from the reference's";
+  if (h->flags & kFlagEmptyInteriorSlice) h->warning = kEmptySliceRemark;
   h->counted = true;
   return CUB_OK;
 }
@@ -1464,6 +1483,292 @@ int cub_get_timings(cub_handle h, float ms[8]) {
 
 uint64_t cub_launch_count(cub_handle h) { return h ? h->launches : 0; }
 int cub_count_was_fused(cub_handle h) { return (h && h->fused_last) ? 1 : 0; }
+
+}  // extern "C"
+
+// ---- label maps: per-label bounds, a region of interest, and every label meshed in its box ----------------------
+namespace {
+
+// the value range of an integer pixel type; false for the float types
+template <typename T>
+bool type_range(long long* lo, long long* hi) {
+  if constexpr (std::is_integral<T>::value) {
+    *lo = (long long)std::numeric_limits<T>::min();
+    *hi = (long long)std::numeric_limits<T>::max();
+    return true;
+  }
+  return false;
+}
+
+bool integer_range(int dtype, long long* lo, long long* hi) {
+  bool integral = false;
+  DISPATCH_PIXEL(dtype, integral = type_range<T>(lo, hi));
+  return integral;
+}
+
+// a z-slab: cub_set_slab, or a generated slab of a taller image
+bool has_slab(cub_handle h) { return h->slab_set || h->local_z0 != 0 || h->image_nz != h->dims[2]; }
+
+// k_label_bounds over the current volume into out[n * 8] (host), then the host form of the table
+int label_bounds(cub_handle h, long long first, uint32_t n, uint64_t* out) {
+  CU_TRY(h, cudaSetDevice(h->device));
+  CUB_TRY(ensure(h, h->label_table, (size_t)n * 8));
+  CU_TRY(h, cudaMemsetAsync(h->label_table.p, 0, (size_t)n * 8 * sizeof(unsigned long long), h->stream));
+  const unsigned long long X = h->dims[0], rows = h->dims[1] * h->dims[2];
+  // a warp sums its lanes' counts in 32 bits: more warps until one sees fewer than 2^32 voxels
+  unsigned long long blocks = std::min<unsigned long long>((rows + 7) / 8, (unsigned long long)h->num_sms * kLabelCtasPerSm);
+  const unsigned long long warp_rows = (1ull << 32) / X - 1;
+  blocks = std::max(blocks, (rows + warp_rows * 8 - 1) / (warp_rows * 8));
+  if (blocks >= (1ull << 31)) return fail(h, CUB_ERR_UNSUPPORTED, "volume too large for cub_label_bounds");
+  const unsigned f = (unsigned)(unsigned long long)first;
+  switch (h->dtype) {
+#define CUB_LABEL_BOUNDS(CODE, T)                                                                                      \
+    case CODE:                                                                                                         \
+      k_label_bounds<T><<<(unsigned)blocks, kLabelThreads, 0, h->stream>>>(static_cast<const T*>(h->d_vol), (unsigned)X, \
+                                                                         (unsigned)h->dims[1], rows, f, n, h->label_table.p); \
+      break;
+    CUB_LABEL_BOUNDS(CUB_U8, unsigned char)
+    CUB_LABEL_BOUNDS(CUB_I8, signed char)
+    CUB_LABEL_BOUNDS(CUB_U16, unsigned short)
+    CUB_LABEL_BOUNDS(CUB_I16, short)
+    CUB_LABEL_BOUNDS(CUB_U32, unsigned int)
+    CUB_LABEL_BOUNDS(CUB_I32, int)
+#undef CUB_LABEL_BOUNDS
+    default: return fail(h, CUB_ERR_UNSUPPORTED, "label bounds need an integer pixel type");
+  }
+  h->launches++;
+  CU_TRY(h, cudaGetLastError());
+  CU_TRY(h, cudaMemcpyAsync(out, h->label_table.p, (size_t)n * 8 * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
+  CU_TRY(h, cudaStreamSynchronize(h->stream));
+  for (size_t i = 0; i < n; ++i) {
+    uint64_t* e = out + 8 * i;
+    if (e[0] == 0) {
+      for (int k = 1; k < 8; ++k) e[k] = 0;
+    } else {
+      for (int k = 1; k < 4; ++k) e[k] = (uint64_t)(~(uint32_t)e[k]);
+    }
+  }
+  return CUB_OK;
+}
+
+// back to the whole volume (the region index stays the caller's)
+void clear_roi(cub_handle h) {
+  if (!h->roi_on) return;
+  h->d_vol = h->full_vol;
+  for (int k = 0; k < 3; ++k) {
+    h->dims[k] = h->full_dims[k];
+    h->i0[k] -= (long long)h->roi_lo[k];
+    h->roi_lo[k] = 0;
+  }
+  h->image_nz = h->own_z1 = h->dims[2];
+  h->roi_on = false;
+}
+
+// the box [lo, lo + size) of the whole volume becomes the volume: in place when it is whole rows and slices, else a
+// copy (k_gather_box); the region index moves by lo
+int apply_roi(cub_handle h, const uint64_t lo[3], const uint64_t size[3]) {
+  clear_roi(h);
+  const uint64_t* d = h->dims;
+  const size_t pb = (size_t)h->pix_bytes;
+  if (lo[0] == 0 && lo[1] == 0 && size[0] == d[0] && size[1] == d[1]) {
+    h->full_vol = h->d_vol;
+    h->d_vol = static_cast<const unsigned char*>(h->d_vol) + (size_t)lo[2] * d[0] * d[1] * pb;
+  } else {
+    CUB_TRY(ensure(h, h->roi_buf, (size_t)size[0] * size[1] * size[2] * pb));
+    const unsigned long long rows = size[1] * size[2];
+    const unsigned blocks = (unsigned)std::min<unsigned long long>(rows, (unsigned long long)h->num_sms * 32);
+    const unsigned threads = size[0] >= 256 ? 256 : (size[0] >= 64 ? 64 : 32);
+    switch (pb) {
+#define CUB_GATHER(W)                                                                                                       \
+      k_gather_box<W><<<blocks, threads, 0, h->stream>>>(static_cast<const W*>(h->d_vol), reinterpret_cast<W*>(h->roi_buf.p), \
+                                                         d[0], d[1], lo[0], lo[1], lo[2], size[0], size[1], rows)
+      case 1: CUB_GATHER(uint8_t); break;
+      case 2: CUB_GATHER(uint16_t); break;
+      case 4: CUB_GATHER(uint32_t); break;
+      default: CUB_GATHER(unsigned long long); break;
+#undef CUB_GATHER
+    }
+    h->launches++;
+    CU_TRY(h, cudaGetLastError());
+    h->full_vol = h->d_vol;
+    h->d_vol = h->roi_buf.p;
+  }
+  for (int k = 0; k < 3; ++k) {
+    h->full_dims[k] = d[k];
+    h->roi_lo[k] = lo[k];
+    h->i0[k] += (long long)lo[k];
+  }
+  for (int k = 0; k < 3; ++k) h->dims[k] = size[k];
+  h->image_nz = h->own_z1 = size[2];
+  h->local_z0 = h->own_z0 = 0;
+  h->roi_on = true;
+  return CUB_OK;
+}
+
+// device-to-device append at `used` elements, growing the buffer (and keeping its contents) when needed
+template <typename P>
+int append(cub_handle h, DevBuf<P>& b, size_t used, const P* src, size_t n) {
+  if (n == 0) return CUB_OK;
+  if (!b.p || used + n > b.cap) {
+    const size_t cap = std::max(used + n, b.cap + b.cap / 2);
+    void* p = nullptr;
+    CU_TRY(h, cudaMalloc(&p, cap * sizeof(P)));
+    if (used) CU_TRY(h, cudaMemcpyAsync(p, b.p, used * sizeof(P), cudaMemcpyDeviceToDevice, h->stream));
+    if (b.p) {
+      CU_TRY(h, cudaStreamSynchronize(h->stream));
+      CU_TRY(h, cudaFree(b.p));
+    }
+    b.p = static_cast<P*>(p);
+    b.cap = cap;
+  }
+  CU_TRY(h, cudaMemcpyAsync(b.p + used, src, n * sizeof(P), cudaMemcpyDeviceToDevice, h->stream));
+  return CUB_OK;
+}
+
+std::string label_text(double v) {
+  char buf[32];
+  snprintf(buf, sizeof buf, "%.17g", v);
+  return buf;
+}
+
+// cub_run_labels after its checks: one bounds pass per window of 65536 label values, then count -> emit of every
+// label on its grown box with the running totals as id bases, appended to the concatenation buffers
+int run_labels(cub_handle h, const cub_params* p, const double* labels, uint64_t n, int id_bytes, uint64_t* point_offsets,
+               uint64_t* cell_offsets) {
+  std::vector<long long> sorted(n);
+  for (uint64_t i = 0; i < n; ++i) sorted[i] = (long long)labels[i];
+  std::sort(sorted.begin(), sorted.end());
+  std::vector<uint64_t> bounds(8 * (size_t)n), window;
+  for (size_t i = 0; i < sorted.size();) {
+    size_t j = i;
+    while (j < sorted.size() && sorted[j] - sorted[i] < 65536) ++j;
+    const uint32_t span = (uint32_t)(sorted[j - 1] - sorted[i] + 1);
+    window.resize(8 * (size_t)span);
+    CUB_TRY(label_bounds(h, sorted[i], span, window.data()));
+    for (size_t k = i; k < j; ++k) std::copy_n(&window[8 * (size_t)(sorted[k] - sorted[i])], 8, &bounds[8 * k]);
+    i = j;
+  }
+  const bool tri = p->generate_triangles != 0, cd = p->save_pixel_as_cell_data != 0;
+  const size_t cell_bytes = (size_t)(tri ? 3 : 4) * id_bytes;
+  const uint64_t whole[3] = {h->dims[0], h->dims[1], h->dims[2]};
+  uint64_t n_points = 0, n_cells = 0;
+  std::string warned;
+  for (uint64_t i = 0; i < n; ++i) {
+    point_offsets[i] = n_points;
+    cell_offsets[i] = n_cells;
+    const long long k = (long long)labels[i];
+    const uint64_t* b = &bounds[8 * (size_t)(std::lower_bound(sorted.begin(), sorted.end(), k) - sorted.begin())];
+    if (b[0] == 0) continue;
+    // the label's bounding box grown by one voxel and clipped to the image: the same mesh as on the whole volume
+    uint64_t lo[3], size[3];
+    for (int a = 0; a < 3; ++a) {
+      lo[a] = b[1 + a] > 0 ? b[1 + a] - 1 : 0;
+      size[a] = std::min(b[4 + a] + 1, whole[a] - 1) + 1 - lo[a];
+    }
+    CUB_TRY(apply_roi(h, lo, size));
+    h->range_on = true;
+    h->range_lo = h->range_hi = labels[i];
+    CUB_TRY(count_launch(h, p));
+    CUB_TRY(count_finish(h));
+    if (h->flags & kFlagEmptyInteriorSlice) warned += (warned.empty() ? "" : ", ") + label_text(labels[i]);
+    CUB_TRY(cub_set_id_base(h, n_points, n_cells));
+    CUB_TRY(emit_launch(h, id_bytes, true));
+    CUB_TRY(append(h, h->cat_points, 3 * (size_t)n_points, h->points.p + 3 * (size_t)h->ghost_v, 3 * (size_t)h->n_points));
+    CUB_TRY(append(h, h->cat_cells, (size_t)n_cells * cell_bytes, h->cells.p, (size_t)h->n_cells * cell_bytes));
+    if (cd) CUB_TRY(append(h, h->cat_celldata, (size_t)n_cells * h->pix_bytes, h->celldata.p, (size_t)h->n_cells * h->pix_bytes));
+    n_points += h->n_points;
+    n_cells += h->n_cells;
+  }
+  point_offsets[n] = n_points;
+  cell_offsets[n] = n_cells;
+  // the concatenation becomes the handle's result (cub_fetch, cub_device_buffers); the per-label buffers are the
+  // concatenation buffers of the next call
+  std::swap(h->points, h->cat_points);
+  std::swap(h->cells, h->cat_cells);
+  if (cd) std::swap(h->celldata, h->cat_celldata);
+  h->params = *p;
+  h->n_points = n_points;
+  h->n_cells = n_cells;
+  h->n_quads = tri ? n_cells / 2 : n_cells;
+  h->ghost_v = 0;
+  h->verts_per_cell = tri ? 3 : 4;
+  h->id_bytes = id_bytes;
+  h->count_queued = false;
+  h->counted = h->emitted = true;
+  h->emit_unverified = false;
+  h->warning = warned.empty() ? std::string() : std::string(kEmptySliceRemark) + " (label " + warned + ")";
+  return CUB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int cub_label_bounds(cub_handle h, int64_t first_label, uint32_t n_labels, uint64_t* out) {
+  if (!h) return CUB_ERR_INVALID;
+  if (!h->has_volume) return fail(h, CUB_ERR_INVALID, "cub_label_bounds before cub_set_volume");
+  long long lo = 0, hi = 0;
+  if (!integer_range(h->dtype, &lo, &hi)) return fail(h, CUB_ERR_UNSUPPORTED, "label bounds need an integer pixel type");
+  if (!out) return fail(h, CUB_ERR_INVALID, "out is null");
+  if (h->roi_on || has_slab(h)) return fail(h, CUB_ERR_INVALID, "cub_label_bounds runs on a whole volume: no region of interest or z-slab");
+  if (n_labels < 1 || n_labels > 65536) return fail(h, CUB_ERR_INVALID, "n_labels = %u is not in [1, 65536]", n_labels);
+  if (first_label < lo || first_label + (long long)n_labels - 1 > hi)
+    return fail(h, CUB_ERR_INVALID, "label window [%lld, %lld] is not inside the pixel type's range [%lld, %lld]",
+                (long long)first_label, (long long)first_label + n_labels - 1, lo, hi);
+  return label_bounds(h, first_label, n_labels, out);
+}
+
+int cub_set_region_of_interest(cub_handle h, const uint64_t lo[3], const uint64_t size[3]) {
+  if (!h) return CUB_ERR_INVALID;
+  if (!h->has_volume) return fail(h, CUB_ERR_INVALID, "cub_set_region_of_interest before cub_set_volume");
+  CU_TRY(h, cudaSetDevice(h->device));
+  h->counted = h->emitted = h->count_queued = false;
+  if (!lo) {
+    clear_roi(h);
+    return CUB_OK;
+  }
+  if (!h->roi_on && has_slab(h)) return fail(h, CUB_ERR_UNSUPPORTED, "a region of interest cannot be combined with a z-slab");
+  if (!size) return fail(h, CUB_ERR_INVALID, "size is null");
+  const uint64_t* d = h->roi_on ? h->full_dims : h->dims;
+  for (int a = 0; a < 3; ++a)
+    if (size[a] == 0 || lo[a] >= d[a] || size[a] > d[a] - lo[a])
+      return fail(h, CUB_ERR_INVALID, "region of interest [%llu, %llu + %llu) on axis %d is empty or leaves the volume (%llu)",
+                  (unsigned long long)lo[a], (unsigned long long)lo[a], (unsigned long long)size[a], a, (unsigned long long)d[a]);
+  return apply_roi(h, lo, size);
+}
+
+int cub_run_labels(cub_handle h, const cub_params* p, const double* labels, uint64_t n_labels, int id_bytes,
+                   uint64_t* point_offsets, uint64_t* cell_offsets) {
+  if (!h) return CUB_ERR_INVALID;
+  if (!h->has_volume) return fail(h, CUB_ERR_INVALID, "cub_run_labels before cub_set_volume");
+  long long lo = 0, hi = 0;
+  if (!integer_range(h->dtype, &lo, &hi)) return fail(h, CUB_ERR_UNSUPPORTED, "label meshes need an integer pixel type");
+  if (!p || (n_labels && !labels) || !point_offsets || !cell_offsets) return fail(h, CUB_ERR_INVALID, "null argument");
+  if (p->project_vertices)
+    return fail(h, CUB_ERR_INVALID, "vertex projection needs an iso-surface and a label has none: turn project_vertices off");
+  if (h->roi_on) return fail(h, CUB_ERR_INVALID, "cub_run_labels runs on the whole volume: clear the region of interest");
+  if (has_slab(h)) return fail(h, CUB_ERR_INVALID, "cub_run_labels does not run on a z-slab");
+  if (id_bytes != 4 && id_bytes != 8) return fail(h, CUB_ERR_INVALID, "id_bytes must be 4 or 8");
+  for (uint64_t i = 0; i < n_labels; ++i)
+    if (std::isnan(labels[i]) || iso_as_pixel(h->dtype, labels[i]) != labels[i])
+      return fail(h, CUB_ERR_INVALID, "label %.17g is not representable in the pixel type", labels[i]);
+  {
+    std::vector<double> s(labels, labels + n_labels);
+    std::sort(s.begin(), s.end());
+    for (size_t i = 1; i < s.size(); ++i)
+      if (s[i] == s[i - 1]) return fail(h, CUB_ERR_INVALID, "label %.17g is given twice", s[i]);
+  }
+  CU_TRY(h, cudaSetDevice(h->device));
+  const bool range_on = h->range_on;
+  const double range_lo = h->range_lo, range_hi = h->range_hi;
+  const int rc = run_labels(h, p, labels, n_labels, id_bytes, point_offsets, cell_offsets);
+  clear_roi(h);
+  h->range_on = range_on;
+  h->range_lo = range_lo;
+  h->range_hi = range_hi;
+  if (rc != CUB_OK) h->counted = h->emitted = h->count_queued = false;
+  return rc;
+}
 
 }  // extern "C"
 

@@ -22,6 +22,9 @@ class Mesh:
     points: np.ndarray
     cells: np.ndarray
     cell_data: np.ndarray | None = None
+    # SetLabelValues: label i's points and cells start at these offsets (n_labels + 1 entries, the last the totals)
+    label_point_offsets: np.ndarray | None = None
+    label_cell_offsets: np.ndarray | None = None
 
     def GetNumberOfPoints(self) -> int:
         return int(self.points.shape[0])
@@ -54,6 +57,7 @@ class CuberilleImageToMeshFilter:
         self._border_faces = False
         self._projection_method = capi.PROJECT_DEFAULT
         self._inside_range = None   # (lower, upper): range mode instead of the iso value
+        self._labels = None         # [k, ...]: every label meshed in one call (cub_run_labels)
         self._thr = 0.5
         self._step = -1.0
         self._relax = 0.95
@@ -117,6 +121,12 @@ class CuberilleImageToMeshFilter:
     def GetInsideRangeLower(self): return None if self._inside_range is None else self._inside_range[0]
     def GetInsideRangeUpper(self): return None if self._inside_range is None else self._inside_range[1]
 
+    # extension: every label of a label map in one Update() (cub_run_labels), each meshed as the range [k, k] and
+    # concatenated in the given order; the output's label_point_offsets / label_cell_offsets give each label's part.
+    # None or an empty list turns it off.
+    def SetLabelValues(self, labels): self._set("_labels", None if labels is None or len(labels) == 0 else list(labels))
+    def GetLabelValues(self): return self._labels
+
     def SetProjectVertexSurfaceDistanceThreshold(self, v):
         # itkSetClampMacro(.., 0.0, NumericTraits<InputPixelType>::max())  h:210
         hi = float("inf")
@@ -155,15 +165,28 @@ class CuberilleImageToMeshFilter:
         if self._image is None:
             raise RuntimeError("Input is not set")  # SetNumberOfRequiredInputs(1), txx:33
         img = self._image
+        if self._labels is not None:
+            if self._project:
+                raise RuntimeError("SetLabelValues meshes labels, which have no iso-surface to project onto: call "
+                                   "ProjectVerticesToIsoSurfaceOff()")
+            if self._inside_range is not None:
+                raise RuntimeError("SetLabelValues and an inside range (SetInsideRange / SetLabelValue) exclude each other: "
+                                   "call InsideRangeOff()")
+            if not np.issubdtype(img.data.dtype, np.integer):
+                raise RuntimeError("SetLabelValues needs an integer pixel type")
         if self._step < 0.0:
             self._step = max(img.spacing) * 0.25  # sticky, txx:82-85
         self._handle.set_volume(img.data, img.spacing, img.origin, img.direction)
         self._handle.set_region_index(getattr(img, "region_index", (0, 0, 0)))
         if self._inside_range is not None:
             self._handle.set_inside_range(*self._inside_range)
-        self._handle.run(self.params(), self._id_bytes)
+        offsets = (None, None)
+        if self._labels is not None:
+            offsets = self._handle.run_labels(self.params(), self._labels, self._id_bytes)
+        else:
+            self._handle.run(self.params(), self._id_bytes)
         pts, cells, cd = self._handle.fetch(self._cell_data)
-        self._output = Mesh(pts, cells, cd)
+        self._output = Mesh(pts, cells, cd, *offsets)
         self._modified = False
 
     def GetOutput(self) -> Mesh:
@@ -172,4 +195,5 @@ class CuberilleImageToMeshFilter:
     def __str__(self):  # PrintSelf, txx:501-520
         return (f"IsoSurfaceValue: {self._iso}\nGenerateTriangleFaces: {int(self._triangles)}\n"
                 f"ProjectVerticesToIsoSurface: {int(self._project)}\n"
-                + (f"InsideRange: [{self._inside_range[0]}, {self._inside_range[1]}]\n" if self._inside_range is not None else ""))
+                + (f"InsideRange: [{self._inside_range[0]}, {self._inside_range[1]}]\n" if self._inside_range is not None else "")
+                + (f"LabelValues: {' '.join(str(k) for k in self._labels)}\n" if self._labels is not None else ""))
