@@ -38,16 +38,11 @@ namespace {
 
 // tuning knobs, read from the environment ONCE per handle (cub_create) and clamped to sane values
 struct Knobs {
-  int count_cfg = -1;        // CUB_COUNT_CFG: sweep tile configuration (-1: by row length)
-  int k1_packed = 1;         // CUB_K1_PACKED: 4-bytes-per-lane classify for 8/16-bit pixels
   int k1_ctas = 32;          // CUB_K1_CTAS_PER_SM: grid cap of the classification kernel
-  int fuse = 1;              // CUB_FUSE: classification + ownership sweep in one warp-specialised kernel (k_fused.cuh)
   int fuse_tz = 0;           // CUB_FUSE_TZ: slices per sweep tile of the fused kernel (0: pick_tz)
   int fuse_ctas = 4;         // CUB_FUSE_CTAS_PER_SM
   int fuse_batch = 8;        // CUB_FUSE_BATCH: classification tasks (4 KB of a row each) per ticket and per publication
-  int pdl = -1;              // CUB_PDL: programmatic dependent launch between the kernels of a step (-1: by volume size)
   int scan_ctas = 8;         // CUB_SCAN_CTAS_PER_SM
-  int scan_rows = 1;         // CUB_SCAN_ROWS: the one-pass scan kernel for rows of at most two segments
   int proj_ctas = 6;         // CUB_PROJ_CTAS_PER_SM
   int proj_refill = 18;      // CUB_PROJ_REFILL: lanes of a warp that keep iterating before the warp serves the idle ones
 };
@@ -80,17 +75,9 @@ cudaError_t launch_sweep(SweepArgs a, cudaStream_t stream, int num_sms) {
   return cudaGetLastError();
 }
 
-cudaError_t dispatch_sweep(const SweepArgs& a, cudaStream_t st, int num_sms, int cfg_knob) {
-  // wide tiles (16 voxel words per row) for big volumes, narrow ones (8) when a row has few words
-  const int cfg = cfg_knob >= 0 ? cfg_knob : (a.g.Wx > 8 ? 2 : 10);
-  switch (cfg) {
-    case 0: return launch_sweep<SweepCfg<17, 15, 1, MODE_COUNT>>(a, st, num_sms);
-    case 1: return launch_sweep<SweepCfg<17, 15, 2, MODE_COUNT>>(a, st, num_sms);
-    case 2: return launch_sweep<SweepCfg<17, 7, 2, MODE_COUNT>>(a, st, num_sms);
-    case 3: return launch_sweep<SweepCfg<17, 7, 4, MODE_COUNT>>(a, st, num_sms);
-    default: return launch_sweep<SweepCfg<9, 14, 2, MODE_COUNT>>(a, st, num_sms);
-  }
-}
+// the sweep tile shapes: 16 voxel words per row for big volumes, 8 when a row has few words
+using WideTile = SweepCfg<17, 7, 2>;
+using NarrowTile = SweepCfg<9, 14, 2>;
 
 constexpr size_t kCtrlHead = kInfoWords + 4;  // info block, two work counters, the scan's ticket (+ pad)
 
@@ -309,34 +296,85 @@ cudaError_t launch_step(cub_handle h, void (*kern)(P...), dim3 grid, dim3 block,
   return cudaLaunchKernelEx(&cfg, kern, std::forward<A>(args)...);
 }
 
-// K1 on the local slices [z0, z1) (rows are independent), on `stream`, with at most ctas_per_sm resident CTAs
-template <typename T> struct is_packable { static constexpr bool value = false; };
-template <> struct is_packable<uint8_t> { static constexpr bool value = true; };
-template <> struct is_packable<int8_t> { static constexpr bool value = true; };
-template <> struct is_packable<uint16_t> { static constexpr bool value = true; };
-template <> struct is_packable<int16_t> { static constexpr bool value = true; };
+// The kernels of one count, chosen from the input alone (choose_count_route)
+enum class K1Route {
+  fused,   // K1 + K2a as one kernel (k_fused.cuh)
+  packed,  // k_classify_packed: 4 bytes per lane per load, for 8- and 16-bit pixels
+  full,    // k_classify<T, true>: rows of whole tasks
+  ragged,  // k_classify<T, false>
+  padded,  // k_classify_padded: image_border_faces classifies into the padded lattice
+};
 
-template <typename T, bool PACK = is_packable<T>::value>
-struct ClassifyPacked {
-  template <typename In>
-  static bool launch(cub_handle, In, const T*, uint32_t*, const Grid&, unsigned long long, unsigned long long, cudaStream_t) { return false; }
+struct CountRoute {
+  K1Route k1 = K1Route::ragged;
+  bool wide = true;         // sweep tiles of K2a and of the fused kernel's consumers: WideTile, else NarrowTile
+  FuseArgs fuse{};          // k1 == fused: its tasks, batches and tiles (the launch adds the buffers and the sweep range)
+  int fuse_tz = 0;
+  unsigned fuse_blocks = 0;
+  int scan_rows = 0;        // K2b: k_seg_scan_rows<scan_rows> for rows of one or two segments, 0: k_seg_scan
+  bool pdl_on = false;
 };
-template <typename T>
-struct ClassifyPacked<T, true> {
-  // 4 bytes per lane per load (k_classify_packed): rows must be whole warp loads and the buffer 4-byte aligned
-  template <typename In>
-  static bool launch(cub_handle h, In inside, const T* vol, uint32_t* bits, const Grid& g, unsigned long long rows,
-                     unsigned long long max_blocks, cudaStream_t stream) {
-    constexpr int vpl = 4 / (int)sizeof(T);
-    if (g.X % (32 * vpl) != 0 || (reinterpret_cast<uintptr_t>(vol) & 3u) != 0 || h->knobs.k1_packed == 0) return false;
-    const unsigned tasks_per_row = (unsigned)((g.Wx + 31) / 32);
-    const unsigned long long tasks = rows * tasks_per_row;  // cub_count checks rows * groups < 2^32
-    unsigned long long blocks = std::min<unsigned long long>((tasks + 7) / 8, max_blocks);
-    if (blocks < 1) blocks = 1;
-    k_classify_packed<T, In><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, g, inside.param(), (unsigned)tasks, tasks_per_row);
-    return true;
+
+// k_classify_packed exists for the pixel types PackedTraits (k_classify.cuh) describes
+template <typename T, typename = void> struct has_packed_kernel : std::false_type {};
+template <typename T> struct has_packed_kernel<T, std::void_t<decltype(PackedTraits<T>::is_signed)>> : std::true_type {};
+
+constexpr int kFuseStages = 3;
+
+// Everything the count phase launches, from the lattice, the pixel type and the buffer's alignment.  Needs setup_grid
+// and h->NS.
+CountRoute choose_count_route(cub_handle h) {
+  const Grid& g = h->g;
+  const int pb = h->pix_bytes;
+  const uintptr_t vol = reinterpret_cast<uintptr_t>(h->d_vol);
+  CountRoute r;
+  r.wide = g.Wx > 8;
+  r.scan_rows = h->NS <= 2 ? h->NS : 0;
+  // Programmatic dependent launch pays where the kernels are short.  Measured r2, gyroid f32, same box, off -> on:
+  // 512^3 0.456 -> 0.444 ms per step, a 132-slice slab of 1024^2 rows 0.330 -> 0.319, Marschner-Lobb 512^3 0.405 -> 0.395;
+  // 768^3 (453 M voxels) 1.112 -> 1.115, 1024^3 1.985 -> 2.02.  On below 300 M voxels per handle.
+  r.pdl_on = (unsigned long long)g.X * g.Y * g.Zl < 300000000ull;
+
+  bool packable = false;
+  DISPATCH_PIXEL(h->dtype, packable = has_packed_kernel<T>::value);
+  // k_classify_packed: rows must be whole warp loads and the buffer 4-byte aligned
+  const bool packed = !h->pad && packable && g.X % (32 * (4 / pb)) == 0 && (vol & 3u) == 0;
+  // the fused kernel: TMA bulk copies of 16-byte aligned rows; 8- and 16-bit pixels keep the packed kernel where it applies
+  if (!h->pad && !packed && ((size_t)g.X * pb) % 16 == 0 && (vol & 15u) == 0) {
+    FuseArgs& fa = r.fuse;
+    const int wpt = kFuseStageBytes / (32 * pb);  // voxel words per task
+    fa.groups_per_row = (unsigned)((g.Wx + wpt - 1) / wpt);
+    fa.tasks_per_slice = fa.groups_per_row * (unsigned)g.Y;
+    const unsigned long long tasks = (unsigned long long)fa.tasks_per_slice * (unsigned long long)g.Zl;
+    // tasks per ticket / per publication: what the producer warps have in flight (2368 warps x batch x 4 KB) is how far
+    // the consumers run behind, i.e. how long the bitmask words must survive in L2; a publication costs a release fence.
+    // Measured on 1024^3 f32: 6 -> 0.842, 8 -> 0.831, 12 -> 0.839, 16 -> 0.856, 32 -> 0.895, 64 -> 0.924 ms.
+    fa.batch = (unsigned)h->knobs.fuse_batch;
+    const int txw = r.wide ? WideTile::TXW : NarrowTile::TXW, ty = r.wide ? WideTile::TY : NarrowTile::TY;
+    const int gx = (g.Wx + txw - 1) / txw, gy = (g.Y + ty - 1) / ty;
+    const int nz = h->zs1 - h->owner_z_min;
+    // short sweeps: a tile can only start when the slice above its last one is classified, and what is still to sweep
+    // when the producers finish is the kernel's tail; the two warm-up planes per tile cost issue slots the kernel has
+    r.fuse_tz = std::min(h->knobs.fuse_tz > 0 ? h->knobs.fuse_tz : 8, pick_tz(gx, gy, nz, h->num_sms));
+    const unsigned long long tiles = (unsigned long long)gx * gy * ((nz + r.fuse_tz - 1) / r.fuse_tz);
+    if (tasks < (1ull << 32) - 256 && tiles < (1ull << 31)) {
+      fa.n_tasks = (unsigned)tasks;
+      fa.n_batches = (unsigned)((tasks + fa.batch - 1) / fa.batch);
+      fa.n_tiles = (unsigned)tiles; fa.gx = (unsigned)gx; fa.gy = (unsigned)gy;
+      // persistent: every CTA resident (4 per SM: 64 registers x 256 threads, ~47 KB of shared memory)
+      const unsigned long long want = std::max<unsigned long long>((fa.n_batches + 3) / 4, fa.n_tiles);
+      r.fuse_blocks = (unsigned)std::max<unsigned long long>(
+          1, std::min<unsigned long long>(want, (unsigned long long)h->num_sms * h->knobs.fuse_ctas));
+      r.k1 = K1Route::fused;
+      return r;
+    }
   }
-};
+  if (h->pad) r.k1 = K1Route::padded;
+  else if (packed) r.k1 = K1Route::packed;
+  else if (g.X % 32 == 0 && g.Wx % kWordsPerTask == 0) r.k1 = K1Route::full;
+  else r.k1 = K1Route::ragged;
+  return r;
+}
 
 // The inside predicate of the handle's mode, in the pixel type, handed to f: every classification route is instantiated
 // for both (k_classify.cuh), and iso mode keeps its own instantiations rather than running as a range.
@@ -345,101 +383,57 @@ auto with_inside(cub_handle h, F&& f) {
   return h->range_on ? f(Between<T>{(T)h->range_lo, (T)h->range_hi}) : f(AtLeast<T>{(T)h->params.iso_value});
 }
 
-template <typename T, typename In>
-void launch_classify(cub_handle h, In inside, int z0, int z1, cudaStream_t stream, int ctas_per_sm) {
-  const unsigned long long max_blocks = (unsigned long long)h->num_sms * ctas_per_sm;
-  h->launches++;
-  if (h->pad) {
-    // the padded lattice (image_border_faces): z0 / z1 are lattice slices
-    const Grid& gb = h->g;
-    const Grid& gv = h->gv;
-    const unsigned long long words = (unsigned long long)gb.Wx * gb.Y * (z1 - z0);  // < 2^32: checked by cub_count
-    const unsigned long long blocks = std::max<unsigned long long>(1, std::min((words + 7) / 8, max_blocks));
-    uint32_t* bits = h->bits.p + (size_t)z0 * gb.Y * gb.Wp;
-    // slice z0 of the launch is lattice slice z0: the kernel's z origin moves with it
-    const T* vol = static_cast<const T*>(h->d_vol);
-    Grid sub = gb;
-    k_classify_padded<T, In><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, sub, gv.X, gv.Y, gv.Zl, h->zpad_lo - z0,
-                                                                    inside.param(), (unsigned)words);
-    return;
-  }
-  Grid g = h->g;
-  const unsigned groups = (unsigned)((g.Wx + kWordsPerTask - 1) / kWordsPerTask);
-  const unsigned long long rows = (unsigned long long)g.Y * (z1 - z0);
-  const unsigned tasks = (unsigned)(rows * groups);  // dims < 2^31 and cub_count checks rows*groups < 2^32
-  unsigned long long blocks = ((unsigned long long)tasks + 7) / 8;
-  if (blocks > max_blocks) blocks = max_blocks;
-  if (blocks < 1) blocks = 1;
-  const bool full = (g.X % 32 == 0) && (g.Wx % kWordsPerTask == 0);
-  const T* vol = static_cast<const T*>(h->d_vol) + (size_t)z0 * g.Y * g.X;
-  uint32_t* bits = h->bits.p + (size_t)z0 * g.Y * g.Wp;
-  if (ClassifyPacked<T>::launch(h, inside, vol, bits, g, rows, max_blocks, stream)) return;
-  if (full)
-    k_classify<T, true, In><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, g, inside.param(), tasks, groups);
-  else
-    k_classify<T, false, In><<<(unsigned)blocks, 256, 0, stream>>>(vol, bits, g, inside.param(), tasks, groups);
-}
-
-// K1 + K2a as one kernel (k_fused.cuh).  Returns false (nothing launched) where the fused kernel does not apply: the
-// caller then runs the two kernels one after the other.
-constexpr int kFuseStages = 3;
-
 template <typename T, typename C, typename In>
-bool launch_fused_cfg(cub_handle h, In inside, const SweepArgs& ca, unsigned* ctr, unsigned* done) {
+cudaError_t launch_fused(cub_handle h, In inside, const CountRoute& r, const SweepArgs& ca) {
   using Smem = FuseSmem<C, kFuseStages>;
-  constexpr int WPT = kFuseStageBytes / (32 * (int)sizeof(T));
-  const Grid& g = ca.g;
-  FuseArgs fa{};
+  FuseArgs fa = r.fuse;
   fa.sw = ca;
+  fa.sw.tz = r.fuse_tz;
   fa.vol = h->d_vol;
   fa.bits = h->bits.p;
-  fa.groups_per_row = (unsigned)((g.Wx + WPT - 1) / WPT);
-  fa.tasks_per_slice = fa.groups_per_row * (unsigned)g.Y;
-  const unsigned long long tasks = (unsigned long long)fa.tasks_per_slice * (unsigned long long)g.Zl;
-  if (tasks >= (1ull << 32) - 256) return false;
-  fa.n_tasks = (unsigned)tasks;
-  // tasks per ticket / per publication: what the producer warps have in flight (2368 warps x batch x 4 KB) is how far
-  // the consumers run behind, i.e. how long the bitmask words must survive in L2; a publication costs a release fence.
-  // Measured on 1024^3 f32: 6 -> 0.842, 8 -> 0.831, 12 -> 0.839, 16 -> 0.856, 32 -> 0.895, 64 -> 0.924 ms.
-  fa.batch = (unsigned)h->knobs.fuse_batch;
-  fa.n_batches = (unsigned)((tasks + fa.batch - 1) / fa.batch);
-  const int gx = (g.Wx + C::TXW - 1) / C::TXW, gy = (g.Y + C::TY - 1) / C::TY;
-  const int nz = ca.z_end - ca.z_begin;
-  // short sweeps: a tile can only start when the slice above its last one is classified, and what is still to sweep
-  // when the producers finish is the kernel's tail; the two warm-up planes per tile cost issue slots the kernel has
-  fa.sw.tz = std::min(h->knobs.fuse_tz > 0 ? h->knobs.fuse_tz : 8, pick_tz(gx, gy, nz, h->num_sms));
-  const unsigned long long tiles = (unsigned long long)gx * gy * ((nz + fa.sw.tz - 1) / fa.sw.tz);
-  if (tiles >= (1ull << 31)) return false;
-  fa.n_tiles = (unsigned)tiles; fa.gx = (unsigned)gx; fa.gy = (unsigned)gy;
-  fa.ctr = ctr; fa.done = done;
+  fa.ctr = h->d_fuse_ctr; fa.done = h->d_fuse_done;
   auto kern = k_classify_sweep<T, C, kFuseStages, In>;
   // (set on every launch: the attribute belongs to the current device, and one process may drive several)
-  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)) != cudaSuccess) {
-    cudaGetLastError();
-    return false;
-  }
-  // persistent: every CTA resident (4 per SM: 64 registers x 256 threads, ~47 KB of shared memory)
-  const unsigned long long want = std::max<unsigned long long>((fa.n_batches + 3) / 4, fa.n_tiles);
-  const unsigned blocks = (unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>(want, (unsigned long long)h->num_sms * h->knobs.fuse_ctas));
-  kern<<<blocks, kFuseThreads, sizeof(Smem), h->stream>>>(fa, inside.param());
+  const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
+  if (e != cudaSuccess) return e;
+  kern<<<r.fuse_blocks, kFuseThreads, sizeof(Smem), h->stream>>>(fa, inside.param());
   h->launches++;
-  return true;
+  return cudaGetLastError();
 }
 
+// K1 of the route on every local slice (rows are independent), with at most k1_ctas resident CTAs per SM; where the
+// route fuses it, K1 + K2a
 template <typename T, typename In>
-bool launch_fused(cub_handle h, In inside, const SweepArgs& ca, int cfg, unsigned* ctr, unsigned* done) {
-  if (!h->knobs.fuse || h->pad) return false;
-  const Grid& g = ca.g;
-  // 8- and 16-bit pixels keep their own classification kernel (4 pixels per lane per load) where it applies
-  if (is_packable<T>::value && h->knobs.k1_packed && g.X % (32 * (4 / (int)sizeof(T))) == 0 &&
-      (reinterpret_cast<uintptr_t>(h->d_vol) & 3u) == 0)
-    return false;
-  // TMA bulk copies: 16-byte aligned rows
-  if (((size_t)g.X * sizeof(T)) % 16 != 0 || (reinterpret_cast<uintptr_t>(h->d_vol) & 15u) != 0) return false;
-  const int c = cfg >= 0 ? cfg : (g.Wx > 8 ? 2 : 10);
-  if (c == 2) return launch_fused_cfg<T, SweepCfg<17, 7, 2, MODE_COUNT>>(h, inside, ca, ctr, done);
-  if (c == 10) return launch_fused_cfg<T, SweepCfg<9, 14, 2, MODE_COUNT>>(h, inside, ca, ctr, done);
-  return false;
+cudaError_t launch_k1(cub_handle h, In inside, const CountRoute& r, const SweepArgs& ca) {
+  if (r.k1 == K1Route::fused)
+    return r.wide ? launch_fused<T, WideTile>(h, inside, r, ca) : launch_fused<T, NarrowTile>(h, inside, r, ca);
+  const Grid& g = h->g;
+  const T* vol = static_cast<const T*>(h->d_vol);
+  const unsigned long long rows = (unsigned long long)g.Y * g.Zl;
+  const unsigned long long max_blocks = (unsigned long long)h->num_sms * h->knobs.k1_ctas;
+  auto blocks = [&](unsigned long long work) { return (unsigned)std::max(1ull, std::min((work + 7) / 8, max_blocks)); };
+  h->launches++;
+  if (r.k1 == K1Route::padded) {
+    // g is the padded lattice, gv the voxel buffer
+    const unsigned long long words = (unsigned long long)g.Wx * rows;  // < 2^32: checked by cub_count
+    k_classify_padded<T, In><<<blocks(words), 256, 0, h->stream>>>(vol, h->bits.p, g, h->gv.X, h->gv.Y, h->gv.Zl,
+                                                                   h->zpad_lo, inside.param(), (unsigned)words);
+  } else if (r.k1 == K1Route::packed) {
+    if constexpr (has_packed_kernel<T>::value) {  // (the only pixel types choose_count_route gives this route)
+      const unsigned tasks_per_row = (unsigned)((g.Wx + 31) / 32);
+      const unsigned long long tasks = rows * tasks_per_row;  // cub_count checks rows * groups < 2^32
+      k_classify_packed<T, In><<<blocks(tasks), 256, 0, h->stream>>>(vol, h->bits.p, g, inside.param(), (unsigned)tasks,
+                                                                     tasks_per_row);
+    }
+  } else {
+    const unsigned groups = (unsigned)((g.Wx + kWordsPerTask - 1) / kWordsPerTask);
+    const unsigned tasks = (unsigned)(rows * groups);  // dims < 2^31 and cub_count checks rows*groups < 2^32
+    if (r.k1 == K1Route::full)
+      k_classify<T, true, In><<<blocks(tasks), 256, 0, h->stream>>>(vol, h->bits.p, g, inside.param(), tasks, groups);
+    else
+      k_classify<T, false, In><<<blocks(tasks), 256, 0, h->stream>>>(vol, h->bits.p, g, inside.param(), tasks, groups);
+  }
+  return cudaGetLastError();
 }
 
 // capacities of the result buffers, for k_check_caps (and the early record loads of k_vertices)
@@ -567,16 +561,11 @@ int cub_create(int device, void* stream, cub_handle* out) {
     int sms = 0;
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) == cudaSuccess && sms > 0) h->num_sms = sms;
     // the tuning knobs are read here, once, and clamped (a zero would make a launch with no blocks)
-    h->knobs.count_cfg = env_int("CUB_COUNT_CFG", -1, -1, 10);
-    h->knobs.k1_packed = env_int("CUB_K1_PACKED", 1, 0, 1);
     h->knobs.k1_ctas = env_int("CUB_K1_CTAS_PER_SM", 32, 1, 32);
-    h->knobs.fuse = env_int("CUB_FUSE", 1, 0, 1);
     h->knobs.fuse_tz = env_int("CUB_FUSE_TZ", 0, 0, 32);
     h->knobs.fuse_ctas = env_int("CUB_FUSE_CTAS_PER_SM", 4, 1, 4);
-    h->knobs.pdl = env_int("CUB_PDL", -1, -1, 1);
     h->knobs.fuse_batch = env_int("CUB_FUSE_BATCH", 8, 1, 256);
     h->knobs.scan_ctas = env_int("CUB_SCAN_CTAS_PER_SM", 8, 1, 32);
-    h->knobs.scan_rows = env_int("CUB_SCAN_ROWS", 1, 0, 1);
     h->knobs.proj_ctas = env_int("CUB_PROJ_CTAS_PER_SM", 6, 1, 16);
     h->knobs.proj_refill = env_int("CUB_PROJ_REFILL", 18, 1, 32);
   }
@@ -845,6 +834,7 @@ int count_launch(cub_handle h, const cub_params* p) {
   // K2 scan range = voxel slices [owner_z_min, zs1) and corner planes [zs0, zs1]
   const size_t row_begin = (size_t)h->owner_z_min * h->EY;
   const size_t n_rows = (size_t)(h->zs1 + 1 - h->owner_z_min) * h->EY;
+  const CountRoute route = choose_count_route(h);
   // one large scan tile per resident CTA, so that every tile is in flight when the look-backs run; rows with at most
   // two segments take the one-pass kernel, whose warps hold at most 32 * kScanBatches rows (more tiles than resident
   // CTAs are fine: a tile only waits for tiles with earlier tickets)
@@ -853,8 +843,7 @@ int count_launch(cub_handle h, const cub_params* p) {
   const size_t max_tiles = (size_t)h->num_sms * std::max(1, std::min(scan_occ, h->knobs.scan_ctas));
   size_t rows_per_tile = ((n_rows + max_tiles - 1) / max_tiles + kScanWarps - 1) / kScanWarps * kScanWarps;
   if (rows_per_tile < (size_t)kScanWarps) rows_per_tile = kScanWarps;
-  const bool scan_rows = h->NS <= 2 && h->knobs.scan_rows;
-  if (scan_rows) rows_per_tile = std::min<size_t>(rows_per_tile, (size_t)kScanWarps * 32 * kScanBatches);
+  if (route.scan_rows) rows_per_tile = std::min<size_t>(rows_per_tile, (size_t)kScanWarps * 32 * kScanBatches);
   const size_t n_tiles = (n_rows + rows_per_tile - 1) / rows_per_tile;
   {
     const size_t slice_words = ((size_t)g.Zl + 2 + 1) / 2;  // one u32 per slice
@@ -873,31 +862,23 @@ int count_launch(cub_handle h, const cub_params* p) {
   ca.cnt = h->cnt.p; ca.act = h->act.p; ca.own = h->raster ? nullptr : h->own.p;
   ca.slice_any = h->d_slice_any;
   {
-    // Programmatic dependent launch pays where the kernels are short.  Measured r2, gyroid f32, same box, off -> on:
-    // 512^3 0.456 -> 0.444 ms per step, a 132-slice slab of 1024^2 rows 0.330 -> 0.319, Marschner-Lobb 512^3 0.405 -> 0.395;
-    // 768^3 (453 M voxels) 1.112 -> 1.115, 1024^3 1.985 -> 2.02.  On below 300 M voxels per handle.
-    h->pdl_on = h->knobs.pdl < 0 ? (unsigned long long)g.X * g.Y * g.Zl < 300000000ull : h->knobs.pdl != 0;
-    // K1 + K2a: one warp-specialised kernel where it applies (k_fused.cuh), else K1 then K2a on the handle's stream.
-    // The control block (tickets, per-slice progress, scan descriptors, slice occupancy) is cleared first.
+    h->pdl_on = route.pdl_on;
+    // K1 + K2a: one warp-specialised kernel where the route fuses them (k_fused.cuh), else K1 then K2a on the handle's
+    // stream.  The control block (tickets, per-slice progress, scan descriptors, slice occupancy) is cleared first.
     CU_TRY(h, cudaMemsetAsync(h->ctrl.p, 0, h->ctrl_used * sizeof(unsigned long long), h->stream));
     ca.z_begin = h->owner_z_min; ca.z_end = h->zs1;
-    bool fused = false;
     {
       Timer t(h, 0);
-      DISPATCH_PIXEL(h->dtype, (fused = with_inside<T>(h, [&](auto in) {
-                       return launch_fused<T>(h, in, ca, h->knobs.count_cfg, h->d_fuse_ctr, h->d_fuse_done);
-                     })));
-      CU_TRY(h, cudaGetLastError());
-      if (!fused) {
-        DISPATCH_PIXEL(h->dtype, (with_inside<T>(h, [&](auto in) { launch_classify<T>(h, in, 0, g.Zl, h->stream, h->knobs.k1_ctas); })));
-        CU_TRY(h, cudaGetLastError());
-      }
+      cudaError_t k1_launch = cudaSuccess;
+      DISPATCH_PIXEL(h->dtype, (k1_launch = with_inside<T>(h, [&](auto in) { return launch_k1<T>(h, in, route, ca); })));
+      CU_TRY(h, k1_launch);
       t.stop();
     }
-    h->fused_last = fused;
+    h->fused_last = route.k1 == K1Route::fused;
     if (h->timing) cudaEventRecord(h->ev[0], h->stream);
-    if (!fused) {
-      CU_TRY(h, dispatch_sweep(ca, h->stream, h->num_sms, h->knobs.count_cfg));
+    if (!h->fused_last) {
+      CU_TRY(h, route.wide ? launch_sweep<WideTile>(ca, h->stream, h->num_sms)
+                           : launch_sweep<NarrowTile>(ca, h->stream, h->num_sms));
       h->launches++;
     }
   }
@@ -914,8 +895,8 @@ int count_launch(cub_handle h, const cub_params* p) {
     sa.mark_row_c = (h->own_z0 > 0) ? (unsigned)((size_t)(h->zs0 + 1) * h->EY) : 0xffffffffu;
     sa.rows_per_tile = (unsigned)rows_per_tile; sa.n_tiles = (unsigned)n_tiles;
     sa.status = h->d_status; sa.ticket = h->d_ticket; sa.info = h->d_info;
-    if (scan_rows && h->NS == 1) CU_TRY(h, launch_step(h, k_seg_scan_rows<1>, dim3((unsigned)n_tiles), dim3(kScanThreads), true, sa));
-    else if (scan_rows) CU_TRY(h, launch_step(h, k_seg_scan_rows<2>, dim3((unsigned)n_tiles), dim3(kScanThreads), true, sa));
+    if (route.scan_rows == 1) CU_TRY(h, launch_step(h, k_seg_scan_rows<1>, dim3((unsigned)n_tiles), dim3(kScanThreads), true, sa));
+    else if (route.scan_rows == 2) CU_TRY(h, launch_step(h, k_seg_scan_rows<2>, dim3((unsigned)n_tiles), dim3(kScanThreads), true, sa));
     else CU_TRY(h, launch_step(h, k_seg_scan, dim3((unsigned)n_tiles), dim3(kScanThreads), true, sa));
     CU_TRY(h, launch_step(h, k_finalize_info, dim3(1), dim3(256), true, h->d_info, h->raster ? 1 : 0, (const uint32_t*)h->d_slice_any,
                           h->owner_z_min, h->zs1));

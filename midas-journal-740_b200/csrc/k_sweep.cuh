@@ -29,8 +29,6 @@
 
 namespace cbr {
 
-enum { MODE_COUNT = 0 };
-
 struct SweepArgs {
   const uint32_t* bits;
   Grid g;
@@ -46,9 +44,9 @@ struct SweepArgs {
   uint32_t* slice_any;  // [Zl] set to 1 where voxel slice z has an inside voxel (the empty-interior-slice check), may be null
 };
 
-template <int NTX_, int NTY_, int R_, int MODE_>
+template <int NTX_, int NTY_, int R_>
 struct SweepCfg {
-  static constexpr int NTX = NTX_, NTY = NTY_, R = R_, MODE = MODE_;
+  static constexpr int NTX = NTX_, NTY = NTY_, R = R_;
   static constexpr int NT = NTX * NTY;               // live threads
   static constexpr int NTP = (NT + 31) / 32 * 32;    // launched threads
   static constexpr int NW = NTP / 32;
@@ -90,7 +88,7 @@ __device__ __forceinline__ void corner_owners(const uint32_t in[8], uint32_t vm,
 template <typename C, bool FUSED>
 __device__ __forceinline__ void sweep_tile(const SweepArgs& a, SweepSmem<C>& sm, const int t, const int bx, const int by,
                                            const int bz) {
-  constexpr int NTX = C::NTX, NTY = C::NTY, R = C::R, MODE = C::MODE, NT = C::NT, CR = C::CR;
+  constexpr int NTX = C::NTX, NTY = C::NTY, R = C::R, NT = C::NT, CR = C::CR;
   const Grid& g = a.g;
   const bool alive = t < NT;
   const int tt = alive ? t : 0;
@@ -265,47 +263,45 @@ __device__ __forceinline__ void sweep_tile(const SweepArgs& a, SweepSmem<C>& sm,
         O[7] = f1;
       };
 
-      if (MODE == MODE_COUNT) {
-        uint32_t* __restrict__ cntz = a.cnt + (size_t)z * plane_entries;
-        uint32_t* __restrict__ actz = a.act + (size_t)z * plane_entries;
+      uint32_t* __restrict__ cntz = a.cnt + (size_t)z * plane_entries;
+      uint32_t* __restrict__ actz = a.act + (size_t)z * plane_entries;
+#pragma unroll
+      for (int k = 0; k < R; ++k) {
+        const bool vox = (rowok_bits >> k) & 1u, cor = (corner_bits >> k) & 1u;
+        if (!(vox || cor)) continue;
+        uint32_t packed = 0;
+        if (vox) {
+          uint32_t O[8];
+          assemble(k, O);
+          const uint32_t c = lo_c[k + 1] & vc;
+          const uint32_t nf = __popc(c & ~lo_l[k + 1]) + __popc(c & ~lo_c[k]) +
+                              __popc(c & ~__funnelshift_r(lo_c[k + 1], nr >> (5 * k + 4), 1)) +
+                              __popc(c & ~((k == R - 1) ? upc : lo_c[(k == R - 1) ? 0 : k + 2])) +
+                              __popc(c & ~below_c[k]) + __popc(c & ~hi_c[k + 1]);
+          uint32_t nv = 0;
+#pragma unroll
+          for (int l = 0; l < 8; ++l) nv += __popc(O[l]);
+          packed = nv | (nf << 10);
+          // (r2 also tried two 16-byte half records, each written only where it has a bit: fewer bytes stored, but a
+          //  16-byte store leaves half a 32-byte L2 sector to be filled from DRAM - the fused kernel went 0.88 -> 0.98 ms)
+          if (nv && a.own) {  // k_assign walks these instead of sweeping again
+            uint4* __restrict__ o = a.own + 2 * ((size_t)z * plane_entries + (size_t)(e0 + k * a.EW));
+            __stcs(o, make_uint4(O[0], O[1], O[2], O[3]));
+            __stcs(o + 1, make_uint4(O[4], O[5], O[6], O[7]));
+          }
+        }
+        if (cor) {
+          packed |= (uint32_t)__popc(act_prev[k]) << 20;
+          actz[e0 + k * a.EW] = act_prev[k];
+        }
+        cntz[e0 + k * a.EW] = packed;
+      }
+      if (cz == ze && ze == a.z_end) {  // the top corner plane of the range has no voxel slice of its own
 #pragma unroll
         for (int k = 0; k < R; ++k) {
-          const bool vox = (rowok_bits >> k) & 1u, cor = (corner_bits >> k) & 1u;
-          if (!(vox || cor)) continue;
-          uint32_t packed = 0;
-          if (vox) {
-            uint32_t O[8];
-            assemble(k, O);
-            const uint32_t c = lo_c[k + 1] & vc;
-            const uint32_t nf = __popc(c & ~lo_l[k + 1]) + __popc(c & ~lo_c[k]) +
-                                __popc(c & ~__funnelshift_r(lo_c[k + 1], nr >> (5 * k + 4), 1)) +
-                                __popc(c & ~((k == R - 1) ? upc : lo_c[(k == R - 1) ? 0 : k + 2])) +
-                                __popc(c & ~below_c[k]) + __popc(c & ~hi_c[k + 1]);
-            uint32_t nv = 0;
-#pragma unroll
-            for (int l = 0; l < 8; ++l) nv += __popc(O[l]);
-            packed = nv | (nf << 10);
-            // (r2 also tried two 16-byte half records, each written only where it has a bit: fewer bytes stored, but a
-            //  16-byte store leaves half a 32-byte L2 sector to be filled from DRAM - the fused kernel went 0.88 -> 0.98 ms)
-            if (nv && a.own) {  // k_assign walks these instead of sweeping again
-              uint4* __restrict__ o = a.own + 2 * ((size_t)z * plane_entries + (size_t)(e0 + k * a.EW));
-              __stcs(o, make_uint4(O[0], O[1], O[2], O[3]));
-              __stcs(o + 1, make_uint4(O[4], O[5], O[6], O[7]));
-            }
-          }
-          if (cor) {
-            packed |= (uint32_t)__popc(act_prev[k]) << 20;
-            actz[e0 + k * a.EW] = act_prev[k];
-          }
-          cntz[e0 + k * a.EW] = packed;
-        }
-        if (cz == ze && ze == a.z_end) {  // the top corner plane of the range has no voxel slice of its own
-#pragma unroll
-          for (int k = 0; k < R; ++k) {
-            if ((corner_bits >> k) & 1u) {
-              (a.cnt + (size_t)cz * plane_entries)[e0 + k * a.EW] = (uint32_t)__popc(act[k]) << 20;
-              (a.act + (size_t)cz * plane_entries)[e0 + k * a.EW] = act[k];
-            }
+          if ((corner_bits >> k) & 1u) {
+            (a.cnt + (size_t)cz * plane_entries)[e0 + k * a.EW] = (uint32_t)__popc(act[k]) << 20;
+            (a.act + (size_t)cz * plane_entries)[e0 + k * a.EW] = act[k];
           }
         }
       }

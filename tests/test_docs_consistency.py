@@ -6,13 +6,18 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CAPI = os.path.join(ROOT, "midas-journal-740_b200", "csrc", "cuberille_capi.cu")
 
 
-def test_every_tuning_knob_is_documented_and_read_once():
+def documented_knobs():
+    """the variables named in the first column of INTEGRATION.md's tuning-knob table"""
+    doc = open(os.path.join(ROOT, "INTEGRATION.md")).read()
+    table = doc[doc.index("## Tuning knobs"):]
+    table = table[:table.index("\n\n", table.index("|"))]
+    return {n for row in table.splitlines() if row.startswith("| `") for n in re.findall(r"`(CUB_[A-Z0-9_]+)`", row.split("|")[1])}
+
+
+def test_the_knobs_cub_create_reads_are_the_documented_ones():
     src = open(CAPI).read()
     knobs = re.findall(r'env_int\("(CUB_[A-Z0-9_]+)",\s*(-?\d+)', src)
-    assert len(knobs) >= 10
-    doc = open(os.path.join(ROOT, "INTEGRATION.md")).read()
-    for name, default in knobs:
-        assert f"`{name}`" in doc, f"{name} is read by cub_create but missing from INTEGRATION.md"
+    assert {n for n, _ in knobs} == documented_knobs(), "the knobs cub_create reads and INTEGRATION.md's table differ"
     # the environment is read in cub_create only (VERDICT r1: no getenv on the hot path): env_int's own getenv is the one call
     assert src.count("getenv(") == 1
     create = src[src.index("int cub_create("):]
@@ -21,7 +26,7 @@ def test_every_tuning_knob_is_documented_and_read_once():
         assert name in create, f"{name} is not read in cub_create"
 
 
-def test_every_switch_the_tests_and_tools_set_is_read_by_the_library():
+def test_no_test_or_tool_sets_a_switch_the_library_does_not_read():
     """a test that sets a variable the library no longer reads runs the same path twice and checks nothing"""
     src = open(CAPI).read()
     read = set(re.findall(r'env_int\("(CUB_[A-Z0-9_]+)"', src))
@@ -37,7 +42,7 @@ def test_every_switch_the_tests_and_tools_set_is_read_by_the_library():
                 for name in re.findall(r"\bCUB_[A-Z0-9_]+\b", open(path, errors="replace").read()):
                     named.setdefault(name, os.path.relpath(path, ROOT))
     switches = {n: p for n, p in named.items() if n not in api}
-    assert "CUB_FUSE" in switches and "CUB_K1_PACKED" in switches
+    assert "CUB_FUSE_TZ" in switches and "CUB_FUSE_CTAS_PER_SM" in switches
     stale = {n: p for n, p in switches.items() if n not in read and n not in allowed}
     assert not stale, f"variables named under tests/ or tools/ that cuberille_capi.cu does not read: {stale}"
 

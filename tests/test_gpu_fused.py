@@ -1,11 +1,13 @@
 """GPU: the fused classification + ownership-sweep kernel (csrc/k_fused.cuh) against the oracle and against the
-two-kernel path it replaces (CUB_FUSE=0), bit for bit.  The knob is read once per handle in cub_create, so both
-paths can run in one process."""
+two-kernel path it replaces, bit for bit.  The two-kernel path runs on the same volume as a device pointer one pixel
+past a 16-byte boundary, where the fused kernel cannot run.  The tuning knobs are read once per handle in cub_create,
+so several settings can run in one process."""
 import os
 
 import numpy as np
 import pytest
 
+from test_gpu_pixel_edges import set_route_volume
 from util import assert_mesh_equal, gyroid, oracle, pkg, random_volume
 
 pytestmark = pytest.mark.gpu
@@ -28,16 +30,14 @@ class _env:
                 os.environ[k] = v
 
 
-def _handle(fuse, **env):
-    with _env(CUB_FUSE=int(fuse), **env):
+def _handle(**env):
+    with _env(**env):
         return pkg().capi.Handle(0)
 
 
-def _run(h, vol, iso, tri=False, slab=None, spacing=(1.0, 1.0, 1.0)):
+def _run(h, vol, iso, tri=False, two_kernel=False):
     P = pkg()
-    h.set_volume(vol, spacing)
-    if slab is not None:
-        h.set_slab(*slab)
+    buf = set_route_volume(h, vol, misaligned=two_kernel)
     p = P.capi.default_params()
     p.iso_value, p.generate_triangles, p.project_vertices = float(iso), int(tri), 0
     h.count(p)
@@ -45,6 +45,7 @@ def _run(h, vol, iso, tri=False, slab=None, spacing=(1.0, 1.0, 1.0)):
     bits = h.bitmask().copy()
     h.emit(4)
     pts, cells, _ = h.fetch()
+    del buf
     return fused, bits, pts, cells
 
 
@@ -56,13 +57,13 @@ def _run(h, vol, iso, tri=False, slab=None, spacing=(1.0, 1.0, 1.0)):
     (np.float32, (1, 1, 8)), (np.float64, (11, 14, 258)), (np.float64, (6, 9, 30)), (np.int32, (13, 21, 300)),
     (np.uint32, (8, 8, 512)), (np.uint8, (9, 10, 48)), (np.int16, (9, 10, 40)), (np.uint16, (5, 4, 1048)),
 ])
-def test_fused_equals_oracle_and_the_two_kernel_path(dtype, shape):
+def test_fused_equals_oracle_and_the_unaligned_two_kernel_path(dtype, shape):
     O = oracle()
     vol, iso = random_volume(shape, dtype, seed=shape[2] + shape[0], fill=0.5)
-    hf, hu = _handle(1), _handle(0)
+    hf, hu = _handle(), _handle()
     for tri in (False, True):
         ff, bf, pf, cf = _run(hf, vol, iso, tri)
-        fu, bu, pu, cu = _run(hu, vol, iso, tri)
+        fu, bu, pu, cu = _run(hu, vol, iso, tri, two_kernel=True)
         assert ff and not fu, (ff, fu)
         assert np.array_equal(bf, bu), "bitmask differs between the fused and the two-kernel path"
         assert np.array_equal(pf.view(np.uint32), pu.view(np.uint32)) and np.array_equal(cf, cu)
@@ -73,16 +74,17 @@ def test_fused_equals_oracle_and_the_two_kernel_path(dtype, shape):
     hu.close()
 
 
-@pytest.mark.parametrize("env", [dict(), dict(CUB_FUSE_TZ=4), dict(CUB_FUSE_TZ=7, CUB_FUSE_CTAS_PER_SM=1), dict(CUB_COUNT_CFG=10),
-                                 dict(CUB_COUNT_CFG=2)])
-def test_fused_large_noise_volume_equals_the_two_kernel_path(env):
+# rows of 33 voxel words sweep wide tiles, rows of 7 narrow ones (cuberille_capi.cu: choose_count_route)
+@pytest.mark.parametrize("shape", [(150, 210, 1040), (400, 420, 200)])
+@pytest.mark.parametrize("env", [dict(), dict(CUB_FUSE_TZ=4), dict(CUB_FUSE_TZ=7, CUB_FUSE_CTAS_PER_SM=1)])
+def test_fused_large_noise_volume_equals_the_two_kernel_path(env, shape):
     """many tiles, many z chunks, consumers that overtake the producers: everything the count phase leaves behind must
     be identical (mesh, bitmask), on a volume the oracle would need minutes for"""
-    vol, iso = random_volume((150, 210, 1040), np.float32, seed=5, fill=0.35)
-    hf, hu = _handle(1, **env), _handle(0)
+    vol, iso = random_volume(shape, np.float32, seed=5, fill=0.35)
+    hf, hu = _handle(**env), _handle()
     for rep in range(2):  # the second run reuses the control block (tickets, progress counters)
         ff, bf, pf, cf = _run(hf, vol, iso)
-        fu, bu, pu, cu = _run(hu, vol, iso)
+        fu, bu, pu, cu = _run(hu, vol, iso, two_kernel=True)
         assert ff and not fu
         assert np.array_equal(bf, bu)
         assert pf.shape == pu.shape and cf.shape == cu.shape
@@ -103,7 +105,7 @@ def test_fused_z_slabs_concatenate_to_the_single_run():
     pts, cells, pbase, cbase = [], [], 0, 0
     for z0, z1 in zip(bounds[:-1], bounds[1:]):
         lo, hi = max(0, z0 - 2), min(nz, z1 + 2)
-        h = _handle(1)
+        h = _handle()
         h.set_volume(vol[lo:hi])
         h.set_slab(nz, lo, z0, z1)
         n_pts, n_quads = h.count(p)
@@ -126,7 +128,7 @@ def test_fused_falls_back_where_it_does_not_apply():
     P = pkg()
     for dtype, shape in ((np.float32, (4, 5, 50)), (np.uint8, (4, 5, 128))):
         vol, iso = random_volume(shape, dtype, seed=1)
-        h = _handle(1)
+        h = _handle()
         fused, *_ = _run(h, vol, iso)
         assert not fused
         h.close()

@@ -15,8 +15,9 @@ import numpy as np
 import pytest
 
 import range_oracle as R
-from test_gpu_pixel_edges import (DTYPES, DT_IDS, ROUTES, _count_params, _gpu_mesh, _handle, _int_specials,
-                                  _special_floats, assert_same_mesh, pool_volume, route_shape, unpack_bitmask)
+from test_gpu_pixel_edges import (DTYPES, DT_IDS, ROUTES, _count_params, _gpu_mesh, _int_specials, _special_floats,
+                                  assert_same_mesh, pool_volume, route_shape, set_borrowed_volume, set_route_volume,
+                                  unpack_bitmask)
 from util import ROOT, assert_mesh_equal, assert_mesh_equal_up_to_vertex_order, oracle, pkg, read_fixture, smooth_volume
 
 gpu = pytest.mark.gpu
@@ -77,15 +78,16 @@ def _subset(seq, n):
 
 # ---- every route x dtype -------------------------------------------------------------------------------------------------
 @gpu
-@pytest.mark.parametrize("dtype,route", [(d, r) for d in DTYPES for r in sorted(ROUTES) if np.dtype(d).itemsize in ROUTES[r][1]],
+@pytest.mark.parametrize("dtype,route", [(d, r) for d in DTYPES for r in sorted(ROUTES) if np.dtype(d).itemsize in ROUTES[r][0]],
                          ids=lambda v: v if isinstance(v, str) else np.dtype(v).name)
 def test_range_classification_over_the_full_value_range(dtype, route):
-    env, xs, fused = ROUTES[route]
+    xs, misaligned, fused = ROUTES[route]
     vol = pool_volume(dtype, route_shape(dtype, xs[np.dtype(dtype).itemsize]), seed=11)
-    h = _handle(**env)
-    h.set_volume(vol)
+    h = pkg().capi.Handle(0)
+    buf = set_route_volume(h, vol, misaligned)
     check_range_bitmasks(h, vol, range_bounds(dtype), fused, f"{np.dtype(dtype).name} {route} {vol.shape}")
     h.close()
+    del buf
 
 
 @gpu
@@ -93,7 +95,7 @@ def test_range_classification_over_the_full_value_range(dtype, route):
 def test_range_on_the_padded_lattice(dtype):
     """image_border_faces classifies into the padded lattice (k_classify_padded): meshes against the oracle"""
     O, P = oracle(), pkg()
-    vol = pool_volume(dtype, route_shape(dtype, ROUTES["fused"][1][np.dtype(dtype).itemsize]), seed=5)
+    vol = pool_volume(dtype, route_shape(dtype, ROUTES["fused"][0][np.dtype(dtype).itemsize]), seed=5)
     h = P.capi.Handle(0)
     h.set_volume(vol)
     for lo, hi in _subset(range_bounds(dtype), 48):
@@ -109,21 +111,16 @@ def test_range_on_the_padded_lattice(dtype):
 def test_range_classification_of_borrowed_pointers_at_every_alignment(dtype):
     """a device volume at an offset that is a multiple of the pixel size but not of 16 (or 4): the fused and packed
     kernels must not run, the others must classify it as they do an aligned one"""
-    import torch
     P = pkg()
     size = np.dtype(dtype).itemsize
     offsets = sorted({o for o in (size, 4, 8, 12, 16, 24) if o % size == 0})
-    xs = sorted({ROUTES["fused"][1][size]} | ({ROUTES["packed"][1][size]} if size <= 2 else set()))
+    xs = sorted({ROUTES["fused"][0][size]} | ({ROUTES["packed"][0][size]} if size <= 2 else set()))
     bounds = _subset(range_bounds(dtype), 48)
     h = P.capi.Handle(0)
     for nx in xs:
         vol = pool_volume(dtype, route_shape(dtype, nx), seed=nx)
-        raw = torch.from_numpy(vol.reshape(-1).view(np.uint8).copy())
-        buf = torch.zeros(raw.numel() + 64, dtype=torch.uint8, device="cuda")
         for off in offsets:
-            buf[off:off + raw.numel()].copy_(raw)
-            torch.cuda.synchronize()  # (the handle's stream does not wait for torch's)
-            h.set_volume_ptr(buf.data_ptr() + off, dtype, vol.shape[::-1], P.capi.MEM_DEVICE)
+            buf = set_borrowed_volume(h, vol, off)
             h.set_inside_range(*bounds[0])
             h.count(_count_params(0))
             if off % 16:
@@ -163,7 +160,7 @@ def test_range_up_to_the_type_maximum_is_iso_mode(dtype):
     dt = np.dtype(dtype)
     size = dt.itemsize
     h = P.capi.Handle(0)
-    for nx in sorted({ROUTES["fused"][1][size]} | ({ROUTES["packed"][1][size]} if size <= 2 else set())):
+    for nx in sorted({ROUTES["fused"][0][size]} | ({ROUTES["packed"][0][size]} if size <= 2 else set())):
         vol = pool_volume(dtype, route_shape(dtype, nx), seed=21 + nx)
         isos = [lo for lo, _ in _subset(range_bounds(dtype), 24)]
         for iso in isos:

@@ -10,7 +10,6 @@ where the kernel's rsqrt fast path must hand over to the exact division.
 
 The tests marked gpu need a CUDA device; the others check the premises of the GPU tests and run anywhere."""
 import math
-import os
 
 import numpy as np
 import pytest
@@ -21,29 +20,6 @@ gpu = pytest.mark.gpu
 
 DTYPES = [np.uint8, np.int8, np.uint16, np.int16, np.uint32, np.int32, np.float32, np.float64]
 DT_IDS = [np.dtype(d).name for d in DTYPES]
-
-
-class _env:
-    """the tuning knobs are read once, in cub_create: a handle per setting"""
-
-    def __init__(self, **kv):
-        self.kv = {k: str(v) for k, v in kv.items()}
-
-    def __enter__(self):
-        self.old = {k: os.environ.get(k) for k in self.kv}
-        os.environ.update(self.kv)
-
-    def __exit__(self, *a):
-        for k, v in self.old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
-
-
-def _handle(**env):
-    with _env(**env):
-        return pkg().capi.Handle(0)
 
 
 # ---- values ----------------------------------------------------------------------------------------------------------
@@ -131,15 +107,37 @@ def _pixel_bytes(dt):
     return np.dtype(dt).itemsize
 
 
-# ---- classification routes (cuberille_capi.cu: launch_fused, launch_classify, ClassifyPacked) --------------------------
-# row length per pixel size, environment, and whether the fused classification + sweep kernel must have run
+def set_borrowed_volume(h, vol, offset):
+    """`vol` as a borrowed device pointer `offset` bytes into a torch buffer; the buffer is returned and must outlive
+    the handle's use of it"""
+    import torch
+    raw = torch.from_numpy(vol.reshape(-1).view(np.uint8).copy())
+    buf = torch.zeros(raw.numel() + 64, dtype=torch.uint8, device="cuda")
+    buf[offset:offset + raw.numel()].copy_(raw)
+    torch.cuda.synchronize()  # (the handle's stream does not wait for torch's)
+    h.set_volume_ptr(buf.data_ptr() + offset, vol.dtype, vol.shape[::-1], pkg().capi.MEM_DEVICE)
+    return buf
+
+
+def set_route_volume(h, vol, misaligned):
+    """a host upload, or (misaligned) a device pointer one pixel past a 16-byte boundary, where neither the fused
+    kernel (16-byte aligned rows) nor the packed one (4-byte aligned) can run"""
+    if not misaligned:
+        h.set_volume(vol)
+        return None
+    return set_borrowed_volume(h, vol, vol.dtype.itemsize)
+
+
+# ---- classification routes (cuberille_capi.cu: choose_count_route) -------------------------------------------------------
+# row length per pixel size, whether the volume is a misaligned device pointer, and whether the fused classification +
+# sweep kernel must have run
 ROUTES = {
-    "packed": (dict(), {1: 128, 2: 64}, False),                         # 4 bytes per lane: whole warp loads per row
-    "fused": (dict(), {1: 48, 2: 40, 4: 36, 8: 36}, True),              # rows of whole 16-byte groups
-    "fused_unpacked": (dict(CUB_K1_PACKED=0), {1: 128, 2: 64}, True),
-    "full_rows": (dict(CUB_FUSE=0, CUB_K1_PACKED=0), {1: 512, 2: 512, 4: 512, 8: 512}, False),
-    "ragged33": (dict(CUB_FUSE=0), {1: 33, 2: 33, 4: 33, 8: 33}, False),
-    "ragged70": (dict(CUB_FUSE=0), {1: 70, 2: 70, 4: 70, 8: 70}, False),
+    "packed": ({1: 128, 2: 64}, False, False),                          # 4 bytes per lane: whole warp loads per row
+    "fused": ({1: 48, 2: 40, 4: 36, 8: 36}, False, True),               # rows of whole 16-byte groups
+    "fused_unpacked_long_rows": ({1: 4112, 2: 2056}, False, True),      # ... not whole warp loads, and over one 4 KB task
+    "full_rows_unaligned": ({1: 512, 2: 512, 4: 512, 8: 512}, True, False),
+    "ragged33": ({1: 33, 2: 33, 4: 33, 8: 33}, False, False),
+    "ragged70_unaligned": ({1: 70, 2: 70, 4: 70, 8: 70}, True, False),  # (560 bytes of float64 would fuse)
 }
 
 
@@ -170,15 +168,16 @@ def check_bitmasks(h, vol, isos, fused, what):
 
 
 @gpu
-@pytest.mark.parametrize("dtype,route", [(d, r) for d in DTYPES for r in sorted(ROUTES) if _pixel_bytes(d) in ROUTES[r][1]],
+@pytest.mark.parametrize("dtype,route", [(d, r) for d in DTYPES for r in sorted(ROUTES) if _pixel_bytes(d) in ROUTES[r][0]],
                          ids=lambda v: v if isinstance(v, str) else np.dtype(v).name)
 def test_classification_over_the_full_value_range(dtype, route):
-    env, xs, fused = ROUTES[route]
+    xs, misaligned, fused = ROUTES[route]
     vol = pool_volume(dtype, route_shape(dtype, xs[_pixel_bytes(dtype)]), seed=11)
-    h = _handle(**env)
-    h.set_volume(vol)
+    h = pkg().capi.Handle(0)
+    buf = set_route_volume(h, vol, misaligned)
     check_bitmasks(h, vol, iso_values(dtype), fused, f"{np.dtype(dtype).name} {route} {vol.shape}")
     h.close()
+    del buf
 
 
 @gpu
@@ -186,23 +185,18 @@ def test_classification_over_the_full_value_range(dtype, route):
 def test_classification_of_borrowed_pointers_at_every_alignment(dtype):
     """a device volume at an offset that is a multiple of the pixel size but not of 16 (or 4): the fused and packed
     kernels must not run, the others must classify it as they do an aligned one"""
-    import torch
     P = pkg()
     size = _pixel_bytes(dtype)
     offsets = sorted({o for o in (size, 4, 8, 12, 16, 24) if o % size == 0})
-    xs = sorted({ROUTES["fused"][1][size]} | ({ROUTES["packed"][1][size]} if size <= 2 else set()))
+    xs = sorted({ROUTES["fused"][0][size]} | ({ROUTES["packed"][0][size]} if size <= 2 else set()))
     isos = iso_values(dtype)
     if len(isos) > 48:
         isos = isos[::len(isos) // 48]
     h = P.capi.Handle(0)
     for nx in xs:
         vol = pool_volume(dtype, route_shape(dtype, nx), seed=nx)
-        raw = torch.from_numpy(vol.reshape(-1).view(np.uint8).copy())
-        buf = torch.zeros(raw.numel() + 64, dtype=torch.uint8, device="cuda")
         for off in offsets:
-            buf[off:off + raw.numel()].copy_(raw)
-            torch.cuda.synchronize()  # (the handle's stream does not wait for torch's)
-            h.set_volume_ptr(buf.data_ptr() + off, dtype, vol.shape[::-1], P.capi.MEM_DEVICE)
+            buf = set_borrowed_volume(h, vol, off)
             h.count(_count_params(isos[0]))
             if off % 16:
                 assert not h.count_was_fused(), f"fused kernel on a buffer at offset {off}"
@@ -295,7 +289,7 @@ def test_full_range_meshes_and_cell_data(dtype):
     top-bit values and NaN payloads come back byte for byte); the padded lattice (image_border_faces) at the route isos"""
     O, P = oracle(), pkg()
     size = _pixel_bytes(dtype)
-    vol = pool_volume(dtype, route_shape(dtype, ROUTES["fused"][1][size]), seed=5)
+    vol = pool_volume(dtype, route_shape(dtype, ROUTES["fused"][0][size]), seed=5)
     h = P.capi.Handle(0)
     h.set_volume(vol)
     iso = TOP_BIT_ISO[dtype]
