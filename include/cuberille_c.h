@@ -224,11 +224,20 @@ int cub_run_labels(cub_handle h, const cub_params *p, const double *labels, uint
  * (n_cells of the final mesh is n_quads, or 2*n_quads with triangles.)         */
 int cub_count(cub_handle h, const cub_params *p, uint64_t *n_points, uint64_t *n_quads);
 
-/* Slices of halo a z-slab needs below / above its own range for these parameters:
- * 2 / 1 without projection; with projection the reach of a vertex (the geometric
- * sum of its <= max_steps + 2 moves, txx:464-469) plus the interpolation and
- * central-difference footprints.  cub_count refuses a slab whose buffer is
- * shorter (a clamped read would silently change the mesh).                     */
+/* Slices of halo a z-slab needs below / above its own range for these parameters
+ * and the image's geometry (spacing and direction as given to cub_set_volume;
+ * null: 1 and the identity): 2 / 1 without projection; with projection the reach
+ * of a vertex (the geometric sum of its <= max_steps + 2 moves, txx:464-469, in
+ * slices: over spacing[2], or for an oriented image times the 1-norm of the z row
+ * of (D * diag(spacing))^-1) plus the interpolation and central-difference
+ * footprints.  cub_count requires exactly this halo of a slab of an image with
+ * the same geometry, and refuses a shorter buffer (a clamped read would silently
+ * change the mesh).  CUB_ERR_INVALID for a spacing that is not positive and
+ * finite, or a singular or non-finite direction.                               */
+int cub_projection_halo_oriented(const cub_params *p, const double spacing[3], const double direction[9],
+                                 uint64_t *below, uint64_t *above);
+
+/* cub_projection_halo_oriented of a non-oriented image (identity direction).   */
 int cub_projection_halo(const cub_params *p, const double spacing[3],
                         uint64_t *below, uint64_t *above);
 

@@ -32,7 +32,7 @@ SYMBOLS = [
     "cub_synchronize", "cub_device_buffers",
     "cub_debug_bitmask", "cub_debug_project_points", "cub_generate_volume", "cub_download_volume",
     "cub_enable_timing", "cub_get_timings", "cub_launch_count", "cub_count_was_fused",
-    "cub_projection_halo", "cub_count_async", "cub_device_counts", "cub_emit_async", "cub_finish", "cub_last_warning",
+    "cub_projection_halo", "cub_projection_halo_oriented", "cub_count_async", "cub_device_counts", "cub_emit_async", "cub_finish", "cub_last_warning",
     "cub_comm_unique_id", "cub_comm_create", "cub_comm_destroy", "cub_comm_exchange_counts", "cub_comm_counts",
     "cub_comm_gather_mesh", "cub_device_alloc", "cub_device_free", "cub_device_copy",
     "cub_host_register", "cub_host_unregister", "cub_host_alloc", "cub_host_free",
@@ -138,6 +138,8 @@ def load() -> C.CDLL:
     L.cub_count_was_fused.argtypes = [vp]
     L.cub_projection_halo.restype = i
     L.cub_projection_halo.argtypes = [C.POINTER(Params), pd, pu64, pu64]
+    L.cub_projection_halo_oriented.restype = i
+    L.cub_projection_halo_oriented.argtypes = [C.POINTER(Params), pd, pd, pu64, pu64]
     L.cub_count_async.restype = i
     L.cub_count_async.argtypes = [vp, C.POINTER(Params)]
     L.cub_device_counts.restype = i
@@ -178,12 +180,14 @@ def load() -> C.CDLL:
     return L
 
 
-def projection_halo(params: Params, spacing=(1.0, 1.0, 1.0)) -> tuple[int, int]:
-    """Halo slices (below, above) a z-slab needs for these parameters (cub_projection_halo)."""
+def projection_halo(params: Params, spacing=(1.0, 1.0, 1.0), direction=None) -> tuple[int, int]:
+    """Halo slices (below, above) a z-slab of an image with this spacing and direction needs for these parameters
+    (cub_projection_halo_oriented)."""
     lo, hi = C.c_uint64(), C.c_uint64()
-    rc = load().cub_projection_halo(C.byref(params), (C.c_double * 3)(*spacing), C.byref(lo), C.byref(hi))
+    dr = (C.c_double * 9)(*direction) if direction is not None else None
+    rc = load().cub_projection_halo_oriented(C.byref(params), (C.c_double * 3)(*spacing), dr, C.byref(lo), C.byref(hi))
     if rc != 0:
-        raise CuberilleError(rc, "cub_projection_halo")
+        raise CuberilleError(rc, "cub_projection_halo_oriented: bad spacing or direction")
     return lo.value, hi.value
 
 

@@ -516,12 +516,14 @@ int setup_grid(cub_handle h) {
   return CUB_OK;
 }
 
-void compute_step(cub_handle h) {
-  // txx:75-85: auto step length = max spacing * 0.25
-  double ms = h->geom.spacing[0];
-  for (int a = 1; a < 3; ++a) ms = h->geom.spacing[a] > ms ? h->geom.spacing[a] : ms;
-  h->step_used = h->params.step_length < 0.0 ? ms * 0.25 : h->params.step_length;
+// txx:75-85: auto step length = max spacing * 0.25
+double step_length_used(const cub_params& P, const Geom& G) {
+  double ms = G.spacing[0];
+  for (int a = 1; a < 3; ++a) ms = G.spacing[a] > ms ? G.spacing[a] : ms;
+  return P.step_length < 0.0 ? ms * 0.25 : P.step_length;
 }
+
+void compute_step(cub_handle h) { h->step_used = step_length_used(h->params, h->geom); }
 
 }  // namespace
 
@@ -598,6 +600,40 @@ int cub_destroy(cub_handle h) {
 
 const char* cub_last_error(cub_handle h) { return h ? h->err.c_str() : "null handle"; }
 
+// spacing, direction cosines and the matrices built from them (null spacing / direction: 1 / identity), shared by
+// cub_set_volume and cub_projection_halo_oriented so that the halo a slab is cut with and the halo cub_count checks come from
+// the same geometry
+static int make_geom(cub_handle h, const double spacing[3], const double direction[9], Geom& G) {
+  for (int a = 0; a < 3; ++a) {
+    const double s = spacing ? spacing[a] : 1.0;
+    if (!(s > 0.0) || !std::isfinite(s)) return fail(h, CUB_ERR_INVALID, "spacing[%d] must be positive and finite", a);
+    G.spacing[a] = s;
+  }
+  // direction cosines (itk::ImageBase::GetDirection): identity (or null) is the non-oriented image of the
+  // reference's tests; anything else switches TransformIndexToPhysicalPoint, the continuous index and the
+  // gradient to the oriented forms (cbr_common.cuh, k_project.cuh)
+  static const double I[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
+  bool ident = true;
+  for (int i = 0; i < 9; ++i) {
+    const double d = direction ? direction[i] : I[i];
+    if (!std::isfinite(d)) return fail(h, CUB_ERR_INVALID, "direction[%d] is not finite", i);
+    ident = ident && d == I[i];
+  }
+  G.oriented = ident ? 0 : 1;
+  for (int k = 0; k < 9; ++k) {
+    G.dir[k] = ident ? I[k] : direction[k];
+    G.m[k] = G.dir[k] * G.spacing[k % 3];  // D * diag(spacing)
+  }
+  const double* m = G.m;  // cofactor inverse
+  const double c00 = m[4] * m[8] - m[5] * m[7], c01 = m[5] * m[6] - m[3] * m[8], c02 = m[3] * m[7] - m[4] * m[6];
+  const double det = m[0] * c00 + m[1] * c01 + m[2] * c02;
+  if (!(std::fabs(det) > 0.0) || !std::isfinite(det)) return fail(h, CUB_ERR_INVALID, "the direction matrix is singular");
+  G.minv[0] = c00 / det; G.minv[1] = (m[2] * m[7] - m[1] * m[8]) / det; G.minv[2] = (m[1] * m[5] - m[2] * m[4]) / det;
+  G.minv[3] = c01 / det; G.minv[4] = (m[0] * m[8] - m[2] * m[6]) / det; G.minv[5] = (m[2] * m[3] - m[0] * m[5]) / det;
+  G.minv[6] = c02 / det; G.minv[7] = (m[1] * m[6] - m[0] * m[7]) / det; G.minv[8] = (m[0] * m[4] - m[1] * m[3]) / det;
+  return CUB_OK;
+}
+
 static int set_geometry(cub_handle h, int dtype, const uint64_t dims[3], const double spacing[3],
                         const double origin[3], const double direction[9]) {
   if (!dims) return fail(h, CUB_ERR_INVALID, "dims is null");
@@ -605,37 +641,10 @@ static int set_geometry(cub_handle h, int dtype, const uint64_t dims[3], const d
   if (!pb) return fail(h, CUB_ERR_INVALID, "unknown dtype %d", dtype);
   for (int a = 0; a < 3; ++a)
     if (dims[a] == 0 || dims[a] >= (1ull << 31)) return fail(h, CUB_ERR_INVALID, "dims[%d]=%llu out of range", a, (unsigned long long)dims[a]);
+  CUB_TRY(make_geom(h, spacing, direction, h->geom));
   for (int a = 0; a < 3; ++a) {
-    const double s = spacing ? spacing[a] : 1.0;
-    if (!(s > 0.0) || !std::isfinite(s)) return fail(h, CUB_ERR_INVALID, "spacing[%d] must be positive and finite", a);
-    h->geom.spacing[a] = s;
     h->geom.origin[a] = origin ? origin[a] : 0.0;
     h->dims[a] = dims[a];
-  }
-  {
-    // direction cosines (itk::ImageBase::GetDirection): identity (or null) is the non-oriented image of the
-    // reference's tests; anything else switches TransformIndexToPhysicalPoint, the continuous index and the
-    // gradient to the oriented forms (cbr_common.cuh, k_project.cuh)
-    static const double I[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
-    bool ident = true;
-    for (int i = 0; i < 9; ++i) {
-      const double d = direction ? direction[i] : I[i];
-      if (!std::isfinite(d)) return fail(h, CUB_ERR_INVALID, "direction[%d] is not finite", i);
-      ident = ident && d == I[i];
-    }
-    Geom& G = h->geom;
-    G.oriented = ident ? 0 : 1;
-    for (int k = 0; k < 9; ++k) {
-      G.dir[k] = ident ? I[k] : direction[k];
-      G.m[k] = G.dir[k] * G.spacing[k % 3];  // D * diag(spacing)
-    }
-    const double* m = G.m;  // cofactor inverse
-    const double c00 = m[4] * m[8] - m[5] * m[7], c01 = m[5] * m[6] - m[3] * m[8], c02 = m[3] * m[7] - m[4] * m[6];
-    const double det = m[0] * c00 + m[1] * c01 + m[2] * c02;
-    if (!(std::fabs(det) > 0.0) || !std::isfinite(det)) return fail(h, CUB_ERR_INVALID, "the direction matrix is singular");
-    G.minv[0] = c00 / det; G.minv[1] = (m[2] * m[7] - m[1] * m[8]) / det; G.minv[2] = (m[1] * m[5] - m[2] * m[4]) / det;
-    G.minv[3] = c01 / det; G.minv[4] = (m[0] * m[8] - m[2] * m[6]) / det; G.minv[5] = (m[2] * m[3] - m[0] * m[5]) / det;
-    G.minv[6] = c02 / det; G.minv[7] = (m[1] * m[6] - m[0] * m[7]) / det; G.minv[8] = (m[0] * m[4] - m[1] * m[3]) / det;
   }
   h->dtype = dtype;
   h->pix_bytes = pb;
@@ -747,6 +756,18 @@ void projection_reach(const cub_params& P, double step_used, double z_index_per_
   *above = ct + 2;
 }
 
+// the halo of a z-slab of an image with this geometry: what cub_projection_halo_oriented reports and what count_launch requires
+void slab_halo(const cub_params& P, const Geom& G, uint64_t* below, uint64_t* above) {
+  if (!P.project_vertices) {
+    *below = 2;
+    *above = 1;
+    return;
+  }
+  // index-space z travel per unit of physical travel: 1 / spacing_z, or the 1-norm of the z row of M^-1
+  const double zpu = G.oriented ? std::fabs(G.minv[6]) + std::fabs(G.minv[7]) + std::fabs(G.minv[8]) : 1.0 / G.spacing[2];
+  projection_reach(P, step_length_used(P, G), zpu, below, above);
+}
+
 // ---- the count phase, queued on the handle's stream (no host synchronisation) ----------------------------------
 int count_launch(cub_handle h, const cub_params* p) {
   if (!p) return fail(h, CUB_ERR_INVALID, "params is null");
@@ -781,10 +802,7 @@ int count_launch(cub_handle h, const cub_params* p) {
       // a true slab: the projection must not run into the end of the local buffer (its reads would be clamped there
       // and the result would differ from the whole-image run without any error)
       uint64_t below = 0, above = 0;
-      // index-space z travel per unit of physical travel: 1 / spacing_z, or the 1-norm of the z row of M^-1
-      const double zpu = h->geom.oriented ? std::fabs(h->geom.minv[6]) + std::fabs(h->geom.minv[7]) + std::fabs(h->geom.minv[8])
-                                          : 1.0 / h->geom.spacing[2];
-      projection_reach(*p, h->step_used, zpu, &below, &above);
+      slab_halo(*p, h->geom, &below, &above);
       const uint64_t lo = h->own_z0 > below ? h->own_z0 - below : 0;
       const uint64_t hi = h->own_z1 + above < h->image_nz ? h->own_z1 + above : h->image_nz;
       if (h->local_z0 > lo || h->local_z0 + zl < hi)
@@ -1182,16 +1200,17 @@ int cub_count_async(cub_handle h, const cub_params* p) {
   return count_launch(h, p);
 }
 
-int cub_projection_halo(const cub_params* p, const double spacing[3], uint64_t* below, uint64_t* above) {
+int cub_projection_halo_oriented(const cub_params* p, const double spacing[3], const double direction[9],
+                                 uint64_t* below, uint64_t* above) {
   if (!p || !below || !above) return CUB_ERR_INVALID;
-  double sp[3] = {1.0, 1.0, 1.0};
-  if (spacing) for (int a = 0; a < 3; ++a) sp[a] = spacing[a];
-  if (!p->project_vertices) { *below = 2; *above = 1; return CUB_OK; }
-  double ms = sp[0];
-  for (int a = 1; a < 3; ++a) ms = sp[a] > ms ? sp[a] : ms;
-  const double step = p->step_length < 0.0 ? ms * 0.25 : p->step_length;
-  projection_reach(*p, step, 1.0 / sp[2], below, above);
+  Geom G{};
+  CUB_TRY(make_geom(nullptr, spacing, direction, G));
+  slab_halo(*p, G, below, above);
   return CUB_OK;
+}
+
+int cub_projection_halo(const cub_params* p, const double spacing[3], uint64_t* below, uint64_t* above) {
+  return cub_projection_halo_oriented(p, spacing, nullptr, below, above);
 }
 
 int cub_set_id_base(cub_handle h, uint64_t point_id_base, uint64_t cell_id_base) {

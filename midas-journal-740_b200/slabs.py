@@ -24,7 +24,7 @@ class Slab:
 def plan_slabs(image_nz: int, world: int, halo: int = 2, z_range: tuple[int, int] | None = None) -> list[Slab]:
     """Contiguous, near-equal z-slabs of the image (or of its slices `z_range`, e.g. a rank's own range cut once
     more); `halo` >= 2 (classification + first-touch ownership of the shared corner plane); when vertices are
-    projected use capi.projection_halo(params, spacing) (8 for the default parameters and isotropic voxels:
+    projected use capi.projection_halo(params, spacing, direction) (8 for the default parameters and isotropic voxels:
     cub_count refuses a shorter one)."""
     if halo < 2:
         raise ValueError("the halo must be at least 2 slices")
