@@ -41,7 +41,10 @@ enum {
 /* ---- pixel types: TInputImage::PixelType (h:150) ------------------------ */
 enum {
   CUB_U8 = 0, CUB_I8 = 1, CUB_U16 = 2, CUB_I16 = 3,
-  CUB_U32 = 4, CUB_I32 = 5, CUB_F32 = 6, CUB_F64 = 7
+  CUB_U32 = 4, CUB_I32 = 5, CUB_F32 = 6, CUB_F64 = 7,
+  CUB_I64 = 8, CUB_U64 = 9   /* label maps of ITK's IdentifierType and numpy's default int;
+                                an older library of the same ABI version answers
+                                CUB_ERR_INVALID "unknown dtype" */
 };
 
 /* ---- where a caller buffer lives ---------------------------------------- */
@@ -179,7 +182,11 @@ int cub_set_slab(cub_handle h, uint64_t image_nz, uint64_t local_z0,
  * six bounds 0.  Pixels outside the window are ignored.  Integer pixel types
  * only (CUB_ERR_UNSUPPORTED for float32 / float64); 1 <= n_labels <= 65536 and
  * the window must lie inside the pixel type's range, else CUB_ERR_INVALID, as
- * while a region of interest or a z-slab is set.  Synchronises.                */
+ * while a region of interest or a z-slab is set.  Labels are compared in the
+ * pixel type's width, so label 2^32 + 5 of an int64 map is not label 5.  For
+ * uint64 the window must lie in [0, 2^63 - 1], what first_label can express;
+ * pixels above it are ignored like any other pixel outside the window.
+ * Synchronises.                                                                */
 int cub_label_bounds(cub_handle h, int64_t first_label, uint32_t n_labels, uint64_t *out);
 
 /* Region of interest: from now on cub_count / cub_count_async (and
@@ -210,8 +217,12 @@ int cub_set_region_of_interest(cub_handle h, const uint64_t lo[3], const uint64_
  * cub_label_bounds pass finds the boxes, and a label without voxels gives an
  * empty part and launches nothing.  The labels must be pixel values of the
  * volume's integer type (the rule of cub_set_inside_range), each given once,
- * else CUB_ERR_INVALID; so do project_vertices != 0 (a label has no
- * iso-surface), a set region of interest and a z-slab.  A float volume returns
+ * else CUB_ERR_INVALID.  A label is a double, so of int64 / uint64 maps only
+ * the labels a double holds exactly can be given: every one up to 2^53 in
+ * magnitude, and beyond that the even ones, then multiples of 4, ...; and of
+ * uint64 maps only labels up to 2^63 - 1, the windows of cub_label_bounds.
+ * project_vertices != 0 (a label has no iso-surface), a set region of
+ * interest and a z-slab return CUB_ERR_INVALID too.  A float volume returns
  * CUB_ERR_UNSUPPORTED.  The handle's own inside-range setting is left as it
  * was.  cub_last_warning names the labels whose mesh has an empty interior
  * slice.  Synchronises once per label.                                         */

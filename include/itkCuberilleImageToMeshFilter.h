@@ -35,6 +35,7 @@
 #define __itkCuberilleImageToMeshFilter_h
 
 #include <chrono>
+#include <cmath>
 #include <cstdint>
 #include <limits>
 #include <type_traits>
@@ -68,16 +69,19 @@ namespace itk
 
 namespace cuberille_detail
 {
-template <typename T> struct PixelCode;
-template <> struct PixelCode<unsigned char>  { static const int value = CUB_U8; };
-template <> struct PixelCode<signed char>    { static const int value = CUB_I8; };
-template <> struct PixelCode<char>           { static const int value = std::is_signed<char>::value ? CUB_I8 : CUB_U8; };
-template <> struct PixelCode<unsigned short> { static const int value = CUB_U16; };
-template <> struct PixelCode<short>          { static const int value = CUB_I16; };
-template <> struct PixelCode<unsigned int>   { static const int value = CUB_U32; };
-template <> struct PixelCode<int>            { static const int value = CUB_I32; };
-template <> struct PixelCode<float>          { static const int value = CUB_F32; };
-template <> struct PixelCode<double>         { static const int value = CUB_F64; };
+// An integer pixel type maps to the code of its size and signedness, so long and unsigned long (ITK's IdentifierType)
+// land on the 64-bit codes where they are 64 bits wide and on the 32-bit codes where they are not (LLP64).
+template <typename T, bool = std::is_integral<T>::value && !std::is_same<T, bool>::value> struct PixelCode;
+template <typename T> struct PixelCode<T, true>
+{
+  static_assert( sizeof( T ) == 1 || sizeof( T ) == 2 || sizeof( T ) == 4 || sizeof( T ) == 8, "no pixel code of this size" );
+  static const int value = sizeof( T ) == 1 ? ( std::is_signed<T>::value ? CUB_I8 : CUB_U8 )
+                         : sizeof( T ) == 2 ? ( std::is_signed<T>::value ? CUB_I16 : CUB_U16 )
+                         : sizeof( T ) == 4 ? ( std::is_signed<T>::value ? CUB_I32 : CUB_U32 )
+                                            : ( std::is_signed<T>::value ? CUB_I64 : CUB_U64 );
+};
+template <> struct PixelCode<float, false>  { static const int value = CUB_F32; };
+template <> struct PixelCode<double, false> { static const int value = CUB_F64; };
 }
 
 template < class TInputImage, class TOutputMesh, class TInterpolator = itk::LinearInterpolateImageFunction<TInputImage> >
@@ -389,14 +393,15 @@ protected:
         itkExceptionMacro( << "an inside range has no iso-surface to project the vertices onto: call "
                            "ProjectVerticesToIsoSurfaceOff() (projection is on by default)" );
         }
-      this->Check( cub_set_inside_range( m_Handle, 1, static_cast<double>( m_InsideRangeLower ),
-                                         static_cast<double>( m_InsideRangeUpper ) ) );
+      this->Check( cub_set_inside_range( m_Handle, 1, this->PixelAsDouble( m_InsideRangeLower, "inside range bound" ),
+                                         this->PixelAsDouble( m_InsideRangeUpper, "inside range bound" ) ) );
       }
     this->Check( cub_synchronize( m_Handle ) );
     const Clock::time_point t1 = Clock::now();
     cub_params params;
     cub_default_params( &params );
-    params.iso_value = static_cast<double>( m_IsoSurfaceValue );
+    params.iso_value = ( labels || m_InsideRangeOn ) ? static_cast<double>( m_IsoSurfaceValue )
+                                                     : this->PixelAsDouble( m_IsoSurfaceValue, "iso-surface value" );
     params.generate_triangles = m_GenerateTriangleFaces ? 1 : 0;
     params.project_vertices = m_ProjectVerticesToIsoSurface ? 1 : 0;
     params.save_pixel_as_cell_data = m_SavePixelAsCellData ? 1 : 0;
@@ -414,7 +419,8 @@ protected:
     uint64_t numberOfPoints = 0, numberOfCells = 0;
     if ( labels )
       {
-      std::vector<double> values( m_LabelValues.begin(), m_LabelValues.end() );
+      std::vector<double> values;
+      for ( size_t i = 0; i < m_LabelValues.size(); i++ ) { values.push_back( this->PixelAsDouble( m_LabelValues[i], "label" ) ); }
       m_LabelPointOffsets.assign( values.size() + 1, 0 );
       m_LabelCellOffsets.assign( values.size() + 1, 0 );
       this->Check( cub_run_labels( m_Handle, &params, values.data(), values.size(), 4, m_LabelPointOffsets.data(),
@@ -513,6 +519,20 @@ private:
       {
       itkExceptionMacro( << "cuberille C-ABI error " << status << ": " << cub_last_error( m_Handle ) );
       }
+    }
+
+  // A pixel value travels through the C-ABI as a double.  Every value of the 8- to 32-bit types and of float / double
+  // is one; a 64-bit integer beyond 2^53 may not be, and its rounded neighbour would silently take its place.
+  double PixelAsDouble( InputPixelType v, const char * what )
+    {
+    const double d = static_cast<double>( v );
+    if ( std::numeric_limits<InputPixelType>::is_integer &&
+         !( d < std::ldexp( 1.0, std::numeric_limits<InputPixelType>::digits ) && static_cast<InputPixelType>( d ) == v ) )
+      {
+      itkExceptionMacro( << what << " " << static_cast< typename NumericTraits<InputPixelType>::PrintType >( v )
+                         << " is not exactly representable as a double" );
+      }
+    return d;
     }
 
   InputPixelType      m_IsoSurfaceValue;

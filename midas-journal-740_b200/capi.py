@@ -12,7 +12,7 @@ import numpy as np
 
 from . import _build
 
-U8, I8, U16, I16, U32, I32, F32, F64 = range(8)
+U8, I8, U16, I16, U32, I32, F32, F64, I64, U64 = range(10)
 MEM_HOST, MEM_DEVICE = 0, 1
 GEN_GYROID, GEN_MARSCHNER_LOBB, GEN_BLOBS = 0, 1, 2
 ORDER_REFERENCE, ORDER_RASTER = 0, 1
@@ -21,6 +21,7 @@ PROJECT_DEFAULT, PROJECT_ADVANCED, PROJECT_LINESEARCH = 0, 1, 2
 DTYPE_CODES = {
     np.dtype(np.uint8): U8, np.dtype(np.int8): I8, np.dtype(np.uint16): U16, np.dtype(np.int16): I16,
     np.dtype(np.uint32): U32, np.dtype(np.int32): I32, np.dtype(np.float32): F32, np.dtype(np.float64): F64,
+    np.dtype(np.int64): I64, np.dtype(np.uint64): U64,
 }
 CODE_DTYPES = {v: k for k, v in DTYPE_CODES.items()}
 
@@ -54,6 +55,17 @@ class Params(C.Structure):
         ("projection_method", C.c_int32),
         ("reserved", C.c_int32),
     ]
+
+
+def pixel_value(v) -> float:
+    """A pixel value (iso value, range bound, label) as the double the C-ABI takes.  Python and numpy integers beyond
+    2^53 may have no such double; rounding would silently put a neighbouring value in their place, so they raise."""
+    if isinstance(v, (int, np.integer)) and not isinstance(v, bool):
+        d = float(int(v))
+        if int(d) != int(v):
+            raise ValueError(f"pixel value {int(v)} is not exactly representable as a double")
+        return d
+    return float(v)
 
 
 class CuberilleError(RuntimeError):
@@ -255,7 +267,7 @@ class Handle:
         """Range mode: a voxel is inside when lower <= v <= upper in the pixel type (NaN pixels too), instead of
         v >= iso.  Both bounds must be pixel values of the volume's type; a label k is (k, k).  Projection is refused
         while the mode is on.  After set_volume, which turns the mode off."""
-        self._check(self._L.cub_set_inside_range(self._h, 1, float(lower), float(upper)))
+        self._check(self._L.cub_set_inside_range(self._h, 1, pixel_value(lower), pixel_value(upper)))
 
     def clear_inside_range(self):
         """Back to iso mode."""
@@ -282,7 +294,7 @@ class Handle:
     def run_labels(self, params: Params, labels, id_bytes: int = 4):
         """Mesh every label as the range [k, k], concatenated in the given order; returns (point_offsets, cell_offsets),
         n_labels + 1 entries each.  Read the mesh with fetch() / device_buffers()."""
-        lab = np.ascontiguousarray(labels, np.float64).reshape(-1)
+        lab = np.array([pixel_value(k) for k in np.asarray(labels).reshape(-1).tolist()], np.float64)
         po = np.zeros(lab.size + 1, np.uint64)
         co = np.zeros(lab.size + 1, np.uint64)
         self._check(self._L.cub_run_labels(self._h, C.byref(params), lab.ctypes.data_as(C.POINTER(C.c_double)), lab.size,

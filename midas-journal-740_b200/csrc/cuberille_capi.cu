@@ -227,7 +227,7 @@ int pixel_bytes(int dtype) {
     case CUB_U8: case CUB_I8: return 1;
     case CUB_U16: case CUB_I16: return 2;
     case CUB_U32: case CUB_I32: case CUB_F32: return 4;
-    case CUB_F64: return 8;
+    case CUB_F64: case CUB_I64: case CUB_U64: return 8;
     default: return 0;
   }
 }
@@ -242,16 +242,21 @@ int pixel_bytes(int dtype) {
     case CUB_I32: { typedef int            T; CALL; } break; \
     case CUB_F32: { typedef float          T; CALL; } break; \
     case CUB_F64: { typedef double         T; CALL; } break; \
+    case CUB_I64: { typedef long long      T; CALL; } break; \
+    case CUB_U64: { typedef unsigned long long T; CALL; } break; \
     default: break;                                          \
   }
 
 // (double)(T)iso : m_IsoSurfaceValue is an InputPixelType (h:326).  An iso outside an integer T's range (or NaN) has
 // no such value, and converting it to T would be undefined behaviour: it comes back as NaN, which equals no iso.
+// The range is [min, max + 1) with max + 1 (a power of two) as the bound: for the 64-bit types (double)max rounds up
+// to max + 1 itself, which does not convert.
 template <typename T>
 double iso_in_type(double iso) {
-  if (std::is_integral<T>::value &&
-      !(iso >= (double)std::numeric_limits<T>::min() && iso <= (double)std::numeric_limits<T>::max()))
-    return std::numeric_limits<double>::quiet_NaN();
+  if constexpr (std::is_integral<T>::value) {
+    const double end = 2.0 * (double)(std::numeric_limits<T>::max() / 2 + 1);
+    if (!(iso >= (double)std::numeric_limits<T>::min() && iso < end)) return std::numeric_limits<double>::quiet_NaN();
+  }
   return (double)(T)iso;
 }
 
@@ -1489,12 +1494,14 @@ int cub_count_was_fused(cub_handle h) { return (h && h->fused_last) ? 1 : 0; }
 // ---- label maps: per-label bounds, a region of interest, and every label meshed in its box ----------------------
 namespace {
 
-// the value range of an integer pixel type; false for the float types
+// the value range of an integer pixel type, as far as a long long holds it (uint64: [0, 2^63 - 1], the labels an
+// int64 first_label reaches); false for the float types
 template <typename T>
 bool type_range(long long* lo, long long* hi) {
   if constexpr (std::is_integral<T>::value) {
+    const unsigned long long max = (unsigned long long)std::numeric_limits<T>::max();
     *lo = (long long)std::numeric_limits<T>::min();
-    *hi = (long long)std::numeric_limits<T>::max();
+    *hi = max > (unsigned long long)std::numeric_limits<long long>::max() ? std::numeric_limits<long long>::max() : (long long)max;
     return true;
   }
   return false;
@@ -1520,12 +1527,13 @@ int label_bounds(cub_handle h, long long first, uint32_t n, uint64_t* out) {
   const unsigned long long warp_rows = (1ull << 32) / X - 1;
   blocks = std::max(blocks, (rows + warp_rows * 8 - 1) / (warp_rows * 8));
   if (blocks >= (1ull << 31)) return fail(h, CUB_ERR_UNSUPPORTED, "volume too large for cub_label_bounds");
-  const unsigned f = (unsigned)(unsigned long long)first;
   switch (h->dtype) {
 #define CUB_LABEL_BOUNDS(CODE, T)                                                                                      \
     case CODE:                                                                                                         \
       k_label_bounds<T><<<(unsigned)blocks, kLabelThreads, 0, h->stream>>>(static_cast<const T*>(h->d_vol), (unsigned)X, \
-                                                                         (unsigned)h->dims[1], rows, f, n, h->label_table.p); \
+                                                                         (unsigned)h->dims[1], rows,                  \
+                                                                         (LabelKey<T>)(unsigned long long)first, n,   \
+                                                                         h->label_table.p);                           \
       break;
     CUB_LABEL_BOUNDS(CUB_U8, unsigned char)
     CUB_LABEL_BOUNDS(CUB_I8, signed char)
@@ -1533,6 +1541,8 @@ int label_bounds(cub_handle h, long long first, uint32_t n, uint64_t* out) {
     CUB_LABEL_BOUNDS(CUB_I16, short)
     CUB_LABEL_BOUNDS(CUB_U32, unsigned int)
     CUB_LABEL_BOUNDS(CUB_I32, int)
+    CUB_LABEL_BOUNDS(CUB_I64, long long)
+    CUB_LABEL_BOUNDS(CUB_U64, unsigned long long)
 #undef CUB_LABEL_BOUNDS
     default: return fail(h, CUB_ERR_UNSUPPORTED, "label bounds need an integer pixel type");
   }
@@ -1641,11 +1651,13 @@ int run_labels(cub_handle h, const cub_params* p, const double* labels, uint64_t
   std::vector<uint64_t> bounds(8 * (size_t)n), window;
   for (size_t i = 0; i < sorted.size();) {
     size_t j = i;
-    while (j < sorted.size() && sorted[j] - sorted[i] < 65536) ++j;
-    const uint32_t span = (uint32_t)(sorted[j - 1] - sorted[i] + 1);
+    // (label distances in unsigned arithmetic: two int64 labels can be more than 2^63 apart)
+    auto dist = [&](size_t k) { return (unsigned long long)sorted[k] - (unsigned long long)sorted[i]; };
+    while (j < sorted.size() && dist(j) < 65536) ++j;
+    const uint32_t span = (uint32_t)(dist(j - 1) + 1);
     window.resize(8 * (size_t)span);
     CUB_TRY(label_bounds(h, sorted[i], span, window.data()));
-    for (size_t k = i; k < j; ++k) std::copy_n(&window[8 * (size_t)(sorted[k] - sorted[i])], 8, &bounds[8 * k]);
+    for (size_t k = i; k < j; ++k) std::copy_n(&window[8 * (size_t)dist(k)], 8, &bounds[8 * k]);
     i = j;
   }
   const bool tri = p->generate_triangles != 0, cd = p->save_pixel_as_cell_data != 0;
@@ -1712,9 +1724,10 @@ int cub_label_bounds(cub_handle h, int64_t first_label, uint32_t n_labels, uint6
   if (!out) return fail(h, CUB_ERR_INVALID, "out is null");
   if (h->roi_on || has_slab(h)) return fail(h, CUB_ERR_INVALID, "cub_label_bounds runs on a whole volume: no region of interest or z-slab");
   if (n_labels < 1 || n_labels > 65536) return fail(h, CUB_ERR_INVALID, "n_labels = %u is not in [1, 65536]", n_labels);
-  if (first_label < lo || first_label + (long long)n_labels - 1 > hi)
-    return fail(h, CUB_ERR_INVALID, "label window [%lld, %lld] is not inside the pixel type's range [%lld, %lld]",
-                (long long)first_label, (long long)first_label + n_labels - 1, lo, hi);
+  // (the distance to hi in unsigned arithmetic: first_label + n_labels - 1 may not fit a long long)
+  if (first_label < lo || first_label > hi || (unsigned long long)hi - (unsigned long long)first_label < n_labels - 1ull)
+    return fail(h, CUB_ERR_INVALID, "label window of %u labels from %lld is not inside the pixel type's range [%lld, %lld]",
+                n_labels, (long long)first_label, lo, hi);
   return label_bounds(h, first_label, n_labels, out);
 }
 
@@ -1749,9 +1762,14 @@ int cub_run_labels(cub_handle h, const cub_params* p, const double* labels, uint
   if (h->roi_on) return fail(h, CUB_ERR_INVALID, "cub_run_labels runs on the whole volume: clear the region of interest");
   if (has_slab(h)) return fail(h, CUB_ERR_INVALID, "cub_run_labels does not run on a z-slab");
   if (id_bytes != 4 && id_bytes != 8) return fail(h, CUB_ERR_INVALID, "id_bytes must be 4 or 8");
-  for (uint64_t i = 0; i < n_labels; ++i)
+  for (uint64_t i = 0; i < n_labels; ++i) {
     if (std::isnan(labels[i]) || iso_as_pixel(h->dtype, labels[i]) != labels[i])
       return fail(h, CUB_ERR_INVALID, "label %.17g is not representable in the pixel type", labels[i]);
+    // (the windows of cub_label_bounds, and the keys run_labels sorts, are long longs: uint64 labels end at 2^63 - 1,
+    // and (double)hi rounds up to 2^63, so the bound is 2^63 itself)
+    if (hi == std::numeric_limits<long long>::max() && !(labels[i] < 0x1p63))
+      return fail(h, CUB_ERR_INVALID, "label %.17g is above %lld, the largest label a window reaches", labels[i], hi);
+  }
   {
     std::vector<double> s(labels, labels + n_labels);
     std::sort(s.begin(), s.end());

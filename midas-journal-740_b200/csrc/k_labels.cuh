@@ -7,22 +7,32 @@
 // one before, and folds each voxel into one of them: a row that crosses an object goes background -> label ->
 // background without a flush.  Only a third label flushes the older aggregate, and the flushes of a warp are merged per
 // label (__match_any_sync + warp reductions) before one lane issues the atomics.  A 16-byte load whose pixels all equal
-// the lane's current label costs four compares.
+// the lane's current label costs four 32-bit compares, or two 64-bit ones for 8-byte pixels.  Label keys and the
+// pattern are as wide as the pixel: a 64-bit label is compared in 64 bits, so 2^32 + 5 is not label 5.
 #pragma once
+#include <type_traits>
+
 #include "cbr_common.cuh"
 
 namespace cbr {
 
 constexpr int kLabelThreads = 256;
 constexpr int kLabelCtasPerSm = 3;   // resident CTAs per SM at the register budget of __launch_bounds__
-constexpr unsigned kNoLabel = 0xffffffffu;
+
+// the unsigned type of a label's window key and of its compare pattern: 32 bits up to 4-byte pixels, else 64
+template <typename T>
+using LabelKey = typename std::conditional<sizeof(T) == 8, unsigned long long, unsigned>::type;
+
+template <typename K>
+__device__ __forceinline__ constexpr K no_label() { return ~K(0); }
 
 // Table entry of window label i: 8 words {count, ~xmin, ~ymin, ~zmin, xmax, ymax, zmax, 0}.  The minima are stored as
 // 32-bit complements, so every field only grows and the whole table starts from one memset to 0 (the host undoes the
 // complement).
+template <typename K>
 struct LabelAcc {
-  unsigned key;   // window index of the label, or kNoLabel
-  unsigned pat;   // the label's pixel bits replicated over 32 bits (the compare of a whole 16-byte load)
+  K key;   // window index of the label, or no_label<K>()
+  K pat;   // the label's pixel bits replicated over K (the compare of a whole 16-byte load)
   unsigned count;
   unsigned x0, x1, y0, y1, z0, z1;
 };
@@ -33,8 +43,9 @@ __device__ __forceinline__ void label_max(unsigned long long* p, unsigned long l
 }
 
 // Warp-collective: every lane with `flush` adds its aggregate to the table, one atomic per label and field per warp.
-__device__ __forceinline__ void label_flush(unsigned long long* table, const LabelAcc& a, bool flush) {
-  const unsigned m = __match_any_sync(0xffffffffu, flush ? a.key : kNoLabel);
+template <typename K>
+__device__ __forceinline__ void label_flush(unsigned long long* table, const LabelAcc<K>& a, bool flush) {
+  const unsigned m = __match_any_sync(0xffffffffu, flush ? a.key : no_label<K>());
   if (!flush) return;
   const unsigned c = __reduce_add_sync(m, a.count);
   const unsigned nx0 = __reduce_max_sync(m, ~a.x0), ny0 = __reduce_max_sync(m, ~a.y0), nz0 = __reduce_max_sync(m, ~a.z0);
@@ -48,9 +59,13 @@ __device__ __forceinline__ void label_flush(unsigned long long* table, const Lab
 }
 
 template <typename T>
-__device__ __forceinline__ unsigned label_pattern(T v) {
-  const unsigned u = sizeof(T) == 1 ? (unsigned)(unsigned char)v : (sizeof(T) == 2 ? (unsigned)(unsigned short)v : (unsigned)v);
-  return sizeof(T) == 1 ? u * 0x01010101u : (sizeof(T) == 2 ? u * 0x00010001u : u);
+__device__ __forceinline__ LabelKey<T> label_pattern(T v) {
+  if constexpr (sizeof(T) == 8) {
+    return (unsigned long long)v;
+  } else {
+    const unsigned u = sizeof(T) == 1 ? (unsigned)(unsigned char)v : (sizeof(T) == 2 ? (unsigned)(unsigned short)v : (unsigned)v);
+    return sizeof(T) == 1 ? u * 0x01010101u : (sizeof(T) == 2 ? u * 0x00010001u : u);
+  }
 }
 
 template <typename T>
@@ -61,11 +76,20 @@ union LabelChunk {
 
 // One chunk of a row: nv (<= V) pixels from x = x0.  Warp-collective: every lane of the warp calls it, nv = 0 for none.
 template <typename T>
-__device__ __forceinline__ void label_chunk(unsigned long long* table, LabelAcc& a, LabelAcc& b, const LabelChunk<T>& u, int nv,
-                                            unsigned x0, unsigned y, unsigned z, unsigned first, unsigned n) {
+__device__ __forceinline__ void label_chunk(unsigned long long* table, LabelAcc<LabelKey<T>>& a, LabelAcc<LabelKey<T>>& b,
+                                            const LabelChunk<T>& u, int nv, unsigned x0, unsigned y, unsigned z,
+                                            LabelKey<T> first, unsigned n) {
+  using K = LabelKey<T>;
   constexpr int V = 16 / sizeof(T);
-  const bool same = nv == 0 || (nv == V && a.key != kNoLabel && u.w.x == a.pat && u.w.y == a.pat && u.w.z == a.pat &&
-                                u.w.w == a.pat);
+  constexpr K kNoLabel = no_label<K>();
+  // every pixel of a whole 16-byte load is the current label: four 32-bit compares, or two 64-bit ones
+  bool same;
+  if constexpr (sizeof(T) == 8)
+    same = nv == 0 || (nv == V && a.key != kNoLabel && (((unsigned long long)u.w.y << 32) | u.w.x) == a.pat &&
+                       (((unsigned long long)u.w.w << 32) | u.w.z) == a.pat);
+  else
+    same = nv == 0 || (nv == V && a.key != kNoLabel && u.w.x == a.pat && u.w.y == a.pat && u.w.z == a.pat &&
+                       u.w.w == a.pat);
   if (__all_sync(0xffffffffu, same)) {
     if (nv) {
       a.count += V;
@@ -77,14 +101,14 @@ __device__ __forceinline__ void label_chunk(unsigned long long* table, LabelAcc&
   }
 #pragma unroll
   for (int k = 0; k < V; ++k) {
-    unsigned key = (unsigned)u.v[k] - first;   // (the window lies inside the type: no wrap-around reaches [0, n))
+    K key = (K)u.v[k] - first;   // (the window lies inside the type: no wrap-around reaches [0, n))
     if (k >= nv || key >= n) key = kNoLabel;
     const bool flush = key != kNoLabel && key != a.key && key != b.key && b.key != kNoLabel;
     if (__any_sync(0xffffffffu, flush)) label_flush(table, b, flush);
     if (key != kNoLabel) {
       const unsigned x = x0 + k;
       if (key != a.key) {
-        const LabelAcc older = b;
+        const LabelAcc<K> older = b;
         b = a;
         if (key == older.key) {
           a = older;
@@ -106,12 +130,13 @@ __device__ __forceinline__ void label_chunk(unsigned long long* table, LabelAcc&
 // 32-bit: the host sizes the grid so that a warp sees fewer than 2^32 voxels.
 template <typename T>
 __global__ void __launch_bounds__(kLabelThreads, kLabelCtasPerSm)
-    k_label_bounds(const T* __restrict__ vol, unsigned X, unsigned Y, unsigned long long rows, unsigned first, unsigned n,
-                   unsigned long long* __restrict__ table) {
+    k_label_bounds(const T* __restrict__ vol, unsigned X, unsigned Y, unsigned long long rows, LabelKey<T> first,
+                   unsigned n, unsigned long long* __restrict__ table) {
+  using K = LabelKey<T>;
   constexpr int V = 16 / sizeof(T);
   const int lane = threadIdx.x & 31;
   const unsigned long long warps = (unsigned long long)gridDim.x * (kLabelThreads / 32);
-  LabelAcc a{kNoLabel, 0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u}, b = a;   // the current label and the one before
+  LabelAcc<K> a{no_label<K>(), 0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u}, b = a;   // the current label and the one before
   for (unsigned long long r = blockIdx.x * (unsigned long long)(kLabelThreads / 32) + (threadIdx.x >> 5); r < rows; r += warps) {
     const unsigned y = (unsigned)(r % Y), z = (unsigned)(r / Y);
     const T* row = vol + r * X;
@@ -149,8 +174,8 @@ __global__ void __launch_bounds__(kLabelThreads, kLabelCtasPerSm)
       label_chunk<T>(table, a, b, u[1], nv[1], x0[1], y, z, first, n);
     }
   }
-  label_flush(table, a, a.key != kNoLabel);
-  label_flush(table, b, b.key != kNoLabel);
+  label_flush(table, a, a.key != no_label<K>());
+  label_flush(table, b, b.key != no_label<K>());
 }
 
 // cub_set_region_of_interest: the box [lo, lo + size) of an x-fastest volume into a dense buffer, one CTA per row.

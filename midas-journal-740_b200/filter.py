@@ -146,7 +146,7 @@ class CuberilleImageToMeshFilter:
     # -- pipeline ------------------------------------------------------------------------------
     def params(self) -> capi.Params:
         p = capi.default_params()
-        p.iso_value = float(self._iso)
+        p.iso_value = capi.pixel_value(self._iso)
         p.generate_triangles = int(self._triangles)
         p.project_vertices = int(self._project)
         p.save_pixel_as_cell_data = int(self._cell_data)

@@ -15,6 +15,7 @@ import numpy as np
 _MET_TYPES = {
     "MET_UCHAR": np.uint8, "MET_CHAR": np.int8, "MET_USHORT": np.uint16, "MET_SHORT": np.int16,
     "MET_UINT": np.uint32, "MET_INT": np.int32, "MET_FLOAT": np.float32, "MET_DOUBLE": np.float64,
+    "MET_LONG_LONG": np.int64, "MET_ULONG_LONG": np.uint64,
 }
 _MET_NAMES = {np.dtype(v): k for k, v in _MET_TYPES.items()}
 
